@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the occupancy -> SDF hot path on B200 (BASELINE.json metric: SDF Gvoxels/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one ExtractSignedDistanceField<float> over one synthetic occupancy grid.
 Workload (weak scaling, 512^3 voxels per GPU, x-slab sharded):
@@ -404,6 +404,32 @@ def config5_2048(sharded, vdev, synthetic, dev, rank, world, steps):
             "hbm_floor_ms": SDF_BYTES_PER_VOXEL * voxels / world / (peak * 1e9) * 1e3}
 
 
+DUMP_SAMPLE_VOXELS = 4 << 20
+
+
+def dump_outputs(directory, sdf, min_max, rank=0, world=1):
+    """Writes what the last timed step returned, so that two builds can be compared output for
+    output: the SDF's (min, max) and the SDF at a fixed, seeded sample of up to 4 Mi distinct
+    voxel positions in all (the whole field is 512 MiB per GPU), with the flat [x, y, z] indices
+    of the sample. Files: sdf_min_max.npy, sdf_sample.npy, sdf_sample_index.npy (float64 holds
+    every index exactly); at most 48 MiB in all. At N > 1 every rank samples its own y-slab
+    (4 Mi / N positions, indices within the slab) into sdf_sample_rank<r>.npy and
+    sdf_sample_index_rank<r>.npy, and rank 0 writes the global (min, max)."""
+    import numpy as np
+    import torch
+    directory = Path(directory)
+    directory.mkdir(parents=True, exist_ok=True)
+    flat = sdf.reshape(-1)
+    index = np.unique(np.random.default_rng(rank).integers(
+        0, flat.numel(), min(flat.numel(), DUMP_SAMPLE_VOXELS // world)))
+    values = flat[torch.from_numpy(index).to(flat.device)].cpu().numpy()
+    suffix = "" if world == 1 else f"_rank{rank}"
+    if rank == 0:
+        np.save(directory / "sdf_min_max.npy", min_max.cpu().numpy().astype(np.float32))
+    np.save(directory / f"sdf_sample{suffix}.npy", values.astype(np.float32))
+    np.save(directory / f"sdf_sample_index{suffix}.npy", index.astype(np.float64))
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -467,6 +493,9 @@ def run_ours(args):
     ms_per_step = elapsed_ms / args.steps
     value = voxels / (ms_per_step * 1e-3) / 1e9
     sdf_min_max = [float(v) for v in result[1].tolist()]
+    # (before the legs below: the per-kernel timing writes into the same output buffer)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *result, rank=rank, world=n_gpus)
 
     stage_ms = None
     if distributed:
@@ -1030,7 +1059,14 @@ def main():
     parser.add_argument("--exchange", default="auto", choices=["auto", "peer_store", "peer_copy", "nccl"])
     parser.add_argument("--chunks", type=int, default=2,
                         help="x-chunks per slab for overlapping the all-to-all (N > 1)")
+    parser.add_argument("--dump-outputs", metavar="DIR",
+                        help="write the SDF of the last timed step (a fixed sample) and its "
+                             "min/max to DIR/*.npy")
     args = parser.parse_args()
+    if args.steps < 1:
+        parser.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        parser.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -314,3 +314,28 @@ def test_transform_in_place_rejects_what_it_cannot_do_exactly(shared_library):
         vgt.ComputeDistanceFieldTransformInPlace(np.full((4, 4, 4), 2.0 ** 30))
     with pytest.raises(ValueError):
         vgt.ComputeDistanceFieldTransformInPlace(np.zeros((4, 4), dtype=np.float64))
+
+
+def test_bench_dumps_the_sdf_of_its_last_timed_step(shared_library, oracle, tmp_path):
+    # bench.py --dump-outputs end to end: the sampled SDF and its min/max equal the oracle's SDF
+    # of the bench grid at the sampled positions
+    import subprocess
+    import sys
+    from pathlib import Path
+
+    import torch
+    from voxelized_geometry_tools_b200 import synthetic
+    repo = Path(__file__).resolve().parents[1]
+    result = subprocess.run(
+        [sys.executable, str(repo / "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+         "--skip-cpu", "--skip-voxelizer", "--skip-strong", "--dump-outputs", str(tmp_path)],
+        capture_output=True, text=True, timeout=1200)
+    assert result.returncode == 0, result.stderr[-3000:]
+    dims = (512, 512, 512)
+    occupancy = synthetic.clustered_spheres_occupancy_torch(dims, torch.device("cuda", 0)).cpu()
+    want, (lo, hi) = oracle.sdf(occupancy.numpy(), 0.02)
+    index = np.load(tmp_path / "sdf_sample_index.npy").astype(np.int64)
+    assert len(index) > 3_000_000
+    np.testing.assert_array_equal(np.load(tmp_path / "sdf_sample.npy"), want.reshape(-1)[index])
+    np.testing.assert_array_equal(np.load(tmp_path / "sdf_min_max.npy"),
+                                  np.array([lo, hi], dtype=np.float32))

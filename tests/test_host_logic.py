@@ -139,3 +139,40 @@ def test_bench_finds_the_ncu_traffic_of_every_pass():
         entry = json.loads(bench.NCU_TRAFFIC_FILE.read_text())["x".join(map(str, dims))][name]
         checked = bench.ncu_dram_bytes_per_launch(dims, name)
         assert (checked is not None) == (entry.get("sources_sha1") == cuda_build._sources_signature())
+
+
+def test_bench_dumps_a_fixed_sample_of_the_sdf(tmp_path):
+    # bench.py --dump-outputs: the same output gives the same files, so two builds compare
+    # value for value; every file is float32 or float64
+    import importlib.util
+    from pathlib import Path
+
+    import torch
+    repo = Path(__file__).resolve().parents[1]
+    spec = importlib.util.spec_from_file_location("bench_module", repo / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    sdf = torch.from_numpy(np.random.default_rng(3).standard_normal((40, 48, 56), np.float32))
+    min_max = torch.tensor([sdf.min(), sdf.max()])
+    for name in ("a", "b"):
+        bench.dump_outputs(tmp_path / name, sdf, min_max)
+    for name in ("sdf_min_max.npy", "sdf_sample.npy", "sdf_sample_index.npy"):
+        first, second = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert first.dtype in (np.float32, np.float64)
+        np.testing.assert_array_equal(first, second)
+    index = np.load(tmp_path / "a" / "sdf_sample_index.npy").astype(np.int64)
+    assert len(index) > sdf.numel() // 2 and np.all(np.diff(index) > 0)
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "sdf_sample.npy"),
+                                  sdf.numpy().reshape(-1)[index])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "sdf_min_max.npy"), min_max.numpy())
+    # sharded: every rank samples its own slab, rank 0 adds the global min/max
+    for rank in (0, 1):
+        bench.dump_outputs(tmp_path / "sharded", sdf, min_max, rank=rank, world=2)
+    assert sorted(path.name for path in (tmp_path / "sharded").iterdir()) == [
+        "sdf_min_max.npy", "sdf_sample_index_rank0.npy", "sdf_sample_index_rank1.npy",
+        "sdf_sample_rank0.npy", "sdf_sample_rank1.npy"]
+    for rank in (0, 1):
+        index = np.load(tmp_path / "sharded" / f"sdf_sample_index_rank{rank}.npy").astype(np.int64)
+        assert 0 < len(index) <= sdf.numel()
+        np.testing.assert_array_equal(np.load(tmp_path / "sharded" / f"sdf_sample_rank{rank}.npy"),
+                                      sdf.numpy().reshape(-1)[index])
