@@ -464,6 +464,36 @@ VGT_B200_API int vgt_b200_filter_dev(
     const int32_t* d_counts, int32_t num_grids, int64_t num_voxels,
     const vgt_b200_filter_options* filter, int device, float* d_occupancy, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Connected components of the component maps (topology)
+ * ------------------------------------------------------------------------------------------- */
+
+/* Replaces ComputeConnectedComponents (include/voxelized_geometry_tools/topology_computation.hpp:138-196)
+ * as OccupancyComponentMap and TaggedObjectOccupancyComponentMap call it: every cell's component
+ * word gets the number of its connected component, counted from 1 over the 6 face neighbours,
+ * component k being the one whose smallest linear index is the k-th smallest of all components'
+ * smallest indices (the order of the reference's scan). Two face neighbours are connected iff
+ *   cell_bytes 8  (OccupancyComponentCell, component = word 1):
+ *       (occupancy_a > 0.5) == (occupancy_b > 0.5)
+ *   cell_bytes 16 (TaggedObjectOccupancyComponentCell, component = word 2):
+ *       the same and object_id_a == object_id_b
+ * (so unknown cells, 0.5, and NaN join the free cells). Every other byte of every cell is left as
+ * it was. The result does not depend on thread timing.
+ *   cells               host, nx*ny*nz cells (GetMutableRawData().data()), modified in place
+ *   out_num_components  host; the number of components (the reference's return value)
+ * Grids of 2^32 cells or more fail with VGT_B200_ERR_UNSUPPORTED. */
+VGT_B200_API int vgt_b200_connected_components(
+    void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, int device,
+    uint32_t* out_num_components);
+
+/* The same on device-resident cells (ComputeConnectedComponents,
+ * topology_computation.hpp:138-196), asynchronous on `stream`; the count is written to device
+ * memory. Scratch comes from the device's stream-ordered pool: 4 bytes per cell plus about
+ * 0.25 bytes per cell for the ranks. d_cells must be 4-byte aligned. */
+VGT_B200_API int vgt_b200_connected_components_dev(
+    void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, int device,
+    uint32_t* d_num_components, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * On-disk formats (SURVEY.md section 8 f3): the reference's own grid files, so that results
  * computed here round-trip through

@@ -135,6 +135,8 @@ SIGNATURES = {
     "vgt_b200_rasterize_mesh_dev": (_int, [_vp, _i64, _vp, _i64, _vp, _int, _i64, _i64, _i64, _dbl,
                                            _f64p, _f64p, _int, _int, _vp, _vp]),
     "vgt_b200_rasterize_status": (_int, [_int]),
+    "vgt_b200_connected_components": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp]),
+    "vgt_b200_connected_components_dev": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp, _vp]),
     "vgt_b200_grid_file_save": (_int, [ctypes.c_char_p, _int, _int, _vp,
                                        ctypes.POINTER(GridFileInfo), ctypes.c_char_p]),
     "vgt_b200_grid_file_save_dev": (_int, [ctypes.c_char_p, _int, _int, _vp,

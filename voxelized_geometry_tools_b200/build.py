@@ -37,6 +37,8 @@ TRANSLATION_UNITS = [
     ("mesh_rasterizer.cu", ["-fmad=false"]),
     # the reference's file formats (host code; zlib for the compressed forms)
     ("grid_files.cu", []),
+    # connected components of the component maps (union-find labelling)
+    ("connected_components.cu", []),
 ]
 
 

@@ -158,6 +158,32 @@ def edt_final_pass(packed: torch.Tensor, y_offset: int, ny_total: int, resolutio
     return out, min_max
 
 
+def connected_components(cells: torch.Tensor,
+                         num_components: torch.Tensor | None = None) -> torch.Tensor:
+    """ComputeConnectedComponents (topology_computation.hpp:138-196) on device-resident component
+    map cells, in place: ``cells`` is a contiguous int32 or uint32 tensor [nx, ny, nz, words] with
+    2 words per cell (OccupancyComponentCell) or 4 (TaggedObjectOccupancyComponentCell), the
+    occupancy's float bits in word 0. The component word of every cell gets its component's
+    number; the other words are untouched. Returns the number of components as a uint32 device
+    tensor [1] (``num_components`` if given). Asynchronous."""
+    if not cells.is_cuda:
+        raise _capi.BackendUnavailable("cells must live on a CUDA device (no CPU fallback)")
+    if cells.dtype not in (torch.int32, torch.uint32) or not cells.is_contiguous():
+        raise ValueError("cells must be a contiguous int32 or uint32 tensor")
+    if cells.dim() != 4 or cells.shape[3] not in (2, 4):
+        raise ValueError("cells must be [nx, ny, nz, 2] or [nx, ny, nz, 4]")
+    device = cells.device
+    if num_components is None:
+        num_components = torch.empty(1, dtype=torch.uint32, device=device)
+    _require_cuda(num_components, torch.uint32, "num_components")
+    nx, ny, nz, words = cells.shape
+    code = _capi.library().vgt_b200_connected_components_dev(
+        cells.data_ptr(), 4 * words, nx, ny, nz, device.index or 0, num_components.data_ptr(),
+        _stream_handle(device))
+    _capi.check(code)
+    return num_components
+
+
 def raycast_cloud(points_xyz: torch.Tensor, x_gc, max_range: float, counts: torch.Tensor,
                   voxel_size: float) -> torch.Tensor:
     """Accumulates one cloud (float64 or float32 [N, 3], cloud frame) into counts int32

@@ -16,7 +16,8 @@ reference's own (paths relative to the reference checkout):
   tagged_object_occupancy_component_map.hpp:360-575.
 
 Only what the occupancy -> SDF path needs is here: storage, the filled predicate's inputs, the
-Extract entry points and Lock()/min-max. Queries, gradients and serialization are out of scope.
+Extract entry points and Lock()/min-max, plus ``UpdateConnectedComponents`` of the two component
+maps (topology_computation.hpp:138-196). Queries, gradients and serialization are out of scope.
 """
 from __future__ import annotations
 
@@ -401,6 +402,15 @@ class _CellGrid:
         _capi.check(code)
         return self._wrap(out, lo.value, hi.value, parameters)
 
+    def _connected_components(self, device):
+        _capi.require_device(device)
+        count = ctypes.c_uint32()
+        code = _capi.library().vgt_b200_connected_components(
+            self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape, device,
+            ctypes.byref(count))
+        _capi.check(code)
+        return int(count.value)
+
 
 def _scalar_suffix(dtype):
     if np.dtype(dtype) == np.float32:
@@ -424,6 +434,14 @@ class OccupancyComponentMap(_CellGrid):
 
     def ExtractSignedDistanceFieldDouble(self, parameters, device: int = 0):
         return self.ExtractSignedDistanceField(parameters, np.float64, device)
+
+    def UpdateConnectedComponents(self, device: int = 0) -> int:
+        """Labels the connected components of the map into every cell's ``component`` and returns
+        their number (ComputeConnectedComponents, topology_computation.hpp:138-196): face
+        neighbours are connected iff both are filled (> 0.5) or both are not; components are
+        numbered from 1 in the order of their first cell in storage order. Recomputed on every
+        call (nothing is cached)."""
+        return self._connected_components(device)
 
 
 class TaggedObjectOccupancyMap(_CellGrid):
@@ -490,6 +508,15 @@ class TaggedObjectOccupancyComponentMap(TaggedObjectOccupancyMap):
     spatial_segment}; the same SDF entry points (:360-575)."""
 
     CELL = TAGGED_OBJECT_OCCUPANCY_COMPONENT_CELL
+
+    def UpdateConnectedComponents(self, device: int = 0) -> int:
+        """Labels the connected components of the map into every cell's ``component`` and returns
+        their number (ComputeConnectedComponents, topology_computation.hpp:138-196): face
+        neighbours are connected iff both are filled (> 0.5) or both are not, and their object
+        ids are equal; components are numbered from 1 in the order of their first cell in storage
+        order. ``object_id`` and ``spatial_segment`` are left as they are. Recomputed on every
+        call (nothing is cached)."""
+        return self._connected_components(device)
 
 
 def ExtractSignedDistanceFieldFromMask(filled_mask: np.ndarray, origin_transform, frame: str,
