@@ -348,6 +348,47 @@ VGT_B200_API int vgt_b200_sdf_project_out_of_collision_dev(
 VGT_B200_API int vgt_b200_sdf_local_extrema_map_dev(
     const vgt_b200_sdf_view* sdf, int device, double* d_extrema_xyz, void* stream);
 
+/* A device-resident SignedDistanceField<double>: the grid vgt_b200_sdf_f64_dev (or a double
+ * ExtractSignedDistanceField entry) wrote, with the same fields as vgt_b200_sdf_view. */
+typedef struct vgt_b200_sdf_view_f64
+{
+  const double* d_sdf; /* device double[nx*ny*nz] */
+  int64_t nx;
+  int64_t ny;
+  int64_t nz;
+  double resolution;
+  double origin_transform[16];
+} vgt_b200_sdf_view_f64;
+
+/* The same five calls on a SignedDistanceField<double>, with the argument lists, outputs,
+ * statuses and limits of the float entries above. They replace the ScalarType = double
+ * instantiations of the same members (include/.../signed_distance_field.hpp:823-838,
+ * :887-1025, :1051-1092, :1159-1203, :1207-1231). A cell is read as a double and never rounded
+ * through float; where the reference computes in ScalarType, the interior gradient's difference
+ * of two neighbours (:932-943) and the sign test of the extrema walk (:494-534), that arithmetic
+ * is double. */
+VGT_B200_API int vgt_b200_sdf_estimate_distance_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points, int device,
+    double* d_distances, uint8_t* d_valid, void* stream);
+
+VGT_B200_API int vgt_b200_sdf_coarse_gradient_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points,
+    int enable_edge_gradients, int device, double* d_gradients_xyz, uint8_t* d_valid,
+    void* stream);
+
+VGT_B200_API int vgt_b200_sdf_fine_gradient_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points,
+    double nominal_window_size, int device, double* d_gradients_xyz, uint8_t* d_valid,
+    void* stream);
+
+VGT_B200_API int vgt_b200_sdf_project_out_of_collision_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points,
+    double minimum_distance, double stepsize_multiplier, int64_t max_steps, int device,
+    double* d_projected_xyz, uint8_t* d_valid, void* stream);
+
+VGT_B200_API int vgt_b200_sdf_local_extrema_map_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, int device, double* d_extrema_xyz, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Mesh rasterizer (an occupancy producer in front of the SDF path)
  * ------------------------------------------------------------------------------------------- */

@@ -48,6 +48,11 @@ class SdfView(ctypes.Structure):
                 ("resolution", _dbl), ("origin_transform", _dbl * 16)]
 
 
+class SdfViewF64(ctypes.Structure):
+    """struct vgt_b200_sdf_view_f64 (the same fields; d_sdf points at doubles)."""
+    _fields_ = SdfView._fields_
+
+
 class FilterOptions(ctypes.Structure):
     """struct vgt_b200_filter_options."""
     _fields_ = [("percent_seen_free", _dbl), ("outlier_points_threshold", ctypes.c_int32),
@@ -118,6 +123,16 @@ SIGNATURES = {
     "vgt_b200_sdf_local_extrema_map_dev": (_int, [ctypes.POINTER(SdfView), _int, _vp, _vp]),
     "vgt_b200_sdf_project_out_of_collision_dev": (_int, [ctypes.POINTER(SdfView), _vp, _i64, _dbl,
                                                          _dbl, _i64, _int, _vp, _vp, _vp]),
+    "vgt_b200_sdf_estimate_distance_f64_dev": (_int, [ctypes.POINTER(SdfViewF64), _vp, _i64, _int,
+                                                      _vp, _vp, _vp]),
+    "vgt_b200_sdf_coarse_gradient_f64_dev": (_int, [ctypes.POINTER(SdfViewF64), _vp, _i64, _int,
+                                                    _int, _vp, _vp, _vp]),
+    "vgt_b200_sdf_fine_gradient_f64_dev": (_int, [ctypes.POINTER(SdfViewF64), _vp, _i64, _dbl, _int,
+                                                  _vp, _vp, _vp]),
+    "vgt_b200_sdf_local_extrema_map_f64_dev": (_int, [ctypes.POINTER(SdfViewF64), _int, _vp, _vp]),
+    "vgt_b200_sdf_project_out_of_collision_f64_dev": (_int, [ctypes.POINTER(SdfViewF64), _vp, _i64,
+                                                             _dbl, _dbl, _i64, _int, _vp, _vp,
+                                                             _vp]),
     "vgt_b200_voxelize_f64": (_int, [_vp, _i64, _i64, _i64, _dbl, ctypes.POINTER(Cloud),
                                      ctypes.c_int32, ctypes.POINTER(FilterOptions), _int, _vp,
                                      _vp, _f64p]),

@@ -2,19 +2,22 @@
 // points: trilinear distance estimate, coarse and fine gradient, projection out of collision.
 // One thread per query point; the SDF stays where the generation pass left it.
 //
-// Replaces, per point, the reference's SignedDistanceField<float> members
-// (include/voxelized_geometry_tools/signed_distance_field.hpp):
+// Replaces, per point, the reference's SignedDistanceField<float> and SignedDistanceField<double>
+// members (include/voxelized_geometry_tools/signed_distance_field.hpp):
 //   EstimateLocationDistance4d            :823-838, :259-357 (interpolation helpers)
 //   GetLocationCoarseGradient4d           :887-900, :903-1025
 //   GetLocationFineGradient               :1051-1092, :213-255
 //   ProjectLocationOutOfCollisionToMinimumDistance4d :1159-1203
+// Every kernel that reads cells is a template on the stored ScalarType; the two instantiations
+// differ in two statements only, the interior gradient's subtraction and the sign test of the
+// extrema walk, both of which the reference evaluates in ScalarType.
 //
 // THIS TRANSLATION UNIT IS COMPILED WITH -fmad=false so that every expression below evaluates
 // as written (the numpy restatement the tests check against then matches bit for bit).
 // What is pinned by the reference's own source and what is not:
 //   * the coarse gradient, the axis index selection, the half-cell correction, the fine-gradient
 //     window logic and the projection loop are in-tree arithmetic and are mirrored operation by
-//     operation (including the float subtraction of the interior gradient, :932-943, against
+//     operation (including the ScalarType subtraction of the interior gradient, :932-943, against
 //     the double subtraction of the edge gradient, :977-1006);
 //   * the trilinear blend itself lives in common_robotics_utilities::math::TrilinearInterpolate,
 //     which is not in the reference tree (unvendored, unpinned dependency). It is restated here
@@ -32,9 +35,12 @@ namespace queries
 {
 namespace
 {
+// T = the SDF's ScalarType (float or double). A cell is read as T and widened to double where
+// the reference widens it; it never passes through float when T is double.
+template <typename T>
 struct SdfView
 {
-  const float* sdf;
+  const T* sdf;
   int64_t nx;
   int64_t ny;
   int64_t nz;
@@ -68,23 +74,27 @@ __device__ __forceinline__ Vec3 RotateVector(const double* m, const Vec3& v)
               ((m[2] * v.x + m[6] * v.y) + m[10] * v.z) + m[14] * 0.0};
 }
 
-__device__ __forceinline__ double Stored(const SdfView& v, int64_t x, int64_t y, int64_t z)
+template <typename T>
+__device__ __forceinline__ double Stored(const SdfView<T>& v, int64_t x, int64_t y, int64_t z)
 {
   return static_cast<double>(v.sdf[(x * v.ny + y) * v.nz + z]);
 }
 
-__device__ __forceinline__ float StoredFloat(const SdfView& v, int64_t x, int64_t y, int64_t z)
+template <typename T>
+__device__ __forceinline__ T StoredScalar(const SdfView<T>& v, int64_t x, int64_t y, int64_t z)
 {
   return v.sdf[(x * v.ny + y) * v.nz + z];
 }
 
-__device__ __forceinline__ bool InBounds(const SdfView& v, int64_t x, int64_t y, int64_t z)
+template <typename T>
+__device__ __forceinline__ bool InBounds(const SdfView<T>& v, int64_t x, int64_t y, int64_t z)
 {
   return x >= 0 && x < v.nx && y >= 0 && y < v.ny && z >= 0 && z < v.nz;
 }
 
 // LocationToGridIndex4d: grid-frame location and its cell.
-__device__ __forceinline__ void Locate(const SdfView& v, const Vec3& world, Vec3* grid,
+template <typename T>
+__device__ __forceinline__ void Locate(const SdfView<T>& v, const Vec3& world, Vec3* grid,
                                        int64_t* x, int64_t* y, int64_t* z)
 {
   *grid = TransformPoint(v.x_gw, world);
@@ -94,7 +104,8 @@ __device__ __forceinline__ void Locate(const SdfView& v, const Vec3& world, Vec3
 }
 
 // GetCorrectedCenterDistance (:259-273).
-__device__ __forceinline__ double CorrectedCenterDistance(const SdfView& v, int64_t x, int64_t y,
+template <typename T>
+__device__ __forceinline__ double CorrectedCenterDistance(const SdfView<T>& v, int64_t x, int64_t y,
                                                           int64_t z)
 {
   const double nominal = Stored(v, x, y, z);
@@ -149,7 +160,8 @@ __device__ __forceinline__ double AxisRatio(double query, double low, double hig
 }
 
 // EstimateLocationDistance4d (:823-838): false = the location is outside the grid.
-__device__ bool EstimateDistance(const SdfView& v, const Vec3& world, double* distance)
+template <typename T>
+__device__ bool EstimateDistance(const SdfView<T>& v, const Vec3& world, double* distance)
 {
   Vec3 q;
   int64_t ix, iy, iz;
@@ -192,7 +204,8 @@ __device__ bool EstimateDistance(const SdfView& v, const Vec3& world, double* di
 }
 
 // GetGridAlignedIndexCoarseGradient + the rotation into the world frame (:903-1025).
-__device__ bool CoarseGradientAtIndex(const SdfView& v, int64_t x, int64_t y, int64_t z,
+template <typename T>
+__device__ bool CoarseGradientAtIndex(const SdfView<T>& v, int64_t x, int64_t y, int64_t z,
                                       bool enable_edge_gradients, Vec3* gradient)
 {
   if (!InBounds(v, x, y, z))
@@ -202,13 +215,14 @@ __device__ bool CoarseGradientAtIndex(const SdfView& v, int64_t x, int64_t y, in
   Vec3 aligned;
   if (x > 0 && y > 0 && z > 0 && x < v.nx - 1 && y < v.ny - 1 && z < v.nz - 1)
   {
-    // (the difference of two ScalarType = float values is a float; then times a double)
+    // (the difference of two ScalarType values is a ScalarType -- a float subtraction for float,
+    // a double one for double; then times a double)
     const double inv_twice_resolution = 1.0 / (2.0 * v.resolution);
-    aligned.x = static_cast<double>(StoredFloat(v, x + 1, y, z) - StoredFloat(v, x - 1, y, z))
+    aligned.x = static_cast<double>(StoredScalar(v, x + 1, y, z) - StoredScalar(v, x - 1, y, z))
         * inv_twice_resolution;
-    aligned.y = static_cast<double>(StoredFloat(v, x, y + 1, z) - StoredFloat(v, x, y - 1, z))
+    aligned.y = static_cast<double>(StoredScalar(v, x, y + 1, z) - StoredScalar(v, x, y - 1, z))
         * inv_twice_resolution;
-    aligned.z = static_cast<double>(StoredFloat(v, x, y, z + 1) - StoredFloat(v, x, y, z - 1))
+    aligned.z = static_cast<double>(StoredScalar(v, x, y, z + 1) - StoredScalar(v, x, y, z - 1))
         * inv_twice_resolution;
   }
   else if (enable_edge_gradients)
@@ -244,7 +258,8 @@ __device__ bool CoarseGradientAtIndex(const SdfView& v, int64_t x, int64_t y, in
   return true;
 }
 
-__device__ bool CoarseGradientAtLocation(const SdfView& v, const Vec3& world,
+template <typename T>
+__device__ bool CoarseGradientAtLocation(const SdfView<T>& v, const Vec3& world,
                                          bool enable_edge_gradients, Vec3* gradient)
 {
   Vec3 q;
@@ -280,7 +295,8 @@ constexpr uint8_t kInvalid = 0;
 constexpr uint8_t kValid = 1;
 constexpr uint8_t kThrows = 2;   // where the reference throws std::runtime_error
 
-__global__ void EstimateDistanceKernel(SdfView view, const double* __restrict__ points,
+template <typename T>
+__global__ void EstimateDistanceKernel(SdfView<T> view, const double* __restrict__ points,
                                        int64_t count, double* __restrict__ distances,
                                        uint8_t* __restrict__ valid)
 {
@@ -296,7 +312,8 @@ __global__ void EstimateDistanceKernel(SdfView view, const double* __restrict__ 
   valid[i] = ok ? kValid : kInvalid;
 }
 
-__global__ void CoarseGradientKernel(SdfView view, const double* __restrict__ points,
+template <typename T>
+__global__ void CoarseGradientKernel(SdfView<T> view, const double* __restrict__ points,
                                      int64_t count, int enable_edge_gradients,
                                      double* __restrict__ gradients, uint8_t* __restrict__ valid)
 {
@@ -316,9 +333,10 @@ __global__ void CoarseGradientKernel(SdfView view, const double* __restrict__ po
 }
 
 // GetLocationFineGradient (:1051-1092).
-__global__ void FineGradientKernel(SdfView view, const double* __restrict__ points, int64_t count,
-                                   double nominal_window_size, double* __restrict__ gradients,
-                                   uint8_t* __restrict__ valid)
+template <typename T>
+__global__ void FineGradientKernel(SdfView<T> view, const double* __restrict__ points,
+                                   int64_t count, double nominal_window_size,
+                                   double* __restrict__ gradients, uint8_t* __restrict__ valid)
 {
   const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= count)
@@ -360,7 +378,8 @@ __global__ void FineGradientKernel(SdfView view, const double* __restrict__ poin
 // ProjectLocationOutOfCollisionToMinimumDistance4d (:1159-1203). The reference's loop has no
 // iteration bound; here a point that is still in collision after max_steps steps reports
 // kThrows (never seen with the default multiplier: a step is resolution / 10).
-__global__ void ProjectOutOfCollisionKernel(SdfView view, const double* __restrict__ points,
+template <typename T>
+__global__ void ProjectOutOfCollisionKernel(SdfView<T> view, const double* __restrict__ points,
                                             int64_t count, double minimum_distance,
                                             double stepsize_multiplier, int64_t max_steps,
                                             double* __restrict__ projected,
@@ -447,7 +466,8 @@ __global__ void ProjectOutOfCollisionKernel(SdfView view, const double* __restri
 // ------------------------------------------------------------------------------------------------
 constexpr uint32_t kOffGrid = 0xffffffffu;
 
-__global__ void ExtremaSuccessorKernel(SdfView view, uint32_t* __restrict__ successor)
+template <typename T>
+__global__ void ExtremaSuccessorKernel(SdfView<T> view, uint32_t* __restrict__ successor)
 {
   const int64_t cell = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const int64_t count = view.nx * view.ny * view.nz;
@@ -466,7 +486,7 @@ __global__ void ExtremaSuccessorKernel(SdfView view, uint32_t* __restrict__ succ
   const bool flat = fabs(gradient.x) <= step && fabs(gradient.y) <= step && fabs(gradient.z) <= step;
   if (!flat)
   {
-    if (StoredFloat(view, x, y, z) < 0.0f)
+    if (StoredScalar(view, x, y, z) < static_cast<T>(0))
     {
       gradient = Vec3{gradient.x * -1.0, gradient.y * -1.0, gradient.z * -1.0};
     }
@@ -561,7 +581,8 @@ __global__ void ExtremaEntryKernel(const uint32_t* __restrict__ successor,
   }
 }
 
-__global__ void ExtremaWriteKernel(SdfView view, const uint32_t* __restrict__ successor,
+template <typename T>
+__global__ void ExtremaWriteKernel(SdfView<T> view, const uint32_t* __restrict__ successor,
                                    const uint32_t* __restrict__ target,
                                    const uint32_t* __restrict__ lowest,
                                    const uint32_t* __restrict__ entry,
@@ -625,7 +646,10 @@ void InverseRigid(const double* m, double* out)
   }
 }
 
-int MakeView(const vgt_b200_sdf_view* sdf, SdfView* view)
+// CView = vgt_b200_sdf_view (float) or vgt_b200_sdf_view_f64 (double); its d_sdf must be a
+// const T*.
+template <typename CView, typename T>
+int MakeView(const CView* sdf, SdfView<T>* view)
 {
   if (sdf == nullptr || sdf->d_sdf == nullptr)
   {
@@ -668,20 +692,13 @@ int CheckBatch(const void* points, int64_t count, const void* out, const void* v
 
 constexpr int kThreads = 128;
 inline unsigned Blocks(int64_t count) { return static_cast<unsigned>((count + kThreads - 1) / kThreads); }
-}  // namespace
-}  // namespace queries
-}  // namespace vgt_b200
 
-using namespace vgt_b200;
-using namespace vgt_b200::queries;
-
-extern "C"
+// The bodies of the C-ABI entries, one per query; T is the SDF's ScalarType.
+template <typename T, typename CView>
+int EstimateDistanceEntry(const CView* sdf, const double* d_points_xyz, int64_t num_points,
+                          int device, double* d_distances, uint8_t* d_valid, void* stream)
 {
-int vgt_b200_sdf_estimate_distance_dev(
-    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points, int device,
-    double* d_distances, uint8_t* d_valid, void* stream)
-{
-  SdfView view;
+  SdfView<T> view;
   int status = MakeView(sdf, &view);
   if (status == VGT_B200_OK)
   {
@@ -699,11 +716,12 @@ int vgt_b200_sdf_estimate_distance_dev(
   return VGT_B200_OK;
 }
 
-int vgt_b200_sdf_coarse_gradient_dev(
-    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points,
-    int enable_edge_gradients, int device, double* d_gradients_xyz, uint8_t* d_valid, void* stream)
+template <typename T, typename CView>
+int CoarseGradientEntry(const CView* sdf, const double* d_points_xyz, int64_t num_points,
+                        int enable_edge_gradients, int device, double* d_gradients_xyz,
+                        uint8_t* d_valid, void* stream)
 {
-  SdfView view;
+  SdfView<T> view;
   int status = MakeView(sdf, &view);
   if (status == VGT_B200_OK)
   {
@@ -721,12 +739,12 @@ int vgt_b200_sdf_coarse_gradient_dev(
   return VGT_B200_OK;
 }
 
-int vgt_b200_sdf_fine_gradient_dev(
-    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points,
-    double nominal_window_size, int device, double* d_gradients_xyz, uint8_t* d_valid,
-    void* stream)
+template <typename T, typename CView>
+int FineGradientEntry(const CView* sdf, const double* d_points_xyz, int64_t num_points,
+                      double nominal_window_size, int device, double* d_gradients_xyz,
+                      uint8_t* d_valid, void* stream)
 {
-  SdfView view;
+  SdfView<T> view;
   int status = MakeView(sdf, &view);
   if (status == VGT_B200_OK)
   {
@@ -744,10 +762,10 @@ int vgt_b200_sdf_fine_gradient_dev(
   return VGT_B200_OK;
 }
 
-int vgt_b200_sdf_local_extrema_map_dev(
-    const vgt_b200_sdf_view* sdf, int device, double* d_extrema_xyz, void* stream)
+template <typename T, typename CView>
+int LocalExtremaMapEntry(const CView* sdf, int device, double* d_extrema_xyz, void* stream)
 {
-  SdfView view;
+  SdfView<T> view;
   const int status = MakeView(sdf, &view);
   if (status != VGT_B200_OK)
   {
@@ -812,12 +830,13 @@ int vgt_b200_sdf_local_extrema_map_dev(
   return VGT_B200_OK;
 }
 
-int vgt_b200_sdf_project_out_of_collision_dev(
-    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points,
-    double minimum_distance, double stepsize_multiplier, int64_t max_steps, int device,
-    double* d_projected_xyz, uint8_t* d_valid, void* stream)
+template <typename T, typename CView>
+int ProjectOutOfCollisionEntry(const CView* sdf, const double* d_points_xyz,
+                               int64_t num_points, double minimum_distance,
+                               double stepsize_multiplier, int64_t max_steps, int device,
+                               double* d_projected_xyz, uint8_t* d_valid, void* stream)
 {
-  SdfView view;
+  SdfView<T> view;
   int status = MakeView(sdf, &view);
   if (status == VGT_B200_OK)
   {
@@ -839,5 +858,98 @@ int vgt_b200_sdf_project_out_of_collision_dev(
       d_projected_xyz, d_valid); NoteKernelLaunch();
   VGT_CUDA_TRY(cudaGetLastError(), "ProjectOutOfCollisionKernel launch");
   return VGT_B200_OK;
+}
+}  // namespace
+}  // namespace queries
+}  // namespace vgt_b200
+
+using namespace vgt_b200;
+
+extern "C"
+{
+int vgt_b200_sdf_estimate_distance_dev(
+    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points, int device,
+    double* d_distances, uint8_t* d_valid, void* stream)
+{
+  return queries::EstimateDistanceEntry<float>(sdf, d_points_xyz, num_points, device,
+                                               d_distances, d_valid, stream);
+}
+
+int vgt_b200_sdf_estimate_distance_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points, int device,
+    double* d_distances, uint8_t* d_valid, void* stream)
+{
+  return queries::EstimateDistanceEntry<double>(sdf, d_points_xyz, num_points, device,
+                                                d_distances, d_valid, stream);
+}
+
+int vgt_b200_sdf_coarse_gradient_dev(
+    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points,
+    int enable_edge_gradients, int device, double* d_gradients_xyz, uint8_t* d_valid, void* stream)
+{
+  return queries::CoarseGradientEntry<float>(sdf, d_points_xyz, num_points,
+                                             enable_edge_gradients, device, d_gradients_xyz,
+                                             d_valid, stream);
+}
+
+int vgt_b200_sdf_coarse_gradient_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points,
+    int enable_edge_gradients, int device, double* d_gradients_xyz, uint8_t* d_valid, void* stream)
+{
+  return queries::CoarseGradientEntry<double>(sdf, d_points_xyz, num_points,
+                                              enable_edge_gradients, device, d_gradients_xyz,
+                                              d_valid, stream);
+}
+
+int vgt_b200_sdf_fine_gradient_dev(
+    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points,
+    double nominal_window_size, int device, double* d_gradients_xyz, uint8_t* d_valid,
+    void* stream)
+{
+  return queries::FineGradientEntry<float>(sdf, d_points_xyz, num_points, nominal_window_size,
+                                           device, d_gradients_xyz, d_valid, stream);
+}
+
+int vgt_b200_sdf_fine_gradient_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points,
+    double nominal_window_size, int device, double* d_gradients_xyz, uint8_t* d_valid,
+    void* stream)
+{
+  return queries::FineGradientEntry<double>(sdf, d_points_xyz, num_points, nominal_window_size,
+                                            device, d_gradients_xyz, d_valid, stream);
+}
+
+int vgt_b200_sdf_local_extrema_map_dev(
+    const vgt_b200_sdf_view* sdf, int device, double* d_extrema_xyz, void* stream)
+{
+  return queries::LocalExtremaMapEntry<float>(sdf, device, d_extrema_xyz, stream);
+}
+
+int vgt_b200_sdf_local_extrema_map_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, int device, double* d_extrema_xyz, void* stream)
+{
+  return queries::LocalExtremaMapEntry<double>(sdf, device, d_extrema_xyz, stream);
+}
+
+int vgt_b200_sdf_project_out_of_collision_dev(
+    const vgt_b200_sdf_view* sdf, const double* d_points_xyz, int64_t num_points,
+    double minimum_distance, double stepsize_multiplier, int64_t max_steps, int device,
+    double* d_projected_xyz, uint8_t* d_valid, void* stream)
+{
+  return queries::ProjectOutOfCollisionEntry<float>(sdf, d_points_xyz, num_points,
+                                                    minimum_distance, stepsize_multiplier,
+                                                    max_steps, device, d_projected_xyz, d_valid,
+                                                    stream);
+}
+
+int vgt_b200_sdf_project_out_of_collision_f64_dev(
+    const vgt_b200_sdf_view_f64* sdf, const double* d_points_xyz, int64_t num_points,
+    double minimum_distance, double stepsize_multiplier, int64_t max_steps, int device,
+    double* d_projected_xyz, uint8_t* d_valid, void* stream)
+{
+  return queries::ProjectOutOfCollisionEntry<double>(sdf, d_points_xyz, num_points,
+                                                     minimum_distance, stepsize_multiplier,
+                                                     max_steps, device, d_projected_xyz, d_valid,
+                                                     stream);
 }
 }  // extern "C"

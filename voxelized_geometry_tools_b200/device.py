@@ -225,23 +225,31 @@ def filter_grids(counts: torch.Tensor, occupancy: torch.Tensor,
 # --------------------------------------------------------------------------------------------------
 QUERY_NO_VALUE, QUERY_VALUE, QUERY_THROWS = 0, 1, 2
 
+# SDF dtype -> (C view struct, suffix of the C-ABI entry names)
+_SDF_SCALAR_TYPES = {torch.float32: (_capi.SdfView, "_dev"),
+                     torch.float64: (_capi.SdfViewF64, "_f64_dev")}
+
 
 class DeviceSignedDistanceField:
-    """A SignedDistanceField<float> that stays on the GPU: the float grid [nx, ny, nz] plus
-    resolution and origin transform. The batched queries mirror the reference's per-point
-    members (signed_distance_field.hpp:808-1203); points are float64 [N, 3] CUDA tensors in the
-    WORLD frame. Every query returns (values, valid uint8): 1 = value, 0 = the reference returns
-    an empty query, 2 = the reference throws for that point."""
+    """A SignedDistanceField<float> or SignedDistanceField<double> that stays on the GPU: the
+    float32 or float64 grid [nx, ny, nz] plus resolution and origin transform. The batched
+    queries mirror the reference's per-point members (signed_distance_field.hpp:808-1203) for
+    the grid's scalar type; points are float64 [N, 3] CUDA tensors in the WORLD frame. Every
+    query returns (values, valid uint8): 1 = value, 0 = the reference returns an empty query,
+    2 = the reference throws for that point."""
 
     def __init__(self, sdf: torch.Tensor, resolution: float, origin_transform=None):
-        _require_cuda(sdf, torch.float32, "sdf")
+        if sdf.dtype not in _SDF_SCALAR_TYPES:
+            raise ValueError(f"sdf must be a float32 or float64 tensor, not {sdf.dtype}")
+        _require_cuda(sdf, sdf.dtype, "sdf")
         if sdf.dim() != 3:
             raise ValueError("sdf must be indexed [x, y, z]")
         self.sdf = sdf
         self.resolution = float(resolution)
         self.origin_transform = np.eye(4) if origin_transform is None else \
             np.asarray(origin_transform, dtype=np.float64).reshape(4, 4)
-        self._view = _capi.SdfView()
+        view_type, self._entry_suffix = _SDF_SCALAR_TYPES[sdf.dtype]
+        self._view = view_type()
         self._view.d_sdf = sdf.data_ptr()
         self._view.nx, self._view.ny, self._view.nz = (int(d) for d in sdf.shape)
         self._view.resolution = self.resolution
@@ -264,7 +272,7 @@ class DeviceSignedDistanceField:
         shape = (count,) if width == 1 else (count, width)
         values = torch.empty(shape, dtype=torch.float64, device=device)
         valid = torch.empty(count, dtype=torch.uint8, device=device)
-        function = getattr(_capi.library(), name)
+        function = getattr(_capi.library(), name + self._entry_suffix)
         code = function(ctypes.byref(self._view), points.data_ptr(), count, *middle,
                         device.index or 0, values.data_ptr(), valid.data_ptr(),
                         _stream_handle(device))
@@ -272,20 +280,20 @@ class DeviceSignedDistanceField:
         return values, valid
 
     def EstimateLocationDistance(self, points: torch.Tensor):
-        return self._launch("vgt_b200_sdf_estimate_distance_dev", points, 1)
+        return self._launch("vgt_b200_sdf_estimate_distance", points, 1)
 
     def GetLocationCoarseGradient(self, points: torch.Tensor, enable_edge_gradients=False):
-        return self._launch("vgt_b200_sdf_coarse_gradient_dev", points, 3,
+        return self._launch("vgt_b200_sdf_coarse_gradient", points, 3,
                             int(bool(enable_edge_gradients)))
 
     def GetLocationFineGradient(self, points: torch.Tensor, nominal_window_size: float):
-        return self._launch("vgt_b200_sdf_fine_gradient_dev", points, 3,
+        return self._launch("vgt_b200_sdf_fine_gradient", points, 3,
                             float(nominal_window_size))
 
     def ProjectLocationOutOfCollisionToMinimumDistance(
             self, points: torch.Tensor, minimum_distance: float = 0.0,
             stepsize_multiplier: float = 1.0 / 10.0, max_steps: int = 1_000_000):
-        return self._launch("vgt_b200_sdf_project_out_of_collision_dev", points, 3,
+        return self._launch("vgt_b200_sdf_project_out_of_collision", points, 3,
                             float(minimum_distance), float(stepsize_multiplier), int(max_steps))
 
     def ProjectLocationOutOfCollision(self, points: torch.Tensor,
@@ -298,8 +306,8 @@ class DeviceSignedDistanceField:
         ends at, +inf when it leaves the grid (signed_distance_field.hpp:1207-1231)."""
         device = self.sdf.device
         extrema = torch.empty(tuple(self.sdf.shape) + (3,), dtype=torch.float64, device=device)
-        code = _capi.library().vgt_b200_sdf_local_extrema_map_dev(
-            ctypes.byref(self._view), device.index or 0, extrema.data_ptr(),
-            _stream_handle(device))
+        function = getattr(_capi.library(), "vgt_b200_sdf_local_extrema_map" + self._entry_suffix)
+        code = function(ctypes.byref(self._view), device.index or 0, extrema.data_ptr(),
+                        _stream_handle(device))
         _capi.check(code)
         return extrema
