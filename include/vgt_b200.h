@@ -535,6 +535,22 @@ VGT_B200_API int vgt_b200_connected_components_dev(
     void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, int device,
     uint32_t* d_num_components, void* stream);
 
+/* vgt_b200_connected_components (ComputeConnectedComponents, topology_computation.hpp:138-196)
+ * on the map cut into num_slabs x-slabs (the cut of vgt_b200_sdf_f32_multi), slab g on
+ * devices[g]; a device may be listed more than once, so one device labels a map of 2^32 cells or
+ * more when its memory allows. The same bytes and count as vgt_b200_connected_components on every
+ * map that entry accepts. Each slab is labelled on its own, the edges across the x-faces between
+ * slabs are resolved on devices[0], and every slab then writes the reference's numbers.
+ *   1 <= num_slabs <= 8, num_slabs <= nx; num_slabs == 1 is vgt_b200_connected_components.
+ *   Device memory, per slab on its device: the slab's cells + 4 B per cell + about 0.25 B per
+ *   cell + about 4.25 B per component local to the slab; on devices[0] in addition up to 64 B per
+ *   face edge, at most (num_slabs - 1) * ny * nz edges.
+ * Slabs of 2^32 cells or more fail with VGT_B200_ERR_UNSUPPORTED before any device call, and so
+ * does a map of more than 0xFFFFFFFF components, before any cell is written (cells unchanged). */
+VGT_B200_API int vgt_b200_connected_components_multi(
+    void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, const int* devices,
+    int num_slabs, uint32_t* out_num_components);
+
 /* ------------------------------------------------------------------------------------------------
  * On-disk formats (SURVEY.md section 8 f3): the reference's own grid files, so that results
  * computed here round-trip through

@@ -152,6 +152,7 @@ SIGNATURES = {
     "vgt_b200_rasterize_status": (_int, [_int]),
     "vgt_b200_connected_components": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp]),
     "vgt_b200_connected_components_dev": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp, _vp]),
+    "vgt_b200_connected_components_multi": (_int, [_vp, _int, _i64, _i64, _i64, _vp, _int, _vp]),
     "vgt_b200_grid_file_save": (_int, [ctypes.c_char_p, _int, _int, _vp,
                                        ctypes.POINTER(GridFileInfo), ctypes.c_char_p]),
     "vgt_b200_grid_file_save_dev": (_int, [ctypes.c_char_p, _int, _int, _vp,

@@ -4,6 +4,8 @@
 
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <condition_variable>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
@@ -132,11 +134,61 @@ private:
   cudaStream_t stream_ = nullptr;
 };
 
+// Owns a stream created by the entry point (destroyed on scope exit).
+struct StreamGuard
+{
+  cudaStream_t stream = nullptr;
+  ~StreamGuard()
+  {
+    if (stream != nullptr)
+    {
+      cudaStreamDestroy(stream);
+    }
+  }
+};
+
 inline bool ValidDims(int64_t nx, int64_t ny, int64_t nz)
 {
   return nx >= 1 && ny >= 1 && nz >= 1 && nx <= VGT_B200_MAX_AXIS && ny <= VGT_B200_MAX_AXIS
       && nz <= VGT_B200_MAX_AXIS;
 }
+
+// Part `index` of `total` items cut into `parts` near-equal parts (the first total % parts
+// parts get one extra item): the x-slabs of the multi-device entries.
+inline void SplitRange(int64_t total, int parts, int index, int64_t* begin, int64_t* end)
+{
+  const int64_t base = total / parts;
+  const int64_t extra = total % parts;
+  *begin = index * base + std::min<int64_t>(index, extra);
+  *end = *begin + base + (index < extra ? 1 : 0);
+}
+
+// A reusable barrier for the per-device host threads (std::barrier is C++20).
+class ThreadBarrier
+{
+public:
+  explicit ThreadBarrier(int count) : count_(count), waiting_(0), generation_(0) {}
+  void Wait()
+  {
+    std::unique_lock<std::mutex> lock(mutex_);
+    const int generation = generation_;
+    if (++waiting_ == count_)
+    {
+      waiting_ = 0;
+      generation_++;
+      released_.notify_all();
+      return;
+    }
+    released_.wait(lock, [&] { return generation != generation_; });
+  }
+
+private:
+  std::mutex mutex_;
+  std::condition_variable released_;
+  int count_;
+  int waiting_;
+  int generation_;
+};
 }  // namespace vgt_b200
 
 #define VGT_CUDA_TRY(expr, what)                           \

@@ -19,7 +19,15 @@
 //                          new component word; every other word is copied as it was read
 // Scratch, stream-ordered: 4 B per cell (parent) + 1 bit per cell (root mask) + 4 B per 32 cells
 // (word counts / prefix) + the scan's temporary storage.
+#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+
+#include <atomic>
+#include <functional>
+#include <string>
+#include <thread>
+#include <vector>
 
 #include "common.cuh"
 #include "host_transfer.cuh"
@@ -370,6 +378,876 @@ int Launch(void* d_cells, int cell_bytes, const Grid& grid, uint32_t* d_num_comp
   }
   return LaunchAll<4>(static_cast<uint32_t*>(d_cells), grid, d_num_components, stream);
 }
+
+// =============================================================================================
+// The map cut into x-slabs (vgt_b200_connected_components_multi). Slab g = planes [x0_g, x1_g)
+// (SplitRange) on devices[g] is labelled by steps 1-4 above as a grid of its own, with 32-bit
+// local indices; local index l of slab g is global index x0_g * ny * nz + l (64 bits). Because a
+// slab is one contiguous range of storage order and every local root is the smallest index of
+// its local set, the smallest index of a component is a local root in the lowest slab it
+// touches, and only the cells of the x-faces between slabs can join local sets of different
+// slabs. So:
+//   a. per face, FaceEdgesKernel emits (global root of the cell below, global root of the cell
+//      above) where the keys are equal and the edge is not implied by the (y, z - 1) pair;
+//   b. on devices[0] the endpoints are sorted and made unique (the nodes), the edges are mapped
+//      to compact node ids by binary search and joined by union-find with parent <= self;
+//      compact order is global order, so a node's compact root is the smallest global index of
+//      its merged set;
+//   c. per slab, one bit per local component, cleared for the slab's nodes whose compact root is
+//      another node; the bits left are the components whose smallest index lies in the slab,
+//      count_g of them, and component ids are offset_g + 1 + rank among them (offset_g = the
+//      sum of the counts of the slabs below): the reference's numbering;
+//   d. root nodes publish their id to devices[0], every node takes the id of its compact root,
+//      and each slab writes final[local rank] into the component word of its cells.
+// Everything that crosses slabs (face planes and roots, edges, node tables) goes through host
+// memory: it is O(num_slabs * ny * nz).
+// Scratch per slab, on its device: the slab's cells + 4 B per cell (parent) + about 0.25 B per
+// cell (root mask, word prefix) + 4 B per local component (final ids) + about 0.25 B per local
+// component (root bits, word prefix), + O(ny * nz) for the faces and the slab's nodes. On
+// devices[0] in addition, E = at most (num_slabs - 1) * ny * nz edges: at most 64 B per edge
+// (the edges, their sorted endpoints, the nodes, their parents and compact roots).
+// =============================================================================================
+struct Edge
+{
+  uint64_t a, b;  // global indices of two local roots, a in the slab below
+};
+
+// Rank of local root r among the slab's local roots (step 3's mask and step 4's prefix).
+__device__ __forceinline__ uint32_t RootRank(const uint32_t* __restrict__ mask,
+                                             const uint32_t* __restrict__ word_prefix, uint32_t r)
+{
+  const uint32_t below = __ldg(mask + (r >> 5)) & ((1u << (r & 31)) - 1u);
+  return __ldg(word_prefix + (r >> 5)) + static_cast<uint32_t>(__popc(below));
+}
+
+// The local root of each cell of the slab's last x-plane (first = its first local index).
+__global__ void __launch_bounds__(kThreads)
+FaceRootsKernel(uint32_t* parent, uint32_t first, uint32_t plane, uint32_t* __restrict__ roots)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < plane)
+  {
+    roots[k] = Find(parent, first + k);
+  }
+}
+
+// Step a, on the slab above the face: below_cells / below_roots are the last plane of the slab
+// below (its cells and their local roots), cells / parent the slab's own (its first plane is
+// local 0 .. plane - 1). The edge of (y, z) is implied when (y, z - 1) has the same key on both
+// sides: each cell is in its z-neighbour's local set, and (y, z - 1) is joined or implied itself.
+template <int kCellWords>
+__global__ void __launch_bounds__(kThreads)
+FaceEdgesKernel(const uint32_t* __restrict__ below_cells, const uint32_t* __restrict__ below_roots,
+                uint64_t below_base, const uint32_t* __restrict__ cells, uint32_t* parent,
+                uint64_t base, uint32_t plane, uint32_t nz, Edge* __restrict__ edges,
+                uint32_t* __restrict__ edge_count)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  bool emit = false;
+  if (k < plane)
+  {
+    const Key key = CellKey<kCellWords>(cells, k);
+    emit = CellKey<kCellWords>(below_cells, k) == key
+        && !((k % nz) != 0 && CellKey<kCellWords>(cells, k - 1) == key
+             && CellKey<kCellWords>(below_cells, k - 1) == key);
+  }
+  const uint32_t ballot = __ballot_sync(0xffffffffu, emit);
+  if (ballot == 0u)
+  {
+    return;
+  }
+  const int lane = threadIdx.x & 31;
+  uint32_t slot = 0;
+  if (lane == __ffs(ballot) - 1)
+  {
+    slot = atomicAdd(edge_count, static_cast<uint32_t>(__popc(ballot)));
+  }
+  slot = __shfl_sync(0xffffffffu, slot, __ffs(ballot) - 1);
+  if (emit)
+  {
+    slot += static_cast<uint32_t>(__popc(ballot & ((1u << lane) - 1u)));
+    edges[slot] = Edge{below_base + __ldg(below_roots + k), base + Find(parent, k)};
+  }
+}
+
+// Step b: the first index of sorted[0, n) that is >= value.
+__device__ __forceinline__ uint32_t LowerBound(const uint64_t* __restrict__ sorted, uint32_t n,
+                                               uint64_t value)
+{
+  uint32_t lo = 0;
+  uint32_t hi = n;
+  while (lo < hi)
+  {
+    const uint32_t mid = lo + (hi - lo) / 2;
+    if (__ldg(sorted + mid) < value)
+    {
+      lo = mid + 1;
+    }
+    else
+    {
+      hi = mid;
+    }
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(kThreads)
+NodeInitKernel(uint32_t* __restrict__ node_parent, uint32_t num_nodes)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < num_nodes)
+  {
+    node_parent[k] = k;
+  }
+}
+
+__global__ void __launch_bounds__(kThreads)
+NodeUnionKernel(const Edge* __restrict__ edges, uint32_t num_edges,
+                const uint64_t* __restrict__ nodes, uint32_t num_nodes, uint32_t* node_parent)
+{
+  const uint32_t e = blockIdx.x * kThreads + threadIdx.x;
+  if (e < num_edges)
+  {
+    const Edge edge = edges[e];
+    Union(node_parent, LowerBound(nodes, num_nodes, edge.a), LowerBound(nodes, num_nodes, edge.b));
+  }
+}
+
+// node_roots[k] = compact root of k (a separate array: a store into node_parent could be
+// overwritten by another thread's path halving), and where each slab's nodes begin:
+// slab_first[g] = the first node >= slab_base[g] (num_slabs + 1 entries; the last base is the
+// grid's cell count).
+__global__ void __launch_bounds__(kThreads)
+NodeFlattenKernel(uint32_t* node_parent, const uint64_t* __restrict__ nodes, uint32_t num_nodes,
+                  const uint64_t* __restrict__ slab_base, int num_bases,
+                  uint32_t* __restrict__ node_roots, uint32_t* __restrict__ slab_first)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < num_nodes)
+  {
+    node_roots[k] = Find(node_parent, k);
+  }
+  if (k < static_cast<uint32_t>(num_bases))
+  {
+    slab_first[k] = LowerBound(nodes, num_nodes, slab_base[k]);
+  }
+}
+
+// Step c: one bit per local component, set for all but the last word's padding.
+__global__ void __launch_bounds__(kThreads)
+GlobalRootBitsInitKernel(uint32_t* __restrict__ bits, uint32_t num_components)
+{
+  const uint32_t w = blockIdx.x * kThreads + threadIdx.x;
+  if (w < (num_components + 31) / 32)
+  {
+    const uint32_t left = num_components - w * 32;
+    bits[w] = left >= 32 ? 0xffffffffu : ((1u << left) - 1u);
+  }
+}
+
+// Nodes k of the slab (node_first + k in compact ids) whose compact root is another node are not
+// global roots: their bit is cleared.
+__global__ void __launch_bounds__(kThreads)
+ClearMergedBitsKernel(const uint64_t* __restrict__ nodes, const uint32_t* __restrict__ node_roots,
+                      uint32_t count, uint32_t node_first, uint64_t base,
+                      const uint32_t* __restrict__ mask, const uint32_t* __restrict__ word_prefix,
+                      uint32_t* bits)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < count && node_roots[k] != node_first + k)
+  {
+    const uint32_t rank = RootRank(mask, word_prefix, static_cast<uint32_t>(nodes[k] - base));
+    atomicAnd(bits + (rank >> 5), ~(1u << (rank & 31)));
+  }
+}
+
+__global__ void __launch_bounds__(kThreads)
+BitCountsKernel(const uint32_t* __restrict__ bits, uint32_t words, uint32_t* __restrict__ counts)
+{
+  const uint32_t w = blockIdx.x * kThreads + threadIdx.x;
+  if (w < words)
+  {
+    counts[w] = static_cast<uint32_t>(__popc(bits[w]));
+  }
+}
+
+// Step d: final[r] = offset + 1 + rank among the slab's global roots, 0 for merged components
+// (overwritten by ApplyNodeIdsKernel).
+__global__ void __launch_bounds__(kThreads)
+FinalIdsKernel(const uint32_t* __restrict__ bits, const uint32_t* __restrict__ bit_prefix,
+               uint32_t num_components, uint32_t offset, uint32_t* __restrict__ final_ids)
+{
+  const uint32_t r = blockIdx.x * kThreads + threadIdx.x;
+  if (r < num_components)
+  {
+    const uint32_t word = __ldg(bits + (r >> 5));
+    final_ids[r] = ((word >> (r & 31)) & 1u) == 0u
+                 ? 0u
+                 : offset + 1u + __ldg(bit_prefix + (r >> 5))
+                       + static_cast<uint32_t>(__popc(word & ((1u << (r & 31)) - 1u)));
+  }
+}
+
+// ids[k] = final[local rank of node k]: the published id of each root node of the slab.
+__global__ void __launch_bounds__(kThreads)
+PublishNodeIdsKernel(const uint64_t* __restrict__ nodes, uint32_t count, uint64_t base,
+                     const uint32_t* __restrict__ mask, const uint32_t* __restrict__ word_prefix,
+                     const uint32_t* __restrict__ final_ids, uint32_t* __restrict__ ids)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < count)
+  {
+    ids[k] = final_ids[RootRank(mask, word_prefix, static_cast<uint32_t>(nodes[k] - base))];
+  }
+}
+
+// On devices[0]: every node takes the id its compact root published (roots keep theirs).
+__global__ void __launch_bounds__(kThreads)
+NodeIdsFromRootsKernel(const uint32_t* __restrict__ node_roots, uint32_t num_nodes, uint32_t* ids)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < num_nodes && node_roots[k] != k)
+  {
+    ids[k] = ids[node_roots[k]];
+  }
+}
+
+__global__ void __launch_bounds__(kThreads)
+ApplyNodeIdsKernel(const uint64_t* __restrict__ nodes, const uint32_t* __restrict__ ids,
+                   uint32_t count, uint64_t base, const uint32_t* __restrict__ mask,
+                   const uint32_t* __restrict__ word_prefix, uint32_t* __restrict__ final_ids)
+{
+  const uint32_t k = blockIdx.x * kThreads + threadIdx.x;
+  if (k < count)
+  {
+    final_ids[RootRank(mask, word_prefix, static_cast<uint32_t>(nodes[k] - base))] = ids[k];
+  }
+}
+
+// Step 5 of a slab: the component word = final[local rank of the cell's local root]; the other
+// words are copied as read.
+template <int kCellWords>
+__global__ void __launch_bounds__(kThreads)
+WriteSlabComponentsKernel(uint32_t* __restrict__ cells, uint32_t count, uint32_t* parent,
+                          const uint32_t* __restrict__ mask,
+                          const uint32_t* __restrict__ word_prefix,
+                          const uint32_t* __restrict__ final_ids)
+{
+  const uint32_t i = blockIdx.x * kThreads + threadIdx.x;
+  if (i >= count)
+  {
+    return;
+  }
+  const uint32_t component = __ldg(final_ids + RootRank(mask, word_prefix, Find(parent, i)));
+  uint32_t* cell = cells + static_cast<size_t>(i) * kCellWords;
+  uint32_t words[kCellWords];
+#pragma unroll
+  for (int w = 0; w < kCellWords; w++)
+  {
+    words[w] = __ldcs(cell + w);
+  }
+  words[kComponentWord<kCellWords>] = component;
+#pragma unroll
+  for (int w = 0; w < kCellWords; w++)
+  {
+    __stcs(cell + w, words[w]);
+  }
+}
+
+inline uint32_t Blocks(uint64_t threads)
+{
+  return static_cast<uint32_t>((threads + kThreads - 1) / kThreads);
+}
+
+#define VGT_LAUNCHED(what)                                  \
+  do                                                        \
+  {                                                         \
+    NoteKernelLaunch();                                     \
+    VGT_CUDA_TRY(cudaGetLastError(), what " launch");       \
+  } while (0)
+
+// Every check of vgt_b200_connected_components_multi, before any device call.
+int CheckMultiArguments(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                        const int* devices, int num_slabs, const void* num_components)
+{
+  if (cells == nullptr)
+  {
+    return FailInvalid("null cell array");
+  }
+  if (devices == nullptr)
+  {
+    return FailInvalid("null device list");
+  }
+  if (num_components == nullptr)
+  {
+    return FailInvalid("null component count");
+  }
+  if (num_slabs < 1 || num_slabs > 8)
+  {
+    return FailInvalid("1..8 slabs are supported (%d requested)", num_slabs);
+  }
+  if (cell_bytes != 8 && cell_bytes != 16)
+  {
+    return FailInvalid("cell size must be 8 (OccupancyComponentCell) or 16 "
+                       "(TaggedObjectOccupancyComponentCell) bytes");
+  }
+  if (!ValidDims(nx, ny, nz))
+  {
+    return FailInvalid("grid dimensions %lld x %lld x %lld out of range",
+                       static_cast<long long>(nx), static_cast<long long>(ny),
+                       static_cast<long long>(nz));
+  }
+  if (num_slabs > nx)
+  {
+    return FailInvalid("more slabs (%d) than x-planes (%lld)", num_slabs,
+                       static_cast<long long>(nx));
+  }
+  for (int g = 0; g < num_slabs; g++)
+  {
+    if (devices[g] < 0)
+    {
+      return FailInvalid("device ordinal %d out of range", devices[g]);
+    }
+  }
+  const int64_t widest = (nx + num_slabs - 1) / num_slabs * ny * nz;
+  if (widest >= (int64_t{1} << 32))
+  {
+    SetLastError("connected components: slabs of 2^32 cells or more are not supported "
+                 "(%lld cells in the widest of %d slabs)", static_cast<long long>(widest),
+                 num_slabs);
+    return VGT_B200_ERR_UNSUPPORTED;
+  }
+  return VGT_B200_OK;
+}
+
+template <int kCellWords>
+int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
+                             const int* devices, int num_slabs, uint32_t* out_num_components)
+{
+  constexpr size_t kCellBytes = sizeof(uint32_t) * kCellWords;
+  const uint32_t plane = static_cast<uint32_t>(ny * nz);
+  std::vector<int64_t> x_begin(static_cast<size_t>(num_slabs) + 1);
+  for (int g = 0; g < num_slabs; g++)
+  {
+    int64_t end;
+    SplitRange(nx, num_slabs, g, &x_begin[static_cast<size_t>(g)], &end);
+  }
+  x_begin[static_cast<size_t>(num_slabs)] = nx;
+  std::vector<uint64_t> slab_base(static_cast<size_t>(num_slabs) + 1);
+  for (int g = 0; g <= num_slabs; g++)
+  {
+    slab_base[static_cast<size_t>(g)] = static_cast<uint64_t>(x_begin[static_cast<size_t>(g)])
+                                      * plane;
+  }
+
+  // What one slab's thread shows the others between phases (written before a barrier, read
+  // after it). Everything that crosses slabs goes through host memory with plain async copies:
+  // it is O(num_slabs * ny * nz), and neither peer access nor access to another device's
+  // stream-ordered pool is needed.
+  struct Shared
+  {
+    std::vector<uint32_t> last_plane;  // the slab's last x-plane of cells
+    std::vector<uint32_t> face_roots;  // and the local roots of its cells
+    std::vector<Edge> edges;           // the edges of the face below the slab
+    uint64_t num_global_roots = 0;     // count_g
+  };
+  std::vector<Shared> shared(static_cast<size_t>(num_slabs));
+  // the face graph as resolved on devices[0]: the nodes, their compact roots, their ids
+  std::vector<uint64_t> nodes;
+  std::vector<uint32_t> node_roots;
+  std::vector<uint32_t> node_ids;
+  std::vector<uint32_t> slab_first(static_cast<size_t>(num_slabs) + 1, 0);
+  std::atomic<uint64_t> total_components{0};
+
+  ThreadBarrier barrier(num_slabs);
+  std::vector<int> statuses(static_cast<size_t>(num_slabs), VGT_B200_OK);
+  std::vector<std::string> messages(static_cast<size_t>(num_slabs));
+  std::atomic<int> failed{0};
+  const char* const kStoodDown = "another slab failed";
+
+  const auto worker = [&](const int g)
+  {
+    const size_t s = static_cast<size_t>(g);
+    const int device = devices[g];
+    ScopedDevice scoped(device);
+    const int64_t slab_x = x_begin[s + 1] - x_begin[s];
+    const Grid grid{static_cast<uint32_t>(slab_x), static_cast<uint32_t>(ny),
+                    static_cast<uint32_t>(nz), static_cast<uint32_t>(slab_x * plane)};
+    const uint32_t words = (grid.count + 31) / 32;
+    const size_t slab_bytes = kCellBytes * grid.count;
+    char* const h_slab = h_cells + kCellBytes * slab_base[s];
+    uint32_t num_components = 0;
+    uint32_t first_node = 0;
+    uint32_t num_nodes = 0;  // of this slab
+    uint64_t offset = 0;
+
+    StreamGuard guard;
+    StreamScratch<uint32_t> d_cells;
+    StreamScratch<uint32_t> parent;
+    StreamScratch<uint32_t> mask;
+    StreamScratch<uint32_t> word_prefix;  // words + 1 entries
+    StreamScratch<char> scan_storage;
+    StreamScratch<uint32_t> face_roots;
+    StreamScratch<uint32_t> below_plane;
+    StreamScratch<uint32_t> below_roots;
+    StreamScratch<Edge> edges;
+    StreamScratch<uint32_t> edge_count;
+    StreamScratch<uint32_t> bits;
+    StreamScratch<uint32_t> bit_prefix;
+    StreamScratch<uint32_t> final_ids;
+    StreamScratch<uint64_t> my_nodes;
+    StreamScratch<uint32_t> my_roots;
+    StreamScratch<uint32_t> my_ids;
+    // devices[0] only: the face graph
+    StreamScratch<Edge> all_edges;
+    StreamScratch<uint64_t> sorted;
+    StreamScratch<uint64_t> all_nodes;
+    StreamScratch<uint32_t> all_parent;
+    StreamScratch<uint32_t> all_roots;
+    StreamScratch<uint32_t> resolve_words;  // node count, then slab_first[]
+    StreamScratch<uint64_t> d_slab_base;
+    StreamScratch<char> resolve_storage;
+    StagedTransfer transfer;
+    if (num_slabs >= 6)
+    {
+      // enough slab threads to be the parallel copy workers themselves (the shared workers serve
+      // one caller at a time)
+      transfer.UseCallingThreadOnly();
+    }
+    struct DrainOnExit
+    {
+      const StreamGuard& guard;
+      ~DrainOnExit()
+      {
+        if (guard.stream != nullptr)
+        {
+          cudaStreamSynchronize(guard.stream);
+        }
+      }
+    } drain{guard};
+
+    // 1. the slab up, steps 1-4 on it, K_g; the local roots of its last plane for the slab above
+    const auto local_labelling = [&]() -> int
+    {
+      VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+      KeepPoolMemory(device);
+      VGT_CUDA_TRY(cudaStreamCreateWithFlags(&guard.stream, cudaStreamNonBlocking), "stream");
+      cudaStream_t stream = guard.stream;
+      VGT_CUDA_TRY(d_cells.Allocate(static_cast<int64_t>(grid.count) * kCellWords, stream),
+                   "cell slab allocation");
+      VGT_CUDA_TRY(parent.Allocate(grid.count, stream), "parent allocation");
+      VGT_CUDA_TRY(mask.Allocate(words, stream), "root mask allocation");
+      VGT_CUDA_TRY(word_prefix.Allocate(int64_t{words} + 1, stream), "word count allocation");
+      size_t scan_bytes = 0;
+      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, word_prefix.get(),
+                                                 word_prefix.get(), static_cast<int>(words) + 1,
+                                                 stream),
+                   "scan size query");
+      VGT_CUDA_TRY(scan_storage.Allocate(static_cast<int64_t>(std::max<size_t>(scan_bytes, 1)),
+                                         stream),
+                   "scan storage allocation");
+      VGT_CUDA_TRY(cudaMemsetAsync(word_prefix.get() + words, 0, sizeof(uint32_t), stream),
+                   "count reset");
+      VGT_CUDA_TRY(transfer.ToDevice(reinterpret_cast<char*>(d_cells.get()), slab_bytes, h_slab,
+                                     slab_bytes, slab_bytes, 1, stream),
+                   "copy cell slab to device");
+      const uint32_t blocks = Blocks(grid.count);
+      InitRunsKernel<kCellWords><<<blocks, kThreads, 0, stream>>>(d_cells.get(), grid,
+                                                                  parent.get());
+      VGT_LAUNCHED("InitRunsKernel");
+      MergeKernel<kCellWords><<<blocks, kThreads, 0, stream>>>(d_cells.get(), grid, parent.get());
+      VGT_LAUNCHED("MergeKernel");
+      MarkRootsKernel<<<blocks, kThreads, 0, stream>>>(parent.get(), grid.count, mask.get(),
+                                                       word_prefix.get());
+      VGT_LAUNCHED("MarkRootsKernel");
+      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(scan_storage.get(), scan_bytes,
+                                                 word_prefix.get(), word_prefix.get(),
+                                                 static_cast<int>(words) + 1, stream),
+                   "root rank scan");
+      NoteKernelLaunch();
+      NoteKernelLaunch();
+      if (g + 1 < num_slabs)
+      {
+        Shared& face = shared[s];
+        face.last_plane.resize(size_t{plane} * kCellWords);
+        face.face_roots.resize(plane);
+        VGT_CUDA_TRY(face_roots.Allocate(plane, stream), "face root allocation");
+        FaceRootsKernel<<<Blocks(plane), kThreads, 0, stream>>>(
+            parent.get(), grid.count - plane, plane, face_roots.get());
+        VGT_LAUNCHED("FaceRootsKernel");
+        VGT_CUDA_TRY(cudaMemcpyAsync(face.face_roots.data(), face_roots.get(),
+                                     sizeof(uint32_t) * plane, cudaMemcpyDeviceToHost, stream),
+                     "copy face roots to host");
+        VGT_CUDA_TRY(cudaMemcpyAsync(face.last_plane.data(),
+                                     d_cells.get() + size_t{grid.count - plane} * kCellWords,
+                                     kCellBytes * plane, cudaMemcpyDeviceToHost, stream),
+                     "copy face cells to host");
+      }
+      VGT_CUDA_TRY(cudaMemcpyAsync(&num_components, word_prefix.get() + words, sizeof(uint32_t),
+                                   cudaMemcpyDeviceToHost, stream),
+                   "copy local component count");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "slab labelling");
+      return VGT_B200_OK;
+    };
+
+    // 2. the edges of the face below the slab, on the slab's device
+    const auto face_edges = [&]() -> int
+    {
+      if (g == 0)
+      {
+        return VGT_B200_OK;
+      }
+      cudaStream_t stream = guard.stream;
+      const Shared& below = shared[s - 1];
+      VGT_CUDA_TRY(below_plane.Allocate(int64_t{plane} * kCellWords, stream),
+                   "face cell allocation");
+      VGT_CUDA_TRY(below_roots.Allocate(plane, stream), "face root allocation");
+      VGT_CUDA_TRY(edges.Allocate(plane, stream), "edge allocation");
+      VGT_CUDA_TRY(edge_count.Allocate(1, stream), "edge count allocation");
+      VGT_CUDA_TRY(cudaMemcpyAsync(below_plane.get(), below.last_plane.data(),
+                                   kCellBytes * plane, cudaMemcpyHostToDevice, stream),
+                   "copy face cells to device");
+      VGT_CUDA_TRY(cudaMemcpyAsync(below_roots.get(), below.face_roots.data(),
+                                   sizeof(uint32_t) * plane, cudaMemcpyHostToDevice, stream),
+                   "copy face roots to device");
+      VGT_CUDA_TRY(cudaMemsetAsync(edge_count.get(), 0, sizeof(uint32_t), stream),
+                   "edge count reset");
+      FaceEdgesKernel<kCellWords><<<Blocks(plane), kThreads, 0, stream>>>(
+          below_plane.get(), below_roots.get(), slab_base[s - 1], d_cells.get(), parent.get(),
+          slab_base[s], plane, static_cast<uint32_t>(nz), edges.get(), edge_count.get());
+      VGT_LAUNCHED("FaceEdgesKernel");
+      uint32_t count = 0;
+      VGT_CUDA_TRY(cudaMemcpyAsync(&count, edge_count.get(), sizeof(uint32_t),
+                                   cudaMemcpyDeviceToHost, stream),
+                   "copy edge count");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "face edges");
+      shared[s].edges.resize(count);
+      VGT_CUDA_TRY(cudaMemcpyAsync(shared[s].edges.data(), edges.get(), sizeof(Edge) * count,
+                                   cudaMemcpyDeviceToHost, stream),
+                   "copy face edges to host");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "face edges");
+      return VGT_B200_OK;
+    };
+
+    // 3. devices[0]: the face graph resolved into compact roots
+    const auto resolve = [&]() -> int
+    {
+      if (g != 0)
+      {
+        return VGT_B200_OK;
+      }
+      cudaStream_t stream = guard.stream;
+      uint64_t total = 0;
+      for (int f = 1; f < num_slabs; f++)
+      {
+        total += shared[static_cast<size_t>(f)].edges.size();
+      }
+      const uint32_t num_edges = static_cast<uint32_t>(total);  // <= 7 * 2^26
+      const int num_endpoints = static_cast<int>(2 * total);
+      VGT_CUDA_TRY(all_edges.Allocate(std::max<int64_t>(1, num_edges), stream), "edge allocation");
+      VGT_CUDA_TRY(sorted.Allocate(std::max(1, num_endpoints), stream), "endpoint allocation");
+      VGT_CUDA_TRY(all_nodes.Allocate(std::max(1, num_endpoints), stream), "node allocation");
+      VGT_CUDA_TRY(all_parent.Allocate(std::max(1, num_endpoints), stream),
+                   "node parent allocation");
+      VGT_CUDA_TRY(all_roots.Allocate(std::max(1, num_endpoints), stream), "node root allocation");
+      VGT_CUDA_TRY(resolve_words.Allocate(num_slabs + 2, stream), "node count allocation");
+      VGT_CUDA_TRY(d_slab_base.Allocate(num_slabs + 1, stream), "slab base allocation");
+      VGT_CUDA_TRY(cudaMemcpyAsync(d_slab_base.get(), slab_base.data(),
+                                   sizeof(uint64_t) * (num_slabs + 1), cudaMemcpyHostToDevice,
+                                   stream),
+                   "copy slab bases");
+      VGT_CUDA_TRY(cudaMemsetAsync(resolve_words.get(), 0, sizeof(uint32_t), stream),
+                   "node count reset");
+      uint32_t at = 0;
+      for (int f = 1; f < num_slabs; f++)
+      {
+        const std::vector<Edge>& face = shared[static_cast<size_t>(f)].edges;
+        if (!face.empty())
+        {
+          VGT_CUDA_TRY(cudaMemcpyAsync(all_edges.get() + at, face.data(),
+                                       sizeof(Edge) * face.size(), cudaMemcpyHostToDevice, stream),
+                       "gather face edges");
+        }
+        at += static_cast<uint32_t>(face.size());
+      }
+      int end_bit = 1;
+      while (end_bit < 64 && (slab_base[static_cast<size_t>(num_slabs)] >> end_bit) != 0)
+      {
+        end_bit++;
+      }
+      const uint64_t* endpoints = reinterpret_cast<const uint64_t*>(all_edges.get());
+      size_t sort_bytes = 0;
+      size_t unique_bytes = 0;
+      VGT_CUDA_TRY(cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, endpoints, sorted.get(),
+                                                  num_endpoints, 0, end_bit, stream),
+                   "sort size query");
+      VGT_CUDA_TRY(cub::DeviceSelect::Unique(nullptr, unique_bytes, sorted.get(),
+                                             all_nodes.get(), resolve_words.get(),
+                                             num_endpoints, stream),
+                   "unique size query");
+      size_t storage_bytes = std::max<size_t>({sort_bytes, unique_bytes, 1});
+      VGT_CUDA_TRY(resolve_storage.Allocate(static_cast<int64_t>(storage_bytes), stream),
+                   "resolve storage allocation");
+      if (num_endpoints > 0)
+      {
+        VGT_CUDA_TRY(cub::DeviceRadixSort::SortKeys(resolve_storage.get(), sort_bytes, endpoints,
+                                                    sorted.get(), num_endpoints, 0, end_bit,
+                                                    stream),
+                     "endpoint sort");
+        NoteKernelLaunch();
+        VGT_CUDA_TRY(cub::DeviceSelect::Unique(resolve_storage.get(), unique_bytes, sorted.get(),
+                                               all_nodes.get(), resolve_words.get(),
+                                               num_endpoints, stream),
+                     "endpoint unique");
+        NoteKernelLaunch();
+      }
+      uint32_t nodes_total = 0;
+      VGT_CUDA_TRY(cudaMemcpyAsync(&nodes_total, resolve_words.get(), sizeof(uint32_t),
+                                   cudaMemcpyDeviceToHost, stream),
+                   "copy node count");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "face graph nodes");
+      if (num_edges > 0)
+      {
+        NodeInitKernel<<<Blocks(nodes_total), kThreads, 0, stream>>>(all_parent.get(),
+                                                                     nodes_total);
+        VGT_LAUNCHED("NodeInitKernel");
+        NodeUnionKernel<<<Blocks(num_edges), kThreads, 0, stream>>>(
+            all_edges.get(), num_edges, all_nodes.get(), nodes_total, all_parent.get());
+        VGT_LAUNCHED("NodeUnionKernel");
+      }
+      NodeFlattenKernel<<<Blocks(std::max<uint32_t>(nodes_total, num_slabs + 1)), kThreads, 0,
+                          stream>>>(all_parent.get(), all_nodes.get(), nodes_total,
+                                    d_slab_base.get(), num_slabs + 1, all_roots.get(),
+                                    resolve_words.get() + 1);
+      VGT_LAUNCHED("NodeFlattenKernel");
+      VGT_CUDA_TRY(cudaMemcpyAsync(slab_first.data(), resolve_words.get() + 1,
+                                   sizeof(uint32_t) * (num_slabs + 1), cudaMemcpyDeviceToHost,
+                                   stream),
+                   "copy slab node ranges");
+      nodes.resize(nodes_total);
+      node_roots.resize(nodes_total);
+      node_ids.resize(nodes_total);
+      if (nodes_total > 0)
+      {
+        VGT_CUDA_TRY(cudaMemcpyAsync(nodes.data(), all_nodes.get(), sizeof(uint64_t) * nodes_total,
+                                     cudaMemcpyDeviceToHost, stream),
+                     "copy nodes to host");
+        VGT_CUDA_TRY(cudaMemcpyAsync(node_roots.data(), all_roots.get(),
+                                     sizeof(uint32_t) * nodes_total, cudaMemcpyDeviceToHost,
+                                     stream),
+                     "copy node roots to host");
+      }
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "face graph");
+      return VGT_B200_OK;
+    };
+
+    // 4. the slab's global roots: bits, their count (count_g)
+    const auto count_global_roots = [&]() -> int
+    {
+      cudaStream_t stream = guard.stream;
+      first_node = slab_first[s];
+      num_nodes = slab_first[s + 1] - first_node;
+      const uint32_t bit_words = (num_components + 31) / 32;
+      VGT_CUDA_TRY(bits.Allocate(bit_words, stream), "root bit allocation");
+      VGT_CUDA_TRY(bit_prefix.Allocate(int64_t{bit_words} + 1, stream), "root bit prefix allocation");
+      VGT_CUDA_TRY(my_nodes.Allocate(std::max<uint32_t>(1, num_nodes), stream), "node allocation");
+      VGT_CUDA_TRY(my_roots.Allocate(std::max<uint32_t>(1, num_nodes), stream),
+                   "node root allocation");
+      VGT_CUDA_TRY(my_ids.Allocate(std::max<uint32_t>(1, num_nodes), stream), "node id allocation");
+      GlobalRootBitsInitKernel<<<Blocks(bit_words), kThreads, 0, stream>>>(bits.get(),
+                                                                          num_components);
+      VGT_LAUNCHED("GlobalRootBitsInitKernel");
+      if (num_nodes > 0)
+      {
+        VGT_CUDA_TRY(cudaMemcpyAsync(my_nodes.get(), nodes.data() + first_node,
+                                     sizeof(uint64_t) * num_nodes, cudaMemcpyHostToDevice, stream),
+                     "copy slab nodes to device");
+        VGT_CUDA_TRY(cudaMemcpyAsync(my_roots.get(), node_roots.data() + first_node,
+                                     sizeof(uint32_t) * num_nodes, cudaMemcpyHostToDevice, stream),
+                     "copy slab node roots to device");
+        ClearMergedBitsKernel<<<Blocks(num_nodes), kThreads, 0, stream>>>(
+            my_nodes.get(), my_roots.get(), num_nodes, first_node, slab_base[s], mask.get(),
+            word_prefix.get(), bits.get());
+        VGT_LAUNCHED("ClearMergedBitsKernel");
+      }
+      VGT_CUDA_TRY(cudaMemsetAsync(bit_prefix.get() + bit_words, 0, sizeof(uint32_t), stream),
+                   "count reset");
+      BitCountsKernel<<<Blocks(bit_words), kThreads, 0, stream>>>(bits.get(), bit_words,
+                                                                  bit_prefix.get());
+      VGT_LAUNCHED("BitCountsKernel");
+      // (bit_words + 1 <= words + 1: the scan storage of step 4 fits)
+      size_t scan_bytes = 0;
+      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, bit_prefix.get(),
+                                                 bit_prefix.get(),
+                                                 static_cast<int>(bit_words) + 1, stream),
+                   "scan size query");
+      StreamScratch<char> storage;
+      VGT_CUDA_TRY(storage.Allocate(static_cast<int64_t>(std::max<size_t>(scan_bytes, 1)), stream),
+                   "scan storage allocation");
+      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(storage.get(), scan_bytes, bit_prefix.get(),
+                                                 bit_prefix.get(),
+                                                 static_cast<int>(bit_words) + 1, stream),
+                   "global root scan");
+      NoteKernelLaunch();
+      NoteKernelLaunch();
+      uint32_t count = 0;
+      VGT_CUDA_TRY(cudaMemcpyAsync(&count, bit_prefix.get() + bit_words, sizeof(uint32_t),
+                                   cudaMemcpyDeviceToHost, stream),
+                   "copy global root count");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "global roots");
+      shared[s].num_global_roots = count;
+      return VGT_B200_OK;
+    };
+
+    // 5. offsets (refused past 0xFFFFFFFF, before any cell is written), ids of the slab's global
+    //    roots, published to devices[0]
+    const auto publish = [&]() -> int
+    {
+      uint64_t total = 0;
+      for (int f = 0; f < num_slabs; f++)
+      {
+        if (f == g)
+        {
+          offset = total;
+        }
+        total += shared[static_cast<size_t>(f)].num_global_roots;
+      }
+      if (total > 0xFFFFFFFFull)
+      {
+        SetLastError("connected components: %llu components do not fit the 32-bit component word",
+                     static_cast<unsigned long long>(total));
+        return VGT_B200_ERR_UNSUPPORTED;
+      }
+      cudaStream_t stream = guard.stream;
+      VGT_CUDA_TRY(final_ids.Allocate(num_components, stream), "final id allocation");
+      FinalIdsKernel<<<Blocks(num_components), kThreads, 0, stream>>>(
+          bits.get(), bit_prefix.get(), num_components, static_cast<uint32_t>(offset),
+          final_ids.get());
+      VGT_LAUNCHED("FinalIdsKernel");
+      if (num_nodes > 0)
+      {
+        PublishNodeIdsKernel<<<Blocks(num_nodes), kThreads, 0, stream>>>(
+            my_nodes.get(), num_nodes, slab_base[s], mask.get(), word_prefix.get(),
+            final_ids.get(), my_ids.get());
+        VGT_LAUNCHED("PublishNodeIdsKernel");
+        VGT_CUDA_TRY(cudaMemcpyAsync(node_ids.data() + first_node, my_ids.get(),
+                                     sizeof(uint32_t) * num_nodes, cudaMemcpyDeviceToHost, stream),
+                     "publish node ids");
+      }
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "node id publication");
+      total_components = total;  // (the same sum in every slab)
+      return VGT_B200_OK;
+    };
+
+    // 6. devices[0]: every node takes its compact root's id
+    const auto propagate = [&]() -> int
+    {
+      const uint32_t nodes_total = slab_first[static_cast<size_t>(num_slabs)];
+      if (g != 0 || nodes_total == 0)
+      {
+        return VGT_B200_OK;
+      }
+      cudaStream_t stream = guard.stream;
+      StreamScratch<uint32_t> ids;
+      VGT_CUDA_TRY(ids.Allocate(nodes_total, stream), "node id allocation");
+      VGT_CUDA_TRY(cudaMemcpyAsync(ids.get(), node_ids.data(), sizeof(uint32_t) * nodes_total,
+                                   cudaMemcpyHostToDevice, stream),
+                   "copy node ids to device");
+      NodeIdsFromRootsKernel<<<Blocks(nodes_total), kThreads, 0, stream>>>(all_roots.get(),
+                                                                           nodes_total, ids.get());
+      VGT_LAUNCHED("NodeIdsFromRootsKernel");
+      VGT_CUDA_TRY(cudaMemcpyAsync(node_ids.data(), ids.get(), sizeof(uint32_t) * nodes_total,
+                                   cudaMemcpyDeviceToHost, stream),
+                   "copy node ids to host");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "node ids");
+      return VGT_B200_OK;
+    };
+
+    // 7. the final ids of the merged components, then the component word of every cell
+    const auto write = [&]() -> int
+    {
+      cudaStream_t stream = guard.stream;
+      if (num_nodes > 0)
+      {
+        VGT_CUDA_TRY(cudaMemcpyAsync(my_ids.get(), node_ids.data() + first_node,
+                                     sizeof(uint32_t) * num_nodes, cudaMemcpyHostToDevice, stream),
+                     "copy node ids to device");
+        ApplyNodeIdsKernel<<<Blocks(num_nodes), kThreads, 0, stream>>>(
+            my_nodes.get(), my_ids.get(), num_nodes, slab_base[s], mask.get(), word_prefix.get(),
+            final_ids.get());
+        VGT_LAUNCHED("ApplyNodeIdsKernel");
+      }
+      WriteSlabComponentsKernel<kCellWords><<<Blocks(grid.count), kThreads, 0, stream>>>(
+          d_cells.get(), grid.count, parent.get(), mask.get(), word_prefix.get(), final_ids.get());
+      VGT_LAUNCHED("WriteSlabComponentsKernel");
+      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "component write");
+      return VGT_B200_OK;
+    };
+
+    // 8. every slab has written: the cells back
+    const auto copy_back = [&]() -> int
+    {
+      VGT_CUDA_TRY(transfer.ToHost(h_slab, slab_bytes, reinterpret_cast<char*>(d_cells.get()),
+                                   slab_bytes, slab_bytes, 1, guard.stream),
+                   "copy cell slab to host");
+      VGT_CUDA_TRY(cudaStreamSynchronize(guard.stream), "cell copy");
+      return VGT_B200_OK;
+    };
+
+    // Every thread passes every barrier; after the first failure (here or in another slab) the
+    // remaining phases are skipped.
+    int status = VGT_B200_OK;
+    const std::function<int()> phases[] = {local_labelling, face_edges, resolve,
+                                           count_global_roots, publish, propagate, write,
+                                           copy_back};
+    for (const auto& phase : phases)
+    {
+      if (status == VGT_B200_OK && failed.load() != 0)
+      {
+        status = VGT_B200_ERR_DEVICE;
+        messages[s] = kStoodDown;
+      }
+      if (status == VGT_B200_OK)
+      {
+        status = phase();
+        if (status != VGT_B200_OK)
+        {
+          messages[s] = vgt_b200_last_error();  // thread-local text
+          failed.store(1);
+        }
+      }
+      barrier.Wait();
+    }
+    statuses[s] = status;
+  };
+
+  std::vector<std::thread> threads;
+  for (int g = 1; g < num_slabs; g++)
+  {
+    threads.emplace_back(worker, g);
+  }
+  worker(0);
+  for (auto& thread : threads)
+  {
+    thread.join();
+  }
+  // the slab that failed first-hand, not the ones that stood down because of it
+  for (const bool first_hand : {true, false})
+  {
+    for (int g = 0; g < num_slabs; g++)
+    {
+      const size_t s = static_cast<size_t>(g);
+      const bool stood_down = messages[s] == kStoodDown;
+      if (statuses[s] != VGT_B200_OK && stood_down != first_hand)
+      {
+        SetLastError("slab %d (device %d): %s", g, devices[g], messages[s].c_str());
+        return statuses[s];
+      }
+    }
+  }
+  *out_num_components = static_cast<uint32_t>(total_components);
+  return VGT_B200_OK;
+}
 }  // namespace
 }  // namespace components
 }  // namespace vgt_b200
@@ -451,5 +1329,29 @@ int vgt_b200_connected_components(void* cells, int cell_bytes, int64_t nx, int64
   }
   *out_num_components = num_components;
   return VGT_B200_OK;
+}
+
+int vgt_b200_connected_components_multi(void* cells, int cell_bytes, int64_t nx, int64_t ny,
+                                        int64_t nz, const int* devices, int num_slabs,
+                                        uint32_t* out_num_components)
+{
+  const int check = CheckMultiArguments(cells, cell_bytes, nx, ny, nz, devices, num_slabs,
+                                        out_num_components);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  if (num_slabs == 1)
+  {
+    return vgt_b200_connected_components(cells, cell_bytes, nx, ny, nz, devices[0],
+                                         out_num_components);
+  }
+  if (cell_bytes == 8)
+  {
+    return ConnectedComponentsSlabs<2>(static_cast<char*>(cells), nx, ny, nz, devices, num_slabs,
+                                       out_num_components);
+  }
+  return ConnectedComponentsSlabs<4>(static_cast<char*>(cells), nx, ny, nz, devices, num_slabs,
+                                     out_num_components);
 }
 }  // extern "C"

@@ -528,18 +528,6 @@ int LaunchEnvelope(uint32_t* d_in, typename OutputOf<kMode>::Type* d_out,
                                                 d_keys, stream, d_redo_list);
 }
 
-struct StreamGuard
-{
-  cudaStream_t stream = nullptr;
-  ~StreamGuard()
-  {
-    if (stream != nullptr)
-    {
-      cudaStreamDestroy(stream);
-    }
-  }
-};
-
 struct EventGuard
 {
   cudaEvent_t event = nullptr;
@@ -1352,41 +1340,6 @@ int SdfFreeAndNamedHost(const void* h_cells, int cell_bytes, int64_t nx, int64_t
 // once every stream has drained, x pass + finalize on its y-slab, strided copy of the y-slab
 // into its place in the caller's grid.
 // ------------------------------------------------------------------------------------------------
-inline void SplitRange(int64_t total, int parts, int index, int64_t* begin, int64_t* end)
-{
-  const int64_t base = total / parts;
-  const int64_t extra = total % parts;
-  *begin = index * base + std::min<int64_t>(index, extra);
-  *end = *begin + base + (index < extra ? 1 : 0);
-}
-
-// A reusable barrier for the per-device host threads (std::barrier is C++20).
-class ThreadBarrier
-{
-public:
-  explicit ThreadBarrier(int count) : count_(count), waiting_(0), generation_(0) {}
-  void Wait()
-  {
-    std::unique_lock<std::mutex> lock(mutex_);
-    const int generation = generation_;
-    if (++waiting_ == count_)
-    {
-      waiting_ = 0;
-      generation_++;
-      released_.notify_all();
-      return;
-    }
-    released_.wait(lock, [&] { return generation != generation_; });
-  }
-
-private:
-  std::mutex mutex_;
-  std::condition_variable released_;
-  int count_;
-  int waiting_;
-  int generation_;
-};
-
 int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double resolution,
                    int unknown_is_filled, int add_virtual_border, const int* devices,
                    int num_devices, float* h_out, float* out_min, float* out_max)

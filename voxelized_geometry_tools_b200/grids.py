@@ -402,12 +402,21 @@ class _CellGrid:
         _capi.check(code)
         return self._wrap(out, lo.value, hi.value, parameters)
 
-    def _connected_components(self, device):
-        _capi.require_device(device)
+    def _connected_components(self, device, devices=None):
         count = ctypes.c_uint32()
-        code = _capi.library().vgt_b200_connected_components(
-            self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape, device,
-            ctypes.byref(count))
+        if devices and len(devices) > 1:
+            listed = [int(d) for d in devices]
+            for ordinal in sorted(set(listed)):
+                _capi.require_device(ordinal)
+            code = _capi.library().vgt_b200_connected_components_multi(
+                self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape,
+                (ctypes.c_int * len(listed))(*listed), len(listed), ctypes.byref(count))
+        else:
+            device = int(devices[0]) if devices else device
+            _capi.require_device(device)
+            code = _capi.library().vgt_b200_connected_components(
+                self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape, device,
+                ctypes.byref(count))
         _capi.check(code)
         return int(count.value)
 
@@ -435,13 +444,17 @@ class OccupancyComponentMap(_CellGrid):
     def ExtractSignedDistanceFieldDouble(self, parameters, device: int = 0):
         return self.ExtractSignedDistanceField(parameters, np.float64, device)
 
-    def UpdateConnectedComponents(self, device: int = 0) -> int:
+    def UpdateConnectedComponents(self, device: int = 0, devices=None) -> int:
         """Labels the connected components of the map into every cell's ``component`` and returns
         their number (ComputeConnectedComponents, topology_computation.hpp:138-196): face
         neighbours are connected iff both are filled (> 0.5) or both are not; components are
         numbered from 1 in the order of their first cell in storage order. Recomputed on every
-        call (nothing is cached)."""
-        return self._connected_components(device)
+        call (nothing is cached).
+        ``devices``: two or more device ordinals (repeats allowed, at most 8, no more than the
+        map's x size) label the map cut into that many x-slabs, slab g on ``devices[g]``
+        (vgt_b200_connected_components_multi): the same ids and count as on one device, and
+        maps of 2^32 cells or more when no slab reaches 2^32 cells."""
+        return self._connected_components(device, devices)
 
 
 class TaggedObjectOccupancyMap(_CellGrid):
@@ -509,14 +522,18 @@ class TaggedObjectOccupancyComponentMap(TaggedObjectOccupancyMap):
 
     CELL = TAGGED_OBJECT_OCCUPANCY_COMPONENT_CELL
 
-    def UpdateConnectedComponents(self, device: int = 0) -> int:
+    def UpdateConnectedComponents(self, device: int = 0, devices=None) -> int:
         """Labels the connected components of the map into every cell's ``component`` and returns
         their number (ComputeConnectedComponents, topology_computation.hpp:138-196): face
         neighbours are connected iff both are filled (> 0.5) or both are not, and their object
         ids are equal; components are numbered from 1 in the order of their first cell in storage
         order. ``object_id`` and ``spatial_segment`` are left as they are. Recomputed on every
-        call (nothing is cached)."""
-        return self._connected_components(device)
+        call (nothing is cached).
+        ``devices``: two or more device ordinals (repeats allowed, at most 8, no more than the
+        map's x size) label the map cut into that many x-slabs, slab g on ``devices[g]``
+        (vgt_b200_connected_components_multi): the same ids and count as on one device, and
+        maps of 2^32 cells or more when no slab reaches 2^32 cells."""
+        return self._connected_components(device, devices)
 
 
 def ExtractSignedDistanceFieldFromMask(filled_mask: np.ndarray, origin_transform, frame: str,
