@@ -174,6 +174,53 @@ VGT_B200_API int vgt_b200_sdf_free_and_named_f64(
     int unknown_is_filled, int add_virtual_border, int device, double* sdf_out, double* out_min,
     double* out_max);
 
+/* The three cell entries above on a map that lives on the device; they replace the same reference
+ * code (tagged_object_occupancy_map.hpp:199-262, :293-378, occupancy_component_map.hpp:270-306).
+ * Each takes the argument list of its host entry, except that
+ *   d_cells      device cells (4-byte aligned), the layout of `cells` above
+ *   d_sdf_out    device T[nx*ny*nz] (T[num_object_ids][nx*ny*nz] for the batch)
+ *   d_min_max    device T[2] (T[num_object_ids][2] for the batch) or NULL
+ *   stream       a cudaStream_t; the call is asynchronous and stream-ordered on it, its scratch
+ *                comes from the device's stream-ordered pool
+ * object_ids stays a host array; it has been read when the call returns. Every argument is checked
+ * before the first device call, as in the host entries; the batch also refuses num_object_ids *
+ * nx*ny*nz * sizeof(T) bytes beyond int64.
+ * vgt_b200_sdf_from_cells_*_dev classifies the cells into a 1-byte mask, as the host entry does.
+ * vgt_b200_sdf_per_object_*_dev classifies them once per group of 255 distinct ids into a 1-byte
+ * slot map (1 + the id's position in the group; 0 = not filled or another group), and each SDF of
+ * the group runs on "slot == its id's slot": the cells are read ceil(distinct ids / 255) times,
+ * not once per object. Repeated ids and ids absent from the map are allowed; num_object_ids == 0
+ * launches nothing. */
+VGT_B200_API int vgt_b200_sdf_from_cells_f32_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, float* d_sdf_out, float* d_min_max, void* stream);
+
+VGT_B200_API int vgt_b200_sdf_from_cells_f64_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, double* d_sdf_out, double* d_min_max, void* stream);
+
+VGT_B200_API int vgt_b200_sdf_per_object_f32_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, float* d_sdf_out, float* d_min_max, void* stream);
+
+VGT_B200_API int vgt_b200_sdf_per_object_f64_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, double* d_sdf_out, double* d_min_max, void* stream);
+
+VGT_B200_API int vgt_b200_sdf_free_and_named_f32_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, int device, float* d_sdf_out, float* d_min_max,
+    void* stream);
+
+VGT_B200_API int vgt_b200_sdf_free_and_named_f64_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, int device, double* d_sdf_out,
+    double* d_min_max, void* stream);
+
 /* Replaces internal::ComputeDistanceFieldTransformInPlace(DegreeOfParallelism, VoxelGrid<double>&)
  * (include/.../signed_distance_field_generation.hpp:34-37, src/.../signed_distance_field_generation.cpp:258-391):
  * the in-place 3-D squared distance transform D(p) = min over q of f(q) + |p - q|^2 (voxel

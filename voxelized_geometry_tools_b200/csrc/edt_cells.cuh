@@ -77,6 +77,111 @@ __global__ void CellsToMaskKernel(const uint32_t* __restrict__ cells, int cell_w
   mask[i] = filled ? 1 : 0;
 }
 
+// The per-object batch on device cells (MakeSeparateObjectSDFs, tagged_object_occupancy_map.hpp:
+// 249-262) classifies the cells once per group of at most kSlotGroupSize distinct object ids into
+// a 1-byte slot map; SDF k of the batch then takes the three passes on "slot == key of object k".
+// Slot 0 is "not filled, or an object outside the group", so one byte tells 255 ids apart.
+constexpr int kSlotGroupSize = 255;
+
+// A kernel parameter (1 KB), so the host's id list needs no device copy.
+struct SlotGroup
+{
+  uint32_t ids[kSlotGroupSize];  // ascending, distinct
+  int count;
+};
+
+// slots[i] = 0 when the occupancy rule fails or cell i's object id (word 1) is not in the group,
+// else 1 + the id's position in group.ids. Grid-stride over a fixed grid, so that the copy of the
+// group into shared memory is paid per resident block, not per 256 voxels; four voxels per thread
+// and round, their loads issued before any is used.
+__global__ void __launch_bounds__(256) CellsToObjectSlotsKernel(
+    const uint32_t* __restrict__ cells, int cell_words, int64_t count, int unknown_is_filled,
+    const SlotGroup group, uint8_t* __restrict__ slots)
+{
+  constexpr int kPerThread = 4;
+  __shared__ uint32_t ids[kSlotGroupSize];
+  for (int j = threadIdx.x; j < group.count; j += blockDim.x)
+  {
+    ids[j] = group.ids[j];
+  }
+  __syncthreads();
+  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x * kPerThread;
+  for (int64_t base = static_cast<int64_t>(blockIdx.x) * blockDim.x * kPerThread + threadIdx.x;
+       base < count; base += stride)
+  {
+    uint32_t occupancy[kPerThread];
+    uint32_t object_id[kPerThread];
+#pragma unroll
+    for (int j = 0; j < kPerThread; j++)
+    {
+      const int64_t i = base + static_cast<int64_t>(j) * blockDim.x;
+      if (i < count)
+      {
+        occupancy[j] = __ldcs(cells + i * cell_words);
+        object_id[j] = __ldcs(cells + i * cell_words + 1);
+      }
+    }
+#pragma unroll
+    for (int j = 0; j < kPerThread; j++)
+    {
+      const int64_t i = base + static_cast<int64_t>(j) * blockDim.x;
+      if (i >= count)
+      {
+        break;
+      }
+      uint8_t slot = 0;
+      if (IsFilled(__uint_as_float(occupancy[j]), unknown_is_filled))
+      {
+        int low = 0;
+        int high = group.count;
+        while (low < high)
+        {
+          const int middle = (low + high) >> 1;
+          if (ids[middle] < object_id[j])
+          {
+            low = middle + 1;
+          }
+          else
+          {
+            high = middle;
+          }
+        }
+        if (low < group.count && ids[low] == object_id[j])
+        {
+          slot = static_cast<uint8_t>(low + 1);
+        }
+      }
+      slots[i] = slot;
+    }
+  }
+}
+
+// A byte of the slot map as the input of the scalar z scan: filled iff the slot equals the key of
+// the object whose SDF is computed, which the scans take where occupancy inputs take
+// unknown_is_filled.
+struct ObjectSlot
+{
+  uint8_t slot;
+};
+
+__device__ __forceinline__ bool IsFilled(ObjectSlot cell, int key) { return cell.slot == key; }
+
+__device__ __forceinline__ ObjectSlot LoadStreaming(const ObjectSlot* p)
+{
+  return ObjectSlot{__ldcs(reinterpret_cast<const uint8_t*>(p))};
+}
+
+// The same test four slots at a time, for the register and Vec4 scans.
+struct SlotEquals4Source
+{
+  using Vector = uchar4;
+  __device__ static __forceinline__ uint32_t Nibble(const uchar4& v, int key)
+  {
+    return (v.x == key ? 1u : 0u) | (v.y == key ? 2u : 0u) | (v.z == key ? 4u : 0u)
+        | (v.w == key ? 8u : 0u);
+  }
+};
+
 // ExtractFreeAndNamedObjectsSignedDistanceField's merge (tagged_object_occupancy_map.hpp:344-369):
 //   free >= 0 -> free;  else named <= -0 -> named;  else 0.   Then Lock()'s min/max.
 // Grid-stride: a fixed grid, so the min/max atomics are two per warp of the grid, not two per

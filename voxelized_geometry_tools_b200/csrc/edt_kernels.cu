@@ -42,8 +42,10 @@ int LaunchScan(const In* d_in, uint32_t* d_out, int64_t num_lines, int32_t lengt
   const size_t smem = sizeof(uint32_t) * 5 * num_words * kScanWarpsPerBlock;
   const int64_t blocks = (num_lines + kScanWarpsPerBlock - 1) / kScanWarpsPerBlock;
   // 128-bit path: every line must start 16-byte aligned in both buffers.
-  using Source = typename std::conditional<std::is_same<In, float>::value, Float4Source,
-                                           Uchar4Source>::type;
+  using Source = typename std::conditional<
+      std::is_same<In, float>::value, Float4Source,
+      typename std::conditional<std::is_same<In, ObjectSlot>::value, SlotEquals4Source,
+                                Uchar4Source>::type>::type;
   const bool aligned = (length % 4 == 0)
       && (reinterpret_cast<uintptr_t>(d_in) % sizeof(typename Source::Vector) == 0)
       && (reinterpret_cast<uintptr_t>(d_out) % sizeof(uint4) == 0);
@@ -1070,6 +1072,29 @@ int SdfFromCellsOnDevice(const uint32_t* d_cells, int cell_words, int64_t nx, in
                                      d_sdf, d_min_max, stream);
 }
 
+std::vector<uint32_t> SortedDistinct(const uint32_t* object_ids, int64_t num_object_ids)
+{
+  std::vector<uint32_t> sorted(object_ids, object_ids + num_object_ids);
+  std::sort(sorted.begin(), sorted.end());
+  sorted.erase(std::unique(sorted.begin(), sorted.end()), sorted.end());
+  return sorted;
+}
+
+// The id list of CellsToMaskKernel on the device (nothing is allocated for an empty list). The
+// copy from pageable memory has read `sorted` when cudaMemcpyAsync returns.
+int UploadIds(const std::vector<uint32_t>& sorted, StreamScratch<uint32_t>& ids,
+              cudaStream_t stream)
+{
+  if (!sorted.empty())
+  {
+    VGT_CUDA_TRY(ids.Allocate(static_cast<int64_t>(sorted.size()), stream), "id allocation");
+    VGT_CUDA_TRY(cudaMemcpyAsync(ids.get(), sorted.data(), sizeof(uint32_t) * sorted.size(),
+                                 cudaMemcpyHostToDevice, stream),
+                 "copy object ids to device");
+  }
+  return VGT_B200_OK;
+}
+
 // Cells and (sorted) object ids uploaded once for one or several SDFs.
 struct CellUpload
 {
@@ -1090,17 +1115,8 @@ struct CellUpload
       // the slots go back to the cache when `transfer` dies: their DMA must have finished
       VGT_CUDA_TRY(cudaStreamSynchronize(stream), "copy cells to device");
     }
-    sorted.assign(object_ids, object_ids + num_object_ids);
-    std::sort(sorted.begin(), sorted.end());
-    sorted.erase(std::unique(sorted.begin(), sorted.end()), sorted.end());
-    if (!sorted.empty())
-    {
-      VGT_CUDA_TRY(ids.Allocate(static_cast<int64_t>(sorted.size()), stream), "id allocation");
-      VGT_CUDA_TRY(cudaMemcpyAsync(ids.get(), sorted.data(), sizeof(uint32_t) * sorted.size(),
-                                   cudaMemcpyHostToDevice, stream),
-                   "copy object ids to device");
-    }
-    return VGT_B200_OK;
+    sorted = SortedDistinct(object_ids, num_object_ids);
+    return UploadIds(sorted, ids, stream);
   }
 };
 
@@ -1251,8 +1267,56 @@ int SdfFromCellsHost(const void* h_cells, int cell_bytes, int64_t nx, int64_t ny
   return VGT_B200_OK;
 }
 
-// ExtractFreeAndNamedObjectsSignedDistanceField (tagged_object_occupancy_map.hpp:293-378): the
-// SDF of every filled cell, the SDF of the filled cells of named objects (id > 0), merged.
+// ExtractFreeAndNamedObjectsSignedDistanceField (tagged_object_occupancy_map.hpp:293-378) on
+// device-resident cells: the SDF of every filled cell into d_sdf, the SDF of the filled cells of
+// named objects (id > 0) into a scratch, merged into d_sdf. d_min_max may be null.
+template <int kMode>
+int SdfFreeAndNamedOnDevice(const uint32_t* d_cells, int cell_words, int64_t nx, int64_t ny,
+                            int64_t nz, double resolution, int unknown_is_filled,
+                            int add_virtual_border, typename OutputOf<kMode>::Type* d_sdf,
+                            typename OutputOf<kMode>::Type* d_min_max, cudaStream_t stream)
+{
+  using Out = typename OutputOf<kMode>::Type;
+  using Key = typename OutputOf<kMode>::Key;
+  const int64_t count = nx * ny * nz;
+  StreamScratch<Out> d_named;
+  StreamScratch<Key> keys;
+  VGT_CUDA_TRY(d_named.Allocate(count, stream), "SDF allocation");
+  if (d_min_max != nullptr)
+  {
+    VGT_CUDA_TRY(keys.Allocate(2, stream), "min/max scratch");
+  }
+  int status = SdfFromCellsOnDevice<kMode>(d_cells, cell_words, nx, ny, nz, resolution,
+                                           unknown_is_filled, add_virtual_border, kAnyObject,
+                                           nullptr, 0, d_sdf, nullptr, stream);
+  if (status == VGT_B200_OK)
+  {
+    status = SdfFromCellsOnDevice<kMode>(d_cells, cell_words, nx, ny, nz, resolution,
+                                         unknown_is_filled, add_virtual_border, kNamedObjects,
+                                         nullptr, 0, d_named.get(), nullptr, stream);
+  }
+  if (status != VGT_B200_OK)
+  {
+    return status;
+  }
+  if (d_min_max != nullptr)
+  {
+    ResetMinMaxKeysKernel<Key><<<1, 1, 0, stream>>>(keys.get()); NoteKernelLaunch();
+  }
+  const int threads = 256;
+  const int64_t merge_blocks =
+      std::min<int64_t>((count + threads - 1) / threads, MultiprocessorCount() * 16);
+  MergeFreeAndNamedKernel<Out, Key><<<static_cast<unsigned>(merge_blocks), threads, 0, stream>>>(
+          d_sdf, d_named.get(), count, d_sdf, keys.get()); NoteKernelLaunch();
+  if (d_min_max != nullptr)
+  {
+    DecodeMinMaxKernel<Out, Key><<<1, 1, 0, stream>>>(keys.get(), d_min_max); NoteKernelLaunch();
+  }
+  VGT_CUDA_TRY(cudaGetLastError(), "MergeFreeAndNamedKernel launch");
+  return VGT_B200_OK;
+}
+
+// The same on host cells, with the upload and the copy-out.
 template <int kMode>
 int SdfFreeAndNamedHost(const void* h_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
                         double resolution, int unknown_is_filled, int add_virtual_border,
@@ -1261,7 +1325,6 @@ int SdfFreeAndNamedHost(const void* h_cells, int cell_bytes, int64_t nx, int64_t
                         typename OutputOf<kMode>::Type* out_max)
 {
   using Out = typename OutputOf<kMode>::Type;
-  using Key = typename OutputOf<kMode>::Key;
   const int check = CheckCellArguments(h_cells, cell_bytes, h_out, nx, ny, nz, resolution,
                                        nullptr, 0);
   if (check != VGT_B200_OK)
@@ -1283,36 +1346,18 @@ int SdfFreeAndNamedHost(const void* h_cells, int cell_bytes, int64_t nx, int64_t
     return uploaded;
   }
   StreamScratch<Out> d_free;
-  StreamScratch<Out> d_named;
   StreamScratch<Out> d_min_max;
-  StreamScratch<Key> keys;
   VGT_CUDA_TRY(d_free.Allocate(count, stream), "SDF allocation");
-  VGT_CUDA_TRY(d_named.Allocate(count, stream), "SDF allocation");
   VGT_CUDA_TRY(d_min_max.Allocate(2, stream), "min/max allocation");
-  VGT_CUDA_TRY(keys.Allocate(2, stream), "min/max scratch");
-  int status = SdfFromCellsOnDevice<kMode>(upload.cells.get(), cell_bytes / 4, nx, ny, nz,
-                                           resolution, unknown_is_filled, add_virtual_border,
-                                           kAnyObject, nullptr, 0, d_free.get(), nullptr, stream);
-  if (status == VGT_B200_OK)
-  {
-    status = SdfFromCellsOnDevice<kMode>(upload.cells.get(), cell_bytes / 4, nx, ny, nz,
-                                         resolution, unknown_is_filled, add_virtual_border,
-                                         kNamedObjects, nullptr, 0, d_named.get(), nullptr,
-                                         stream);
-  }
+  const int status = SdfFreeAndNamedOnDevice<kMode>(upload.cells.get(), cell_bytes / 4, nx, ny,
+                                                    nz, resolution, unknown_is_filled,
+                                                    add_virtual_border, d_free.get(),
+                                                    d_min_max.get(), stream);
   if (status != VGT_B200_OK)
   {
     cudaStreamSynchronize(stream);
     return status;
   }
-  ResetMinMaxKeysKernel<Key><<<1, 1, 0, stream>>>(keys.get()); NoteKernelLaunch();
-  const int threads = 256;
-  const int64_t merge_blocks =
-      std::min<int64_t>((count + threads - 1) / threads, MultiprocessorCount() * 16);
-  MergeFreeAndNamedKernel<Out, Key><<<static_cast<unsigned>(merge_blocks), threads, 0, stream>>>(
-          d_free.get(), d_named.get(), count, d_free.get(), keys.get()); NoteKernelLaunch();
-  DecodeMinMaxKernel<Out, Key><<<1, 1, 0, stream>>>(keys.get(), d_min_max.get()); NoteKernelLaunch();
-  VGT_CUDA_TRY(cudaGetLastError(), "MergeFreeAndNamedKernel launch");
   Out min_max[2];
   VGT_CUDA_TRY(cudaMemcpyAsync(h_out, d_free.get(), sizeof(Out) * count, cudaMemcpyDeviceToHost,
                                stream),
@@ -1330,6 +1375,156 @@ int SdfFreeAndNamedHost(const void* h_cells, int cell_bytes, int64_t nx, int64_t
     *out_max = min_max[1];
   }
   return VGT_B200_OK;
+}
+
+// The cell entries on device pointers (vgt_b200_sdf_*_dev): asynchronous on the caller's stream.
+// Every argument is checked before the first device call: the host entries' checks, and the
+// alignment the kernels read and write with.
+template <int kMode>
+int CheckDeviceCellArguments(const void* d_cells, int cell_bytes, int64_t nx, int64_t ny,
+                             int64_t nz, double resolution, const uint32_t* object_ids,
+                             int64_t num_object_ids, const typename OutputOf<kMode>::Type* d_sdf,
+                             const typename OutputOf<kMode>::Type* d_min_max)
+{
+  using Out = typename OutputOf<kMode>::Type;
+  const int check = CheckCellArguments(d_cells, cell_bytes, d_sdf, nx, ny, nz, resolution,
+                                       object_ids, num_object_ids);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  if (reinterpret_cast<uintptr_t>(d_cells) % 4 != 0)
+  {
+    return FailInvalid("cell array must be 4-byte aligned");
+  }
+  if (reinterpret_cast<uintptr_t>(d_sdf) % sizeof(Out) != 0
+      || reinterpret_cast<uintptr_t>(d_min_max) % sizeof(Out) != 0)
+  {
+    return FailInvalid("SDF and min/max arrays must be aligned to their scalar type");
+  }
+  return VGT_B200_OK;
+}
+
+template <int kMode>
+int SdfFromCellsDev(const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                    double resolution, int unknown_is_filled, int add_virtual_border,
+                    const uint32_t* object_ids, int64_t num_object_ids, int device,
+                    typename OutputOf<kMode>::Type* d_sdf,
+                    typename OutputOf<kMode>::Type* d_min_max, cudaStream_t stream)
+{
+  const int check = CheckDeviceCellArguments<kMode>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                                    object_ids, num_object_ids, d_sdf, d_min_max);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  KeepPoolMemory(device);
+  const std::vector<uint32_t> sorted = SortedDistinct(object_ids, num_object_ids);
+  StreamScratch<uint32_t> ids;
+  const int uploaded = UploadIds(sorted, ids, stream);
+  if (uploaded != VGT_B200_OK)
+  {
+    return uploaded;
+  }
+  const int num_ids = static_cast<int>(sorted.size());
+  return SdfFromCellsOnDevice<kMode>(static_cast<const uint32_t*>(d_cells), cell_bytes / 4, nx,
+                                     ny, nz, resolution, unknown_is_filled, add_virtual_border,
+                                     num_ids > 0 ? kListedObjects : kAnyObject, ids.get(),
+                                     num_ids, d_sdf, d_min_max, stream);
+}
+
+// MakeSeparateObjectSDFs on device cells: SDF k of the k-th listed id at d_sdf + k * V, its
+// min/max at d_min_max + 2 k. The distinct ids go in groups of kSlotGroupSize; each group's slot
+// map is built with one read of the cells and serves the SDFs of every listed id in the group.
+template <int kMode>
+int SdfPerObjectDev(const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                    double resolution, int unknown_is_filled, int add_virtual_border,
+                    const uint32_t* object_ids, int64_t num_object_ids, int device,
+                    typename OutputOf<kMode>::Type* d_sdf,
+                    typename OutputOf<kMode>::Type* d_min_max, cudaStream_t stream)
+{
+  using Out = typename OutputOf<kMode>::Type;
+  const int check = CheckDeviceCellArguments<kMode>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                                    object_ids, num_object_ids, d_sdf, d_min_max);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  const int64_t count = nx * ny * nz;
+  if (num_object_ids > 0
+      && count * static_cast<int64_t>(sizeof(Out)) > INT64_MAX / num_object_ids)
+  {
+    return FailInvalid("%lld SDFs of %lld voxels overflow a 64-bit byte count",
+                       static_cast<long long>(num_object_ids), static_cast<long long>(count));
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  if (num_object_ids == 0)
+  {
+    return VGT_B200_OK;
+  }
+  KeepPoolMemory(device);
+  const std::vector<uint32_t> sorted = SortedDistinct(object_ids, num_object_ids);
+  std::vector<int64_t> position(static_cast<size_t>(num_object_ids));
+  for (int64_t k = 0; k < num_object_ids; k++)
+  {
+    position[k] = std::lower_bound(sorted.begin(), sorted.end(), object_ids[k]) - sorted.begin();
+  }
+  StreamScratch<uint8_t> slots;
+  VGT_CUDA_TRY(slots.Allocate(count, stream), "object slot map allocation");
+  const ObjectSlot* const d_slots = reinterpret_cast<const ObjectSlot*>(slots.get());
+  const int threads = 256;
+  const int64_t blocks = std::min<int64_t>((count + threads * 4 - 1) / (threads * 4),
+                                           MultiprocessorCount() * 8);
+  for (int64_t first = 0; first < static_cast<int64_t>(sorted.size()); first += kSlotGroupSize)
+  {
+    SlotGroup group{};
+    group.count = static_cast<int>(
+        std::min<int64_t>(kSlotGroupSize, static_cast<int64_t>(sorted.size()) - first));
+    std::copy(sorted.begin() + first, sorted.begin() + first + group.count, group.ids);
+    CellsToObjectSlotsKernel<<<static_cast<unsigned>(blocks), threads, 0, stream>>>(
+        static_cast<const uint32_t*>(d_cells), cell_bytes / 4, count, unknown_is_filled, group,
+        slots.get()); NoteKernelLaunch();
+    VGT_CUDA_TRY(cudaGetLastError(), "CellsToObjectSlotsKernel launch");
+    for (int64_t k = 0; k < num_object_ids; k++)
+    {
+      if (position[k] < first || position[k] >= first + group.count)
+      {
+        continue;
+      }
+      const int key = static_cast<int>(position[k] - first) + 1;
+      const int status = SdfOnDevice<ObjectSlot, kMode>(
+          d_slots, nx, ny, nz, resolution, key, add_virtual_border, d_sdf + k * count,
+          d_min_max == nullptr ? nullptr : d_min_max + 2 * k, stream);
+      if (status != VGT_B200_OK)
+      {
+        return status;
+      }
+    }
+  }
+  return VGT_B200_OK;
+}
+
+template <int kMode>
+int SdfFreeAndNamedDev(const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                       double resolution, int unknown_is_filled, int add_virtual_border,
+                       int device, typename OutputOf<kMode>::Type* d_sdf,
+                       typename OutputOf<kMode>::Type* d_min_max, cudaStream_t stream)
+{
+  const int check = CheckDeviceCellArguments<kMode>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                                    nullptr, 0, d_sdf, d_min_max);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  KeepPoolMemory(device);
+  return SdfFreeAndNamedOnDevice<kMode>(static_cast<const uint32_t*>(d_cells), cell_bytes / 4, nx,
+                                        ny, nz, resolution, unknown_is_filled, add_virtual_border,
+                                        d_sdf, d_min_max, stream);
 }
 // ------------------------------------------------------------------------------------------------
 // One process, several devices: the slab-sharded path of voxelized_geometry_tools_b200/sharded.py
@@ -2031,6 +2226,70 @@ int vgt_b200_sdf_free_and_named_f64(
   return SdfFreeAndNamedHost<kEmitDouble>(cells, cell_bytes, nx, ny, nz, resolution,
                                           unknown_is_filled, add_virtual_border, device, sdf_out,
                                           out_min, out_max);
+}
+
+int vgt_b200_sdf_from_cells_f32_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, float* d_sdf_out, float* d_min_max, void* stream)
+{
+  return SdfFromCellsDev<kEmitFloat>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, object_ids,
+                                     num_object_ids, device, d_sdf_out, d_min_max,
+                                     static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_sdf_from_cells_f64_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, double* d_sdf_out, double* d_min_max, void* stream)
+{
+  return SdfFromCellsDev<kEmitDouble>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                      unknown_is_filled, add_virtual_border, object_ids,
+                                      num_object_ids, device, d_sdf_out, d_min_max,
+                                      static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_sdf_per_object_f32_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, float* d_sdf_out, float* d_min_max, void* stream)
+{
+  return SdfPerObjectDev<kEmitFloat>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, object_ids,
+                                     num_object_ids, device, d_sdf_out, d_min_max,
+                                     static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_sdf_per_object_f64_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, int device, double* d_sdf_out, double* d_min_max, void* stream)
+{
+  return SdfPerObjectDev<kEmitDouble>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                      unknown_is_filled, add_virtual_border, object_ids,
+                                      num_object_ids, device, d_sdf_out, d_min_max,
+                                      static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_sdf_free_and_named_f32_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, int device, float* d_sdf_out,
+    float* d_min_max, void* stream)
+{
+  return SdfFreeAndNamedDev<kEmitFloat>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                        unknown_is_filled, add_virtual_border, device, d_sdf_out,
+                                        d_min_max, static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_sdf_free_and_named_f64_dev(
+    const void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, int device, double* d_sdf_out,
+    double* d_min_max, void* stream)
+{
+  return SdfFreeAndNamedDev<kEmitDouble>(d_cells, cell_bytes, nx, ny, nz, resolution,
+                                         unknown_is_filled, add_virtual_border, device, d_sdf_out,
+                                         d_min_max, static_cast<cudaStream_t>(stream));
 }
 
 int vgt_b200_edt_transform_inplace_f64(double* field, int64_t nx, int64_t ny, int64_t nz,

@@ -184,6 +184,93 @@ def connected_components(cells: torch.Tensor,
     return num_components
 
 
+# SDF dtype -> suffix of the cell entries' C-ABI names
+_CELL_SDF_SUFFIX = {torch.float32: "f32", torch.float64: "f64"}
+
+
+def _cell_entry(cells: torch.Tensor, dtype: torch.dtype, name: str):
+    if not cells.is_cuda:
+        raise _capi.BackendUnavailable("cells must live on a CUDA device (no CPU fallback)")
+    if cells.dtype not in (torch.int32, torch.uint32) or not cells.is_contiguous():
+        raise ValueError("cells must be a contiguous int32 or uint32 tensor")
+    if cells.dim() != 4 or cells.shape[3] not in (2, 4):
+        raise ValueError("cells must be [nx, ny, nz, 2] or [nx, ny, nz, 4]")
+    if dtype not in _CELL_SDF_SUFFIX:
+        raise ValueError(f"the SDF dtype must be torch.float32 or torch.float64, not {dtype}")
+    return getattr(_capi.library(), f"{name}_{_CELL_SDF_SUFFIX[dtype]}_dev")
+
+
+def _object_ids(object_ids) -> np.ndarray:
+    return np.ascontiguousarray([int(i) for i in object_ids], dtype=np.uint32)
+
+
+def signed_distance_field_from_cells(cells: torch.Tensor, resolution: float, objects_to_use=(),
+                                     unknown_is_filled: bool = True,
+                                     add_virtual_border: bool = False,
+                                     dtype: torch.dtype = torch.float32):
+    """ExtractSignedDistanceField<T> of a cell map that lives on the device
+    (tagged_object_occupancy_map.hpp:199-247; with no objects listed also
+    occupancy_component_map.hpp:270-306). ``cells`` has the layout of
+    ``connected_components``: a contiguous int32 or uint32 tensor [nx, ny, nz, 2 | 4], the
+    occupancy's float bits in word 0 and the object id in word 1. A cell is filled iff the
+    occupancy rule holds and (no objects are listed or its object id is listed). Returns
+    (sdf ``dtype`` [nx, ny, nz], min_max ``dtype`` [2]). Asynchronous."""
+    entry = _cell_entry(cells, dtype, "vgt_b200_sdf_from_cells")
+    ids = _object_ids(objects_to_use)
+    device = cells.device
+    nx, ny, nz, words = cells.shape
+    out = torch.empty((nx, ny, nz), dtype=dtype, device=device)
+    min_max = torch.empty(2, dtype=dtype, device=device)
+    code = entry(cells.data_ptr(), 4 * words, nx, ny, nz, float(resolution),
+                 int(unknown_is_filled), int(add_virtual_border),
+                 ids.ctypes.data if ids.size else None, ids.size, device.index or 0,
+                 out.data_ptr(), min_max.data_ptr(), _stream_handle(device))
+    _capi.check(code)
+    return out, min_max
+
+
+def separate_object_sdfs(cells: torch.Tensor, resolution: float, object_ids,
+                         unknown_is_filled: bool = True, add_virtual_border: bool = False,
+                         dtype: torch.dtype = torch.float32):
+    """MakeSeparateObjectSDFs<T> (tagged_object_occupancy_map.hpp:249-262) of a cell map that
+    lives on the device (``cells`` as in ``signed_distance_field_from_cells``): SDF k is the
+    field of the filled cells whose object id is ``object_ids[k]``. Repeated ids and ids absent
+    from the map are allowed. The cells are read once per 255 distinct ids, not once per object.
+    Returns (sdfs ``dtype`` [K, nx, ny, nz], min_max ``dtype`` [K, 2]). Asynchronous."""
+    entry = _cell_entry(cells, dtype, "vgt_b200_sdf_per_object")
+    ids = _object_ids(object_ids)
+    device = cells.device
+    nx, ny, nz, words = cells.shape
+    out = torch.empty((ids.size, nx, ny, nz), dtype=dtype, device=device)
+    min_max = torch.empty((ids.size, 2), dtype=dtype, device=device)
+    if ids.size == 0:
+        return out, min_max
+    code = entry(cells.data_ptr(), 4 * words, nx, ny, nz, float(resolution),
+                 int(unknown_is_filled), int(add_virtual_border), ids.ctypes.data, ids.size,
+                 device.index or 0, out.data_ptr(), min_max.data_ptr(), _stream_handle(device))
+    _capi.check(code)
+    return out, min_max
+
+
+def free_and_named_objects_sdf(cells: torch.Tensor, resolution: float,
+                               unknown_is_filled: bool = True, add_virtual_border: bool = False,
+                               dtype: torch.dtype = torch.float32):
+    """ExtractFreeAndNamedObjectsSignedDistanceField<T> (tagged_object_occupancy_map.hpp:293-378)
+    of a cell map that lives on the device (``cells`` as in
+    ``signed_distance_field_from_cells``). Returns (sdf ``dtype`` [nx, ny, nz],
+    min_max ``dtype`` [2]). Asynchronous."""
+    entry = _cell_entry(cells, dtype, "vgt_b200_sdf_free_and_named")
+    device = cells.device
+    nx, ny, nz, words = cells.shape
+    out = torch.empty((nx, ny, nz), dtype=dtype, device=device)
+    min_max = torch.empty(2, dtype=dtype, device=device)
+    code = entry(cells.data_ptr(), 4 * words, nx, ny, nz, float(resolution),
+                 int(unknown_is_filled), int(add_virtual_border), device.index or 0,
+                 out.data_ptr(), min_max.data_ptr(), _stream_handle(device))
+    _capi.check(code)
+    return out, min_max
+
+
 def raycast_cloud(points_xyz: torch.Tensor, x_gc, max_range: float, counts: torch.Tensor,
                   voxel_size: float) -> torch.Tensor:
     """Accumulates one cloud (float64 or float32 [N, 3], cloud frame) into counts int32
