@@ -113,6 +113,22 @@ VGT_B200_API int vgt_b200_sdf_f64(
     int unknown_is_filled, int add_virtual_border, int device, double* sdf_out, double* out_min,
     double* out_max);
 
+/* vgt_b200_sdf_f64 on SEVERAL devices of one box (ExtractSignedDistanceFieldDouble,
+ * occupancy_map.cpp:250-254): the x-slab / y-slab cut, the exchange and the rules of
+ * vgt_b200_sdf_f32_multi; the same bytes as vgt_b200_sdf_f64 (field, min and max).
+ *   devices, num_devices   1..8 distinct ordinals in [0, 64), no more than nx or ny;
+ *                          1 device = vgt_b200_sdf_f64.
+ *   Device memory, per slab on its device: 4 B per voxel of its x-slab for the occupancy and 4 B
+ *   per voxel for the local-pass scratch; a receive buffer of 4 * nx * ceil(ny / num_devices) * nz
+ *   bytes, kept for the life of the process; 8 B per voxel of its y-slab for the SDF; a magnitude
+ *   table of at most 8 MB.
+ * Every argument, the device list included, is checked before the first device call. Fails with
+ * VGT_B200_ERR_DEVICE when two of the devices cannot reach each other as peers (no fallback). */
+VGT_B200_API int vgt_b200_sdf_f64_multi(
+    const float* occupancy, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max);
+
 /* For grids whose filled predicate is an opaque std::function (the other map types,
  * include/.../signed_distance_field_generation.hpp:115-121): the adapter evaluates the predicate
  * on the host into filled_mask (uint8, non-zero = filled) and calls this. */
@@ -173,6 +189,66 @@ VGT_B200_API int vgt_b200_sdf_free_and_named_f64(
     const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
     int unknown_is_filled, int add_virtual_border, int device, double* sdf_out, double* out_min,
     double* out_max);
+
+/* The three cell entries above on SEVERAL devices of one box, for maps one device cannot hold;
+ * they replace the same reference code (tagged_object_occupancy_map.hpp:199-262, :293-378,
+ * occupancy_component_map.hpp:270-306). Each takes the argument list of its host entry with
+ * `int device` replaced by `devices, num_devices`, and follows vgt_b200_sdf_f32_multi: slab g
+ * of the cells (x-slab) is uploaded to devices[g] once and classified there, the z and y passes
+ * run slab-local with the exchange fused into the y pass (peer stores), and the x pass + finalize
+ * runs on y-slab g. The result is the same bytes as the host entry: every field and min/max pair.
+ *   devices, num_devices   1..8 distinct ordinals in [0, 64), no more than nx or ny;
+ *                          1 device = the host entry.
+ *   vgt_b200_sdf_from_cells_*_multi     one round: the filled mask, the passes.
+ *   vgt_b200_sdf_free_and_named_*_multi two rounds on the resident cell slab (all filled cells,
+ *                                       then named objects), merged on each y-slab.
+ *   vgt_b200_sdf_per_object_*_multi     one round per listed id; the slab is classified once per
+ *                                       group of 255 distinct ids (the slot map of the _dev
+ *                                       batch). sdf_out is T[num_object_ids][nx*ny*nz], out_min /
+ *                                       out_max one value per listed id. Repeated ids and ids
+ *                                       absent from the map are allowed; num_object_ids == 0
+ *                                       launches nothing. num_object_ids * nx*ny*nz * sizeof(T)
+ *                                       beyond int64 is refused.
+ *   Device memory, per slab on its device: its x-slab of cells (cell_bytes per voxel), 1 B per
+ *   voxel of the x-slab for the mask (the slot map of the batch) and 4 B for the local-pass
+ *   scratch; a receive buffer of 4 * nx * ceil(ny / num_devices) * nz bytes, kept for the life
+ *   of the process; sizeof(T) per voxel of its y-slab for the SDF (two y-slabs for
+ *   free-and-named); a magnitude table of at most 4 / 8 MB.
+ * Every argument, the device list included, is checked before the first device call. Fails with
+ * VGT_B200_ERR_DEVICE when two of the devices cannot reach each other as peers (no fallback). */
+VGT_B200_API int vgt_b200_sdf_from_cells_f32_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    float* sdf_out, float* out_min, float* out_max);
+
+VGT_B200_API int vgt_b200_sdf_from_cells_f64_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max);
+
+VGT_B200_API int vgt_b200_sdf_per_object_f32_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    float* sdf_out, float* out_min, float* out_max);
+
+VGT_B200_API int vgt_b200_sdf_per_object_f64_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max);
+
+VGT_B200_API int vgt_b200_sdf_free_and_named_f32_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
+    float* sdf_out, float* out_min, float* out_max);
+
+VGT_B200_API int vgt_b200_sdf_free_and_named_f64_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max);
 
 /* The three cell entries above on a map that lives on the device; they replace the same reference
  * code (tagged_object_occupancy_map.hpp:199-262, :293-378, occupancy_component_map.hpp:270-306).

@@ -84,6 +84,8 @@ SIGNATURES = {
     "vgt_b200_sdf_f32_multi": (_int, [_vp, _i64, _i64, _i64, _dbl, _int, _int,
                                       ctypes.POINTER(ctypes.c_int), _int, _vp, _f32p, _f32p]),
     "vgt_b200_sdf_f64": (_int, [_vp, _i64, _i64, _i64, _dbl, _int, _int, _int, _vp, _f64p, _f64p]),
+    "vgt_b200_sdf_f64_multi": (_int, [_vp, _i64, _i64, _i64, _dbl, _int, _int,
+                                      ctypes.POINTER(ctypes.c_int), _int, _vp, _f64p, _f64p]),
     "vgt_b200_sdf_from_mask_f32": (_int, [_vp, _i64, _i64, _i64, _dbl, _int, _int, _vp, _f32p,
                                           _f32p]),
     "vgt_b200_sdf_from_mask_f64": (_int, [_vp, _i64, _i64, _i64, _dbl, _int, _int, _vp, _f64p,
@@ -100,6 +102,18 @@ SIGNATURES = {
                                                _vp, _f32p, _f32p]),
     "vgt_b200_sdf_free_and_named_f64": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _int,
                                                _vp, _f64p, _f64p]),
+    "vgt_b200_sdf_from_cells_f32_multi": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _vp, _i64,
+                                                 ctypes.POINTER(ctypes.c_int), _int, _vp, _f32p, _f32p]),
+    "vgt_b200_sdf_from_cells_f64_multi": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _vp, _i64,
+                                                 ctypes.POINTER(ctypes.c_int), _int, _vp, _f64p, _f64p]),
+    "vgt_b200_sdf_per_object_f32_multi": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _vp, _i64,
+                                                 ctypes.POINTER(ctypes.c_int), _int, _vp, _vp, _vp]),
+    "vgt_b200_sdf_per_object_f64_multi": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _vp, _i64,
+                                                 ctypes.POINTER(ctypes.c_int), _int, _vp, _vp, _vp]),
+    "vgt_b200_sdf_free_and_named_f32_multi": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int,
+                                                     ctypes.POINTER(ctypes.c_int), _int, _vp, _f32p, _f32p]),
+    "vgt_b200_sdf_free_and_named_f64_multi": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int,
+                                                     ctypes.POINTER(ctypes.c_int), _int, _vp, _f64p, _f64p]),
     "vgt_b200_sdf_from_cells_f32_dev": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _vp,
                                                _i64, _int, _vp, _vp, _vp]),
     "vgt_b200_sdf_from_cells_f64_dev": (_int, [_vp, _int, _i64, _i64, _i64, _dbl, _int, _int, _vp,

@@ -37,7 +37,7 @@ namespace b200
 {
 namespace detail
 {
-// (float / double overloads over the C-ABI pairs)
+// (float / double overloads over the C-ABI pairs; `int device` or a device list)
 inline int CallCells(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
                      double resolution, bool unknown_is_filled, bool border,
                      const uint32_t* ids, int64_t num_ids, int device, float* out, float* lo,
@@ -90,6 +90,61 @@ inline int CallFreeAndNamed(const void* cells, int cell_bytes, int64_t nx, int64
                                          unknown_is_filled ? 1 : 0, border ? 1 : 0, device, out,
                                          lo, hi);
 }
+// the same over the multi-device entries, the device list in place of `device`
+inline int CallCells(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                     double resolution, bool unknown_is_filled, bool border,
+                     const uint32_t* ids, int64_t num_ids, const std::vector<int>& devices,
+                     float* out, float* lo, float* hi)
+{
+  return vgt_b200_sdf_from_cells_f32_multi(
+      cells, cell_bytes, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
+      ids, num_ids, devices.data(), static_cast<int>(devices.size()), out, lo, hi);
+}
+inline int CallCells(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                     double resolution, bool unknown_is_filled, bool border,
+                     const uint32_t* ids, int64_t num_ids, const std::vector<int>& devices,
+                     double* out, double* lo, double* hi)
+{
+  return vgt_b200_sdf_from_cells_f64_multi(
+      cells, cell_bytes, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
+      ids, num_ids, devices.data(), static_cast<int>(devices.size()), out, lo, hi);
+}
+inline int CallPerObject(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                         double resolution, bool unknown_is_filled, bool border,
+                         const uint32_t* ids, int64_t num_ids, const std::vector<int>& devices,
+                         float* out, float* lo, float* hi)
+{
+  return vgt_b200_sdf_per_object_f32_multi(
+      cells, cell_bytes, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
+      ids, num_ids, devices.data(), static_cast<int>(devices.size()), out, lo, hi);
+}
+inline int CallPerObject(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                         double resolution, bool unknown_is_filled, bool border,
+                         const uint32_t* ids, int64_t num_ids, const std::vector<int>& devices,
+                         double* out, double* lo, double* hi)
+{
+  return vgt_b200_sdf_per_object_f64_multi(
+      cells, cell_bytes, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
+      ids, num_ids, devices.data(), static_cast<int>(devices.size()), out, lo, hi);
+}
+inline int CallFreeAndNamed(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                            double resolution, bool unknown_is_filled, bool border,
+                            const std::vector<int>& devices,
+                            float* out, float* lo, float* hi)
+{
+  return vgt_b200_sdf_free_and_named_f32_multi(
+      cells, cell_bytes, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
+      devices.data(), static_cast<int>(devices.size()), out, lo, hi);
+}
+inline int CallFreeAndNamed(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
+                            double resolution, bool unknown_is_filled, bool border,
+                            const std::vector<int>& devices,
+                            double* out, double* lo, double* hi)
+{
+  return vgt_b200_sdf_free_and_named_f64_multi(
+      cells, cell_bytes, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
+      devices.data(), static_cast<int>(devices.size()), out, lo, hi);
+}
 
 template <typename MapType>
 struct CellsOf
@@ -120,10 +175,14 @@ inline void FinishSdf(SignedDistanceField<ScalarType>& sdf, ScalarType minimum, 
 
 // ExtractSignedDistanceField<T>(objects_to_use, parameters) of the tagged maps; with an empty
 // list (or for OccupancyComponentMap, which has no object ids) every filled cell counts.
-template <typename MapType, typename ScalarType>
+// `device` of each function below: one ordinal (int), or a std::vector<int> of several, which
+// cuts the map into one x-slab per device (the *_multi entries) for maps one device cannot
+// hold, with the same result.
+template <typename MapType, typename ScalarType, typename Devices = int>
 inline SignedDistanceField<ScalarType> ExtractSignedDistanceFieldFromCellMap(
     const MapType& map, const std::vector<uint32_t>& objects_to_use,
-    const SignedDistanceFieldGenerationParameters<ScalarType>& parameters, const int device = 0)
+    const SignedDistanceFieldGenerationParameters<ScalarType>& parameters,
+    const Devices& device = 0)
 {
   detail::RequireUniform(map);
   SignedDistanceField<ScalarType> sdf(map.OriginTransform(), map.Frame(), map.ControlSizes(),
@@ -141,10 +200,11 @@ inline SignedDistanceField<ScalarType> ExtractSignedDistanceFieldFromCellMap(
 }
 
 // MakeSeparateObjectSDFs<T>(object_ids, parameters): the cells are uploaded once, one SDF per id.
-template <typename MapType, typename ScalarType>
+template <typename MapType, typename ScalarType, typename Devices = int>
 inline std::map<uint32_t, SignedDistanceField<ScalarType>> MakeSeparateObjectSDFs(
     const MapType& map, const std::vector<uint32_t>& object_ids,
-    const SignedDistanceFieldGenerationParameters<ScalarType>& parameters, const int device = 0)
+    const SignedDistanceFieldGenerationParameters<ScalarType>& parameters,
+    const Devices& device = 0)
 {
   detail::RequireUniform(map);
   std::map<uint32_t, SignedDistanceField<ScalarType>> per_object_sdfs;
@@ -176,10 +236,10 @@ inline std::map<uint32_t, SignedDistanceField<ScalarType>> MakeSeparateObjectSDF
 
 // MakeAllObjectSDFs<T>(parameters): every object id > 0 present in the map
 // (tagged_object_occupancy_map.hpp:264-291).
-template <typename MapType, typename ScalarType>
+template <typename MapType, typename ScalarType, typename Devices = int>
 inline std::map<uint32_t, SignedDistanceField<ScalarType>> MakeAllObjectSDFs(
     const MapType& map, const SignedDistanceFieldGenerationParameters<ScalarType>& parameters,
-    const int device = 0)
+    const Devices& device = 0)
 {
   std::set<uint32_t> present;
   for (const auto& cell : map.GetImmutableRawData())
@@ -189,16 +249,16 @@ inline std::map<uint32_t, SignedDistanceField<ScalarType>> MakeAllObjectSDFs(
       present.insert(cell.ObjectId());
     }
   }
-  return MakeSeparateObjectSDFs<MapType, ScalarType>(
+  return MakeSeparateObjectSDFs<MapType, ScalarType, Devices>(
       map, std::vector<uint32_t>(present.begin(), present.end()), parameters, device);
 }
 
 // ExtractFreeAndNamedObjectsSignedDistanceField<T>(parameters): both SDFs and the merge on the
 // device (tagged_object_occupancy_map.hpp:293-378).
-template <typename MapType, typename ScalarType>
+template <typename MapType, typename ScalarType, typename Devices = int>
 inline SignedDistanceField<ScalarType> ExtractFreeAndNamedObjectsSignedDistanceField(
     const MapType& map, const SignedDistanceFieldGenerationParameters<ScalarType>& parameters,
-    const int device = 0)
+    const Devices& device = 0)
 {
   detail::RequireUniform(map);
   SignedDistanceField<ScalarType> sdf(map.OriginTransform(), map.Frame(), map.ControlSizes(),

@@ -111,6 +111,22 @@ inline int CallOccupancy(const float* occ, int64_t nx, int64_t ny, int64_t nz, d
   return vgt_b200_sdf_f64(occ, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0, border ? 1 : 0,
                           device, out, lo, hi);
 }
+inline int CallOccupancy(const float* occ, int64_t nx, int64_t ny, int64_t nz, double resolution,
+                         bool unknown_is_filled, bool border, const std::vector<int>& devices,
+                         float* out, float* lo, float* hi)
+{
+  return vgt_b200_sdf_f32_multi(occ, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0,
+                                border ? 1 : 0, devices.data(), static_cast<int>(devices.size()),
+                                out, lo, hi);
+}
+inline int CallOccupancy(const float* occ, int64_t nx, int64_t ny, int64_t nz, double resolution,
+                         bool unknown_is_filled, bool border, const std::vector<int>& devices,
+                         double* out, double* lo, double* hi)
+{
+  return vgt_b200_sdf_f64_multi(occ, nx, ny, nz, resolution, unknown_is_filled ? 1 : 0,
+                                border ? 1 : 0, devices.data(), static_cast<int>(devices.size()),
+                                out, lo, hi);
+}
 }  // namespace detail
 
 // Drop-in for internal::ExtractSignedDistanceField(grid, is_filled_fn, frame, parameters)
@@ -183,11 +199,12 @@ inline SignedDistanceField<SDFScalarType> ExtractSignedDistanceFieldFromOccupanc
   FinishAndLock(new_sdf, minimum, maximum);
   return new_sdf;
 }
-// The same on several devices of the box (vgt_b200_sdf_f32_multi: x-slabs, one per device, the
-// exchange fused into the y pass as NVLink peer stores). SignedDistanceField<float> only.
-template <typename OccupancyMapType>
-inline SignedDistanceField<float> ExtractSignedDistanceFieldFromOccupancyMap(
-    const OccupancyMapType& map, const SignedDistanceFieldGenerationParameters<float>& parameters,
+// The same on several devices of the box (vgt_b200_sdf_f32_multi / vgt_b200_sdf_f64_multi:
+// x-slabs, one per device, the exchange fused into the y pass as NVLink peer stores).
+template <typename OccupancyMapType, typename SDFScalarType>
+inline SignedDistanceField<SDFScalarType> ExtractSignedDistanceFieldFromOccupancyMap(
+    const OccupancyMapType& map,
+    const SignedDistanceFieldGenerationParameters<SDFScalarType>& parameters,
     const std::vector<int>& devices)
 {
   if (!map.HasUniformVoxelSize())
@@ -195,14 +212,14 @@ inline SignedDistanceField<float> ExtractSignedDistanceFieldFromOccupancyMap(
     throw std::invalid_argument("Grid must have uniform resolution");
   }
   const float* occupancy = reinterpret_cast<const float*>(map.GetImmutableRawData().data());
-  SignedDistanceField<float> new_sdf(
+  SignedDistanceField<SDFScalarType> new_sdf(
       map.OriginTransform(), map.Frame(), map.ControlSizes(), parameters.OOBValue());
-  float minimum = 0;
-  float maximum = 0;
-  ThrowOnError(vgt_b200_sdf_f32_multi(
+  SDFScalarType minimum = 0;
+  SDFScalarType maximum = 0;
+  ThrowOnError(detail::CallOccupancy(
       occupancy, map.NumXVoxels(), map.NumYVoxels(), map.NumZVoxels(), map.VoxelXSize(),
-      parameters.UnknownIsFilled() ? 1 : 0, parameters.AddVirtualBorder() ? 1 : 0, devices.data(),
-      static_cast<int>(devices.size()), new_sdf.GetMutableRawData().data(), &minimum, &maximum));
+      parameters.UnknownIsFilled(), parameters.AddVirtualBorder(), devices,
+      new_sdf.GetMutableRawData().data(), &minimum, &maximum));
   FinishAndLock(new_sdf, minimum, maximum);
   return new_sdf;
 }

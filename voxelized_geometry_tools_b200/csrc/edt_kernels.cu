@@ -1528,22 +1528,98 @@ int SdfFreeAndNamedDev(const void* d_cells, int cell_bytes, int64_t nx, int64_t 
 }
 // ------------------------------------------------------------------------------------------------
 // One process, several devices: the slab-sharded path of voxelized_geometry_tools_b200/sharded.py
-// behind one C call, so that a C++ caller of OccupancyMap::ExtractSignedDistanceField can use
-// every GPU of the box. One host thread per device runs that device's share: upload of its
-// x-slab, z scan + y pass with the exchange fused in (peer stores into the other devices'
-// receive buffers: cudaMalloc memory with peer access enabled), a barrier between the threads
-// once every stream has drained, x pass + finalize on its y-slab, strided copy of the y-slab
-// into its place in the caller's grid.
+// behind one C call, so that a C++ caller of the SDF members can use every GPU of the box, and a
+// map that one device cannot hold gets its SDF. One host thread per device runs that device's
+// share: upload of its x-slab, z scan + y pass with the exchange fused in (peer stores into the
+// other devices' receive buffers: cudaMalloc memory with peer access enabled), a barrier between
+// the threads once every stream has drained, x pass + finalize on its y-slab, strided copy of the
+// y-slab into its place in the caller's grid. A call runs one or more such rounds on the same
+// resident input slab (free-and-named: two; the per-object batch: one per listed id).
 // ------------------------------------------------------------------------------------------------
-int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double resolution,
-                   int unknown_is_filled, int add_virtual_border, const int* devices,
-                   int num_devices, float* h_out, float* out_min, float* out_max)
+
+// The grid of a multi-device call and its cut: x-slab g of the input and y-slab g of the result
+// belong to devices[g].
+struct MultiGrid
 {
-  const int check = CheckSdfArguments(h_in, h_out, nx, ny, nz, resolution);
-  if (check != VGT_B200_OK)
+  int64_t nx, ny, nz;
+  double resolution;
+  int add_virtual_border;
+  int num_devices;
+  int64_t Plane() const { return ny * nz; }
+};
+
+// What the per-slab steps of one device see.
+struct SlabPart
+{
+  int index;
+  int64_t x0, x1, y0, y1;
+  cudaStream_t stream;
+  StagedTransfer* transfer;
+  uint32_t* scratch;            // 4 bytes per voxel of the x-slab, the z scan's output
+  const uint64_t* peer_bases;   // every device's receive buffer
+  int64_t Voxels(const MultiGrid& grid) const { return (x1 - x0) * grid.Plane(); }
+};
+
+// z scan of the part's input slab, then the y pass, whose output goes straight into every
+// device's receive buffer.
+template <typename In>
+int ExchangeLocalPasses(const In* d_slab, int unknown_is_filled, const MultiGrid& grid,
+                        const SlabPart& part)
+{
+  return RunLocalPasses<In>(d_slab, part.x1 - part.x0, grid.ny, grid.nz, unknown_is_filled,
+                            part.scratch, part.scratch, part.stream, grid.num_devices,
+                            part.peer_bases, part.x0, part.index);
+}
+
+// y-slab [nx][rows][nz] -> rows [y0, y1) of the caller's [nx][ny][nz] grid (a strided 2-D
+// copy), and the slab's min/max into h_min_max[2]. Both land when the stream has drained.
+template <typename Out>
+int CopySlabToHost(const Out* d_slab, const Out* d_min_max, const MultiGrid& grid,
+                   const SlabPart& part, Out* h_grid, Out* h_min_max)
+{
+  const int64_t rows = part.y1 - part.y0;
+  VGT_CUDA_TRY(part.transfer->ToHost(reinterpret_cast<char*>(h_grid + part.y0 * grid.nz),
+                                     sizeof(Out) * static_cast<size_t>(grid.Plane()),
+                                     reinterpret_cast<const char*>(d_slab),
+                                     sizeof(Out) * static_cast<size_t>(rows * grid.nz),
+                                     sizeof(Out) * static_cast<size_t>(rows * grid.nz),
+                                     static_cast<size_t>(grid.nx), part.stream),
+               "copy SDF slab to host");
+  VGT_CUDA_TRY(cudaMemcpyAsync(h_min_max, d_min_max, sizeof(Out) * 2, cudaMemcpyDeviceToHost,
+                               part.stream),
+               "copy min/max to host");
+  return VGT_B200_OK;
+}
+
+// extrema: [result][device][min, max] -> out_min[result], out_max[result] (either may be null).
+template <typename Out>
+void CombineExtrema(const std::vector<Out>& extrema, int num_devices, int64_t results,
+                    Out* out_min, Out* out_max)
+{
+  for (int64_t k = 0; k < results; k++)
   {
-    return check;
+    const Out* row = extrema.data() + 2 * k * num_devices;
+    Out low = row[0];
+    Out high = row[1];
+    for (int g = 1; g < num_devices; g++)
+    {
+      low = std::min(low, row[2 * g]);
+      high = std::max(high, row[2 * g + 1]);
+    }
+    if (out_min != nullptr)
+    {
+      out_min[k] = low;
+    }
+    if (out_max != nullptr)
+    {
+      out_max[k] = high;
+    }
   }
+}
+
+// 1..8 distinct devices.
+int CheckDeviceList(const int* devices, int num_devices)
+{
   if (devices == nullptr || num_devices < 1 || num_devices > 8)
   {
     return FailInvalid("1..8 devices are supported");
@@ -1558,15 +1634,46 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
       }
     }
   }
-  if (num_devices == 1)
+  return VGT_B200_OK;
+}
+
+// The cell and double entries also refuse an ordinal outside [0, 64) (the receive-buffer cache's
+// range) before any device call.
+int CheckMultiDeviceList(const int* devices, int num_devices, int64_t nx, int64_t ny)
+{
+  const int check = CheckDeviceList(devices, num_devices);
+  if (check != VGT_B200_OK)
   {
-    return SdfFromHost<float, kEmitFloat>(h_in, nx, ny, nz, resolution, unknown_is_filled,
-                                          add_virtual_border, devices[0], h_out, out_min, out_max);
+    return check;
   }
-  if (num_devices > nx || num_devices > ny)
+  for (int g = 0; g < num_devices; g++)
+  {
+    if (devices[g] < 0 || devices[g] >= 64)
+    {
+      return FailInvalid("device ordinal %d out of range", devices[g]);
+    }
+  }
+  if (num_devices > 1 && (num_devices > nx || num_devices > ny))
   {
     return FailInvalid("more devices than voxels along x or y");
   }
+  return VGT_B200_OK;
+}
+
+// The driver of every multi-device entry. Work supplies the per-slab steps:
+//   typename Work::Slab                      per-device state, built on that device's thread
+//   int Local(Slab&, const SlabPart&, r)     enqueue the input of round r and the local passes
+//                                            (ExchangeLocalPasses)
+//   bool FinalMinMax(r)                      whether the final pass of round r reduces min/max
+//   int Emit(Slab&, const SlabPart&, r, Out* const* d_slabs, Out* d_min_max)
+//                                            what becomes of the y-slab of round r
+//   int slab_buffers                         y-slabs kept (round r writes d_slabs[r % count])
+// The driver synchronises the stream after Local and after Emit.
+template <int kMode, typename Work>
+int SdfMultiDevice(const MultiGrid& grid, const int* devices, int64_t rounds, const Work& job)
+{
+  using Out = typename OutputOf<kMode>::Type;
+  const int num_devices = grid.num_devices;
   // Peer access between every pair (a one-time, process-wide driver setting; "already enabled"
   // is fine). Without it the fused exchange cannot run: no silent fallback.
   for (int a = 0; a < num_devices; a++)
@@ -1594,9 +1701,8 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
       cudaGetLastError();
     }
   }
-  const int64_t plane = ny * nz;
-  const int64_t widest_part = (ny + num_devices - 1) / num_devices;
-  const int64_t receive_words = nx * widest_part * nz;
+  const int64_t widest_part = (grid.ny + num_devices - 1) / num_devices;
+  const int64_t receive_words = grid.nx * widest_part * grid.nz;
   // Receive buffers: plain cudaMalloc (peer-mapped once access is enabled; pool memory would
   // need per-pool access grants). cudaMalloc / cudaFree of half a gigabyte per device and call
   // costs more than the passes, so one buffer per device is kept for the life of the process
@@ -1640,8 +1746,6 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
   ThreadBarrier barrier(num_devices);
   std::vector<int> statuses(static_cast<size_t>(num_devices), VGT_B200_OK);
   std::vector<std::string> messages(static_cast<size_t>(num_devices));
-  std::vector<float> minima(static_cast<size_t>(num_devices));
-  std::vector<float> maxima(static_cast<size_t>(num_devices));
   std::atomic<int> failed{0};
 
   const auto worker = [&](const int g)
@@ -1649,14 +1753,16 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
     int status = VGT_B200_OK;
     const int device = devices[g];
     ScopedDevice scoped(device);
-    int64_t x0, x1, y0, y1;
-    SplitRange(nx, num_devices, g, &x0, &x1);
-    SplitRange(ny, num_devices, g, &y0, &y1);
+    SlabPart part{};
+    part.index = g;
+    SplitRange(grid.nx, num_devices, g, &part.x0, &part.x1);
+    SplitRange(grid.ny, num_devices, g, &part.y0, &part.y1);
+    part.peer_bases = peer_bases.data();
     StreamGuard guard;
-    StreamScratch<float> d_occupancy;
     StreamScratch<uint32_t> d_scratch;
-    StreamScratch<float> d_sdf;
-    StreamScratch<float> d_min_max;
+    StreamScratch<Out> d_slabs[2];
+    StreamScratch<Out> d_min_max;
+    typename Work::Slab slab;
     StagedTransfer transfer;
     if (num_devices >= 6)
     {
@@ -1664,6 +1770,7 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
       // serve one caller at a time); with fewer devices the shared workers copy faster
       transfer.UseCallingThreadOnly();
     }
+    part.transfer = &transfer;
     // (runs first on every exit path: nothing is queued when the buffers are released)
     struct DrainOnExit
     {
@@ -1676,79 +1783,104 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
         }
       }
     } drain{guard};
-    // Up to the barrier: every thread must reach it, whatever happens before.
-    const auto local_passes = [&]() -> int
+    const auto local_passes = [&](int64_t round) -> int
     {
-      VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
-      KeepPoolMemory(device);
-      VGT_CUDA_TRY(cudaStreamCreateWithFlags(&guard.stream, cudaStreamNonBlocking), "stream");
-      const int64_t slab_voxels = (x1 - x0) * plane;
-      VGT_CUDA_TRY(d_occupancy.Allocate(slab_voxels, guard.stream), "occupancy slab allocation");
-      VGT_CUDA_TRY(d_scratch.Allocate(slab_voxels, guard.stream), "local pass scratch allocation");
-      const size_t slab_bytes = sizeof(float) * static_cast<size_t>(slab_voxels);
-      VGT_CUDA_TRY(transfer.ToDevice(reinterpret_cast<char*>(d_occupancy.get()), slab_bytes,
-                                     reinterpret_cast<const char*>(h_in + x0 * plane), slab_bytes,
-                                     slab_bytes, 1, guard.stream),
-                   "copy occupancy slab to device");
-      const int local = RunLocalPasses<float>(d_occupancy.get(), x1 - x0, ny, nz,
-                                              unknown_is_filled, d_scratch.get(), d_scratch.get(),
-                                              guard.stream, num_devices, peer_bases.data(), x0, g);
+      if (round == 0)
+      {
+        VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+        KeepPoolMemory(device);
+        VGT_CUDA_TRY(cudaStreamCreateWithFlags(&guard.stream, cudaStreamNonBlocking), "stream");
+        part.stream = guard.stream;
+        VGT_CUDA_TRY(d_scratch.Allocate(part.Voxels(grid), part.stream),
+                     "local pass scratch allocation");
+        part.scratch = d_scratch.get();
+      }
+      const int local = job.Local(slab, part, round);
       if (local != VGT_B200_OK)
       {
         return local;
       }
-      VGT_CUDA_TRY(cudaStreamSynchronize(guard.stream), "slab-local passes");
+      VGT_CUDA_TRY(cudaStreamSynchronize(part.stream), "slab-local passes");
       return VGT_B200_OK;
     };
-    const auto final_pass = [&]() -> int
+    const auto final_pass = [&](int64_t round) -> int
     {
-      cudaStream_t stream = guard.stream;
-      const int64_t rows = y1 - y0;
-      VGT_CUDA_TRY(d_sdf.Allocate(nx * rows * nz, stream), "SDF slab allocation");
-      VGT_CUDA_TRY(d_min_max.Allocate(2, stream), "min/max allocation");
-      const int final_status = RunFinalPass<kEmitFloat>(
-          receive[static_cast<size_t>(g)], nx, rows, nz, y0, ny, resolution, add_virtual_border,
-          d_sdf.get(), d_min_max.get(), stream);
+      const int64_t rows = part.y1 - part.y0;
+      StreamScratch<Out>& target = d_slabs[round % job.slab_buffers];
+      if (target.get() == nullptr)
+      {
+        VGT_CUDA_TRY(target.Allocate(grid.nx * rows * grid.nz, part.stream),
+                     "SDF slab allocation");
+      }
+      if (d_min_max.get() == nullptr)
+      {
+        VGT_CUDA_TRY(d_min_max.Allocate(2, part.stream), "min/max allocation");
+      }
+      const int final_status = RunFinalPass<kMode>(
+          receive[static_cast<size_t>(g)], grid.nx, rows, grid.nz, part.y0, grid.ny,
+          grid.resolution, grid.add_virtual_border, target.get(),
+          job.FinalMinMax(round) ? d_min_max.get() : nullptr, part.stream);
       if (final_status != VGT_B200_OK)
       {
         return final_status;
       }
-      // y-slab [nx][rows][nz] -> rows of the caller's [nx][ny][nz] grid (a strided 2-D copy)
-      VGT_CUDA_TRY(transfer.ToHost(reinterpret_cast<char*>(h_out + y0 * nz),
-                                   sizeof(float) * static_cast<size_t>(plane),
-                                   reinterpret_cast<const char*>(d_sdf.get()),
-                                   sizeof(float) * static_cast<size_t>(rows * nz),
-                                   sizeof(float) * static_cast<size_t>(rows * nz),
-                                   static_cast<size_t>(nx), stream),
-                   "copy SDF slab to host");
-      float min_max[2];
-      VGT_CUDA_TRY(cudaMemcpyAsync(min_max, d_min_max.get(), sizeof(min_max),
-                                   cudaMemcpyDeviceToHost, stream),
-                   "copy min/max to host");
-      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "SDF generation");
-      minima[static_cast<size_t>(g)] = min_max[0];
-      maxima[static_cast<size_t>(g)] = min_max[1];
+      Out* const slabs[2] = {d_slabs[0].get(), d_slabs[1].get()};
+      const int emitted = job.Emit(slab, part, round, slabs, d_min_max.get());
+      if (emitted != VGT_B200_OK)
+      {
+        return emitted;
+      }
+      VGT_CUDA_TRY(cudaStreamSynchronize(part.stream), "SDF generation");
       return VGT_B200_OK;
     };
-    status = local_passes();
-    if (status != VGT_B200_OK)
+    const auto fail = [&](int code)
     {
+      status = code;
       messages[static_cast<size_t>(g)] = vgt_b200_last_error();  // thread-local text
       failed.store(1);
-    }
-    // every device's stores into every receive buffer have landed
-    barrier.Wait();
-    if (status == VGT_B200_OK && failed.load() != 0)
+    };
+    const auto stand_down = [&]()
     {
       status = VGT_B200_ERR_DEVICE;
       messages[static_cast<size_t>(g)] = "another device failed";
-    }
-    else if (status == VGT_B200_OK)
+    };
+    // Every thread reaches every barrier, whatever has failed before.
+    for (int64_t round = 0; round < rounds; round++)
     {
-      status = final_pass();
-      if (status != VGT_B200_OK)
+      if (status == VGT_B200_OK && failed.load() != 0)
       {
-        messages[static_cast<size_t>(g)] = vgt_b200_last_error();
+        stand_down();
+      }
+      if (status == VGT_B200_OK)
+      {
+        const int local = local_passes(round);
+        if (local != VGT_B200_OK)
+        {
+          fail(local);
+        }
+      }
+      // every device's stores into every receive buffer have landed
+      barrier.Wait();
+      if (status == VGT_B200_OK && failed.load() != 0)
+      {
+        stand_down();
+      }
+      else if (status == VGT_B200_OK)
+      {
+        const int final_status = final_pass(round);
+        if (final_status != VGT_B200_OK)
+        {
+          fail(final_status);
+        }
+      }
+      // The exchange of round r + 1 stores into the other devices' receive buffers, which their
+      // final pass of round r reads. One receive buffer per device and this barrier, rather than
+      // two buffers used alternately: the receive buffer is the largest allocation after the
+      // cells, and final_pass has drained its stream (the copy-out waits for it anyway), so the
+      // barrier costs no more than the slowest device's final pass.
+      if (round + 1 < rounds)
+      {
+        barrier.Wait();
       }
     }
     statuses[static_cast<size_t>(g)] = status;
@@ -1776,14 +1908,327 @@ int SdfMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz, double
       }
     }
   }
-  if (out_min != nullptr)
+  return VGT_B200_OK;
+}
+
+// OccupancyMap: the float occupancy slab, one round.
+template <int kMode>
+struct OccupancySlabs
+{
+  using Out = typename OutputOf<kMode>::Type;
+  struct Slab
   {
-    *out_min = *std::min_element(minima.begin(), minima.end());
-  }
-  if (out_max != nullptr)
+    StreamScratch<float> occupancy;
+  };
+  MultiGrid grid;
+  const float* h_in;
+  int unknown_is_filled;
+  Out* h_out;
+  mutable std::vector<Out> extrema;  // [device][min, max]
+  int slab_buffers = 1;
+
+  int Local(Slab& slab, const SlabPart& part, int64_t) const
   {
-    *out_max = *std::max_element(maxima.begin(), maxima.end());
+    const int64_t voxels = part.Voxels(grid);
+    VGT_CUDA_TRY(slab.occupancy.Allocate(voxels, part.stream), "occupancy slab allocation");
+    const size_t bytes = sizeof(float) * static_cast<size_t>(voxels);
+    VGT_CUDA_TRY(part.transfer->ToDevice(reinterpret_cast<char*>(slab.occupancy.get()), bytes,
+                                         reinterpret_cast<const char*>(h_in
+                                                                       + part.x0 * grid.Plane()),
+                                         bytes, bytes, 1, part.stream),
+                 "copy occupancy slab to device");
+    return ExchangeLocalPasses<float>(slab.occupancy.get(), unknown_is_filled, grid, part);
   }
+  bool FinalMinMax(int64_t) const { return true; }
+  int Emit(Slab&, const SlabPart& part, int64_t, Out* const* d_slabs, Out* d_min_max) const
+  {
+    return CopySlabToHost(d_slabs[0], d_min_max, grid, part, h_out,
+                          extrema.data() + 2 * part.index);
+  }
+};
+
+template <int kMode>
+int SdfOccupancyMultiDevice(const float* h_in, int64_t nx, int64_t ny, int64_t nz,
+                            double resolution, int unknown_is_filled, int add_virtual_border,
+                            const int* devices, int num_devices,
+                            typename OutputOf<kMode>::Type* h_out,
+                            typename OutputOf<kMode>::Type* out_min,
+                            typename OutputOf<kMode>::Type* out_max)
+{
+  const int check = CheckSdfArguments(h_in, h_out, nx, ny, nz, resolution);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  const int listed = CheckDeviceList(devices, num_devices);
+  if (listed != VGT_B200_OK)
+  {
+    return listed;
+  }
+  if (num_devices == 1)
+  {
+    return SdfFromHost<float, kMode>(h_in, nx, ny, nz, resolution, unknown_is_filled,
+                                     add_virtual_border, devices[0], h_out, out_min, out_max);
+  }
+  if (num_devices > nx || num_devices > ny)
+  {
+    return FailInvalid("more devices than voxels along x or y");
+  }
+  OccupancySlabs<kMode> job{};
+  job.grid = MultiGrid{nx, ny, nz, resolution, add_virtual_border, num_devices};
+  job.h_in = h_in;
+  job.unknown_is_filled = unknown_is_filled;
+  job.h_out = h_out;
+  job.extrema.resize(2 * static_cast<size_t>(num_devices));
+  const int status = SdfMultiDevice<kMode>(job.grid, devices, 1, job);
+  if (status != VGT_B200_OK)
+  {
+    return status;
+  }
+  CombineExtrema(job.extrema, num_devices, 1, out_min, out_max);
+  return VGT_B200_OK;
+}
+
+enum CellMember
+{
+  kCellSdf = 0,        // the objects_to_use SDF
+  kCellFreeAndNamed = 1,
+  kCellPerObject = 2   // MakeSeparateObjectSDFs
+};
+
+// The three cell-map members: the cell slab is uploaded in round 0 and stays resident.
+//   kCellSdf:          one round on the filled mask (CellsToMaskKernel with the sorted id list).
+//   kCellFreeAndNamed: round 0 on all filled cells, round 1 on the filled cells of named objects
+//                      (id > 0); both y-slabs are kept and merged elementwise, which is exact on
+//                      a y-slab.
+//   kCellPerObject:    one round per listed id, in the order of the id's sorted position so that
+//                      each group of kSlotGroupSize distinct ids is classified once per slab
+//                      (CellsToObjectSlotsKernel); round r runs the z scan on "slot == key".
+template <int kMode>
+struct CellSlabs
+{
+  using Out = typename OutputOf<kMode>::Type;
+  using Key = typename OutputOf<kMode>::Key;
+  struct Slab
+  {
+    StreamScratch<uint32_t> cells;
+    StreamScratch<uint8_t> mask;  // the filled mask, or the slot map of the batch
+    StreamScratch<uint32_t> ids;
+    StreamScratch<Key> keys;
+    int64_t group = -1;           // the slot group `mask` holds
+  };
+  MultiGrid grid;
+  CellMember member;
+  const void* h_cells;
+  int cell_bytes;
+  int unknown_is_filled;
+  std::vector<uint32_t> sorted;    // distinct ids, ascending
+  std::vector<int64_t> position;   // kCellPerObject: index of object_ids[k] in `sorted`
+  std::vector<int64_t> order;      // kCellPerObject: round -> k
+  Out* h_out;
+  mutable std::vector<Out> extrema;  // [result][device][min, max]
+  int slab_buffers = 1;
+
+  int Local(Slab& slab, const SlabPart& part, int64_t round) const
+  {
+    const int64_t voxels = part.Voxels(grid);
+    const int cell_words = cell_bytes / 4;
+    if (round == 0)
+    {
+      VGT_CUDA_TRY(slab.cells.Allocate(voxels * cell_words, part.stream),
+                   "cell slab allocation");
+      VGT_CUDA_TRY(slab.mask.Allocate(voxels, part.stream), "filled mask allocation");
+      const size_t bytes = static_cast<size_t>(voxels) * cell_bytes;
+      const char* source = static_cast<const char*>(h_cells)
+          + static_cast<size_t>(part.x0 * grid.Plane()) * cell_bytes;
+      VGT_CUDA_TRY(part.transfer->ToDevice(reinterpret_cast<char*>(slab.cells.get()), bytes,
+                                           source, bytes, bytes, 1, part.stream),
+                   "copy cell slab to device");
+      if (member == kCellSdf)
+      {
+        const int uploaded = UploadIds(sorted, slab.ids, part.stream);
+        if (uploaded != VGT_B200_OK)
+        {
+          return uploaded;
+        }
+      }
+    }
+    const int threads = 256;
+    if (member == kCellPerObject)
+    {
+      const int64_t slot = position[static_cast<size_t>(order[static_cast<size_t>(round)])];
+      const int64_t group = slot / kSlotGroupSize;
+      if (group != slab.group)
+      {
+        SlotGroup ids{};
+        const int64_t first = group * kSlotGroupSize;
+        ids.count = static_cast<int>(
+            std::min<int64_t>(kSlotGroupSize, static_cast<int64_t>(sorted.size()) - first));
+        std::copy(sorted.begin() + first, sorted.begin() + first + ids.count, ids.ids);
+        const int64_t blocks = std::min<int64_t>((voxels + threads * 4 - 1) / (threads * 4),
+                                                 MultiprocessorCount() * 8);
+        CellsToObjectSlotsKernel<<<static_cast<unsigned>(blocks), threads, 0, part.stream>>>(
+            slab.cells.get(), cell_words, voxels, unknown_is_filled, ids, slab.mask.get()); NoteKernelLaunch();
+        VGT_CUDA_TRY(cudaGetLastError(), "CellsToObjectSlotsKernel launch");
+        slab.group = group;
+      }
+      const int key = static_cast<int>(slot % kSlotGroupSize) + 1;
+      return ExchangeLocalPasses<ObjectSlot>(reinterpret_cast<const ObjectSlot*>(slab.mask.get()),
+                                             key, grid, part);
+    }
+    int rule = kAnyObject;
+    if (member == kCellSdf && !sorted.empty())
+    {
+      rule = kListedObjects;
+    }
+    else if (member == kCellFreeAndNamed && round == 1)
+    {
+      rule = kNamedObjects;
+    }
+    const int num_ids = (rule == kListedObjects) ? static_cast<int>(sorted.size()) : 0;
+    CellsToMaskKernel<<<static_cast<unsigned>((voxels + threads - 1) / threads), threads, 0,
+                        part.stream>>>(slab.cells.get(), cell_words, voxels, unknown_is_filled,
+                                       rule, num_ids > 0 ? slab.ids.get() : nullptr, num_ids,
+                                       slab.mask.get()); NoteKernelLaunch();
+    VGT_CUDA_TRY(cudaGetLastError(), "CellsToMaskKernel launch");
+    return ExchangeLocalPasses<uint8_t>(slab.mask.get(), 0, grid, part);
+  }
+  bool FinalMinMax(int64_t) const { return member != kCellFreeAndNamed; }
+  int Emit(Slab& slab, const SlabPart& part, int64_t round, Out* const* d_slabs,
+           Out* d_min_max) const
+  {
+    const int64_t count = grid.nx * grid.ny * grid.nz;
+    if (member == kCellSdf)
+    {
+      return CopySlabToHost(d_slabs[0], d_min_max, grid, part, h_out,
+                            extrema.data() + 2 * part.index);
+    }
+    if (member == kCellPerObject)
+    {
+      const int64_t k = order[static_cast<size_t>(round)];
+      return CopySlabToHost(d_slabs[0], d_min_max, grid, part, h_out + k * count,
+                            extrema.data() + 2 * (k * grid.num_devices + part.index));
+    }
+    if (round == 0)
+    {
+      return VGT_B200_OK;  // the all-filled y-slab waits in d_slabs[0] for the named one
+    }
+    // SdfFreeAndNamedOnDevice's merge on the y-slab: d_slabs[0] = merge(free, named)
+    const int64_t slab_voxels = grid.nx * (part.y1 - part.y0) * grid.nz;
+    if (slab.keys.get() == nullptr)
+    {
+      VGT_CUDA_TRY(slab.keys.Allocate(2, part.stream), "min/max scratch");
+    }
+    ResetMinMaxKeysKernel<Key><<<1, 1, 0, part.stream>>>(slab.keys.get()); NoteKernelLaunch();
+    const int threads = 256;
+    const int64_t merge_blocks =
+        std::min<int64_t>((slab_voxels + threads - 1) / threads, MultiprocessorCount() * 16);
+    MergeFreeAndNamedKernel<Out, Key>
+        <<<static_cast<unsigned>(merge_blocks), threads, 0, part.stream>>>(
+            d_slabs[0], d_slabs[1], slab_voxels, d_slabs[0], slab.keys.get()); NoteKernelLaunch();
+    DecodeMinMaxKernel<Out, Key><<<1, 1, 0, part.stream>>>(slab.keys.get(), d_min_max); NoteKernelLaunch();
+    VGT_CUDA_TRY(cudaGetLastError(), "MergeFreeAndNamedKernel launch");
+    return CopySlabToHost(d_slabs[0], d_min_max, grid, part, h_out,
+                          extrema.data() + 2 * part.index);
+  }
+};
+
+template <int kMode>
+int SdfCellsMultiDevice(CellMember member, const void* h_cells, int cell_bytes, int64_t nx,
+                        int64_t ny, int64_t nz, double resolution, int unknown_is_filled,
+                        int add_virtual_border, const uint32_t* object_ids,
+                        int64_t num_object_ids, const int* devices, int num_devices,
+                        typename OutputOf<kMode>::Type* h_out,
+                        typename OutputOf<kMode>::Type* out_min,
+                        typename OutputOf<kMode>::Type* out_max)
+{
+  using Out = typename OutputOf<kMode>::Type;
+  if (member == kCellFreeAndNamed)
+  {
+    object_ids = nullptr;
+    num_object_ids = 0;
+  }
+  const int check = CheckCellArguments(h_cells, cell_bytes, h_out, nx, ny, nz, resolution,
+                                       object_ids, num_object_ids);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  const int listed = CheckMultiDeviceList(devices, num_devices, nx, ny);
+  if (listed != VGT_B200_OK)
+  {
+    return listed;
+  }
+  const int64_t count = nx * ny * nz;
+  if (member == kCellPerObject && num_object_ids > 0
+      && count * static_cast<int64_t>(sizeof(Out)) > INT64_MAX / num_object_ids)
+  {
+    return FailInvalid("%lld SDFs of %lld voxels overflow a 64-bit byte count",
+                       static_cast<long long>(num_object_ids), static_cast<long long>(count));
+  }
+  if (num_devices == 1)
+  {
+    if (member == kCellFreeAndNamed)
+    {
+      return SdfFreeAndNamedHost<kMode>(h_cells, cell_bytes, nx, ny, nz, resolution,
+                                        unknown_is_filled, add_virtual_border, devices[0], h_out,
+                                        out_min, out_max);
+    }
+    return SdfFromCellsHost<kMode>(h_cells, cell_bytes, nx, ny, nz, resolution,
+                                   unknown_is_filled, add_virtual_border, object_ids,
+                                   num_object_ids, member == kCellPerObject, devices[0], h_out,
+                                   out_min, out_max);
+  }
+  // (every device answers before the id list is read; an empty batch launches nothing, but it
+  // still needs the devices it was asked to use)
+  for (int g = 0; g < num_devices; g++)
+  {
+    ScopedDevice scoped(devices[g]);
+    VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  }
+  if (member == kCellPerObject && num_object_ids == 0)
+  {
+    return VGT_B200_OK;
+  }
+  CellSlabs<kMode> job{};
+  job.grid = MultiGrid{nx, ny, nz, resolution, add_virtual_border, num_devices};
+  job.member = member;
+  job.h_cells = h_cells;
+  job.cell_bytes = cell_bytes;
+  job.unknown_is_filled = unknown_is_filled;
+  job.h_out = h_out;
+  job.sorted = SortedDistinct(object_ids, num_object_ids);
+  int64_t rounds = 1;
+  int64_t results = 1;
+  if (member == kCellFreeAndNamed)
+  {
+    rounds = 2;
+    job.slab_buffers = 2;
+  }
+  else if (member == kCellPerObject)
+  {
+    rounds = results = num_object_ids;
+    job.position.resize(static_cast<size_t>(num_object_ids));
+    job.order.resize(static_cast<size_t>(num_object_ids));
+    for (int64_t k = 0; k < num_object_ids; k++)
+    {
+      job.position[static_cast<size_t>(k)] =
+          std::lower_bound(job.sorted.begin(), job.sorted.end(), object_ids[k])
+          - job.sorted.begin();
+      job.order[static_cast<size_t>(k)] = k;
+    }
+    std::stable_sort(job.order.begin(), job.order.end(), [&](int64_t a, int64_t b)
+    {
+      return job.position[static_cast<size_t>(a)] < job.position[static_cast<size_t>(b)];
+    });
+  }
+  job.extrema.resize(2 * static_cast<size_t>(results * num_devices));
+  const int status = SdfMultiDevice<kMode>(job.grid, devices, rounds, job);
+  if (status != VGT_B200_OK)
+  {
+    return status;
+  }
+  CombineExtrema(job.extrema, num_devices, results, out_min, out_max);
   return VGT_B200_OK;
 }
 
@@ -2139,8 +2584,29 @@ int vgt_b200_sdf_f32_multi(
     int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
     float* sdf_out, float* out_min, float* out_max)
 {
-  return SdfMultiDevice(occupancy, nx, ny, nz, resolution, unknown_is_filled, add_virtual_border,
-                        devices, num_devices, sdf_out, out_min, out_max);
+  return SdfOccupancyMultiDevice<kEmitFloat>(occupancy, nx, ny, nz, resolution,
+                                             unknown_is_filled, add_virtual_border, devices,
+                                             num_devices, sdf_out, out_min, out_max);
+}
+
+int vgt_b200_sdf_f64_multi(
+    const float* occupancy, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max)
+{
+  const int check = CheckSdfArguments(occupancy, sdf_out, nx, ny, nz, resolution);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  const int listed = CheckMultiDeviceList(devices, num_devices, nx, ny);
+  if (listed != VGT_B200_OK)
+  {
+    return listed;
+  }
+  return SdfOccupancyMultiDevice<kEmitDouble>(occupancy, nx, ny, nz, resolution,
+                                              unknown_is_filled, add_virtual_border, devices,
+                                              num_devices, sdf_out, out_min, out_max);
 }
 
 int vgt_b200_sdf_f64(
@@ -2226,6 +2692,70 @@ int vgt_b200_sdf_free_and_named_f64(
   return SdfFreeAndNamedHost<kEmitDouble>(cells, cell_bytes, nx, ny, nz, resolution,
                                           unknown_is_filled, add_virtual_border, device, sdf_out,
                                           out_min, out_max);
+}
+
+int vgt_b200_sdf_from_cells_f32_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    float* sdf_out, float* out_min, float* out_max)
+{
+  return SdfCellsMultiDevice<kEmitFloat>(kCellSdf, cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, object_ids, num_object_ids,
+                                     devices, num_devices, sdf_out, out_min, out_max);
+}
+
+int vgt_b200_sdf_from_cells_f64_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max)
+{
+  return SdfCellsMultiDevice<kEmitDouble>(kCellSdf, cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, object_ids, num_object_ids,
+                                     devices, num_devices, sdf_out, out_min, out_max);
+}
+
+int vgt_b200_sdf_per_object_f32_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    float* sdf_out, float* out_min, float* out_max)
+{
+  return SdfCellsMultiDevice<kEmitFloat>(kCellPerObject, cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, object_ids, num_object_ids,
+                                     devices, num_devices, sdf_out, out_min, out_max);
+}
+
+int vgt_b200_sdf_per_object_f64_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const uint32_t* object_ids,
+    int64_t num_object_ids, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max)
+{
+  return SdfCellsMultiDevice<kEmitDouble>(kCellPerObject, cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, object_ids, num_object_ids,
+                                     devices, num_devices, sdf_out, out_min, out_max);
+}
+
+int vgt_b200_sdf_free_and_named_f32_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
+    float* sdf_out, float* out_min, float* out_max)
+{
+  return SdfCellsMultiDevice<kEmitFloat>(kCellFreeAndNamed, cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, nullptr, 0,
+                                     devices, num_devices, sdf_out, out_min, out_max);
+}
+
+int vgt_b200_sdf_free_and_named_f64_multi(
+    const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, double resolution,
+    int unknown_is_filled, int add_virtual_border, const int* devices, int num_devices,
+    double* sdf_out, double* out_min, double* out_max)
+{
+  return SdfCellsMultiDevice<kEmitDouble>(kCellFreeAndNamed, cells, cell_bytes, nx, ny, nz, resolution,
+                                     unknown_is_filled, add_virtual_border, nullptr, 0,
+                                     devices, num_devices, sdf_out, out_min, out_max);
 }
 
 int vgt_b200_sdf_from_cells_f32_dev(

@@ -280,22 +280,20 @@ class OccupancyMap:
     def ExtractSignedDistanceField(self, parameters: SignedDistanceFieldGenerationParameters,
                                    dtype=np.float32, device: int = 0,
                                    devices=None) -> SignedDistanceField:
-        """devices (float32 only): several device ordinals -> the slab-sharded multi-device call
-        (vgt_b200_sdf_f32_multi), same result bit for bit."""
-        _capi.require_device(device if not devices else int(devices[0]))
+        """devices: several device ordinals -> the slab-sharded multi-device call
+        (vgt_b200_sdf_f32_multi / vgt_b200_sdf_f64_multi), same result bit for bit."""
+        device, listed = _device_choice(device, devices)
         lib = _capi.library()
         occupancy = self._data
         nx, ny, nz = self._sizes.shape
         out = np.empty(self._sizes.shape, dtype=dtype)
-        if devices and len(devices) > 1:
-            if np.dtype(dtype) != np.float32:
-                raise ValueError("the multi-device entry produces SignedDistanceField<float>")
-            lo, hi = ctypes.c_float(), ctypes.c_float()
-            listed = (ctypes.c_int * len(devices))(*[int(d) for d in devices])
-            code = lib.vgt_b200_sdf_f32_multi(
+        if listed is not None:
+            suffix, scalar = _scalar_suffix(dtype)
+            lo, hi = scalar(), scalar()
+            code = getattr(lib, f"vgt_b200_sdf_{suffix}_multi")(
                 occupancy.ctypes.data, nx, ny, nz, self._sizes.voxel_size,
                 int(parameters.UnknownIsFilled()), int(parameters.AddVirtualBorder()), listed,
-                len(devices), out.ctypes.data, ctypes.byref(lo), ctypes.byref(hi))
+                len(listed), out.ctypes.data, ctypes.byref(lo), ctypes.byref(hi))
         elif np.dtype(dtype) == np.float32:
             lo, hi = ctypes.c_float(), ctypes.c_float()
             code = lib.vgt_b200_sdf_f32(
@@ -320,8 +318,22 @@ class OccupancyMap:
     def ExtractSignedDistanceFieldFloat(self, parameters, device: int = 0, devices=None):
         return self.ExtractSignedDistanceField(parameters, np.float32, device, devices)
 
-    def ExtractSignedDistanceFieldDouble(self, parameters, device: int = 0):
-        return self.ExtractSignedDistanceField(parameters, np.float64, device)
+    def ExtractSignedDistanceFieldDouble(self, parameters, device: int = 0, devices=None):
+        return self.ExtractSignedDistanceField(parameters, np.float64, device, devices)
+
+
+def _device_choice(device, devices):
+    """The device arguments of the SDF members: ``devices=None`` runs on ``device``, one entry on
+    that device, and two or more on the multi-device entry, which cuts the map into one x-slab per
+    listed device (distinct ordinals, at most 8). Returns (device, ctypes device list or None)."""
+    if not devices:
+        _capi.require_device(device)
+        return device, None
+    ordinals = [int(d) for d in devices]
+    _capi.require_device(ordinals[0])
+    if len(ordinals) == 1:
+        return ordinals[0], None
+    return ordinals[0], (ctypes.c_int * len(ordinals))(*ordinals)
 
 
 # Packed cell layouts of the other map types; the reference pins their sizes with static_asserts
@@ -387,18 +399,27 @@ class _CellGrid:
         sdf.Lock()
         return sdf
 
-    def _from_cells(self, objects_to_use, parameters, dtype, device):
-        _capi.require_device(device)
+    @staticmethod
+    def _cell_entry(name, suffix, device, devices):
+        """The host entry vgt_b200_<name>_<suffix> and its device argument, or its multi-device
+        entry and its (device list, count) arguments."""
+        device, listed = _device_choice(device, devices)
+        lib = _capi.library()
+        if listed is None:
+            return getattr(lib, f"vgt_b200_{name}_{suffix}"), (device,)
+        return getattr(lib, f"vgt_b200_{name}_{suffix}_multi"), (listed, len(listed))
+
+    def _from_cells(self, objects_to_use, parameters, dtype, device, devices=None):
         suffix, scalar = _scalar_suffix(dtype)
+        function, device_arguments = self._cell_entry("sdf_from_cells", suffix, device, devices)
         ids = np.ascontiguousarray(list(objects_to_use), dtype=np.uint32)
         out = np.empty(self._sizes.shape, dtype=dtype)
         lo, hi = scalar(), scalar()
-        function = getattr(_capi.library(), "vgt_b200_sdf_from_cells_" + suffix)
         code = function(self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape,
                         self._sizes.voxel_size, int(parameters.UnknownIsFilled()),
                         int(parameters.AddVirtualBorder()),
-                        ids.ctypes.data if ids.size else None, ids.size, device, out.ctypes.data,
-                        ctypes.byref(lo), ctypes.byref(hi))
+                        ids.ctypes.data if ids.size else None, ids.size, *device_arguments,
+                        out.ctypes.data, ctypes.byref(lo), ctypes.byref(hi))
         _capi.check(code)
         return self._wrap(out, lo.value, hi.value, parameters)
 
@@ -435,14 +456,18 @@ class OccupancyComponentMap(_CellGrid):
 
     CELL = OCCUPANCY_COMPONENT_CELL
 
-    def ExtractSignedDistanceField(self, parameters, dtype=np.float32, device: int = 0):
-        return self._from_cells((), parameters, dtype, device)
+    def ExtractSignedDistanceField(self, parameters, dtype=np.float32, device: int = 0,
+                                   devices=None):
+        """``devices``: two or more distinct device ordinals (at most 8) cut the map into one
+        x-slab per device (vgt_b200_sdf_from_cells_*_multi), for maps one device cannot hold;
+        the same field and min/max as on one device."""
+        return self._from_cells((), parameters, dtype, device, devices)
 
-    def ExtractSignedDistanceFieldFloat(self, parameters, device: int = 0):
-        return self.ExtractSignedDistanceField(parameters, np.float32, device)
+    def ExtractSignedDistanceFieldFloat(self, parameters, device: int = 0, devices=None):
+        return self.ExtractSignedDistanceField(parameters, np.float32, device, devices)
 
-    def ExtractSignedDistanceFieldDouble(self, parameters, device: int = 0):
-        return self.ExtractSignedDistanceField(parameters, np.float64, device)
+    def ExtractSignedDistanceFieldDouble(self, parameters, device: int = 0, devices=None):
+        return self.ExtractSignedDistanceField(parameters, np.float64, device, devices)
 
     def UpdateConnectedComponents(self, device: int = 0, devices=None) -> int:
         """Labels the connected components of the map into every cell's ``component`` and returns
@@ -463,54 +488,61 @@ class TaggedObjectOccupancyMap(_CellGrid):
     CELL = TAGGED_OBJECT_OCCUPANCY_CELL
 
     def ExtractSignedDistanceField(self, objects_to_use, parameters, dtype=np.float32,
-                                   device: int = 0):
+                                   device: int = 0, devices=None):
         """Filled = occupancy rule and (no objects listed or object id listed)
-        (tagged_object_occupancy_map.hpp:199-247)."""
-        return self._from_cells(objects_to_use, parameters, dtype, device)
+        (tagged_object_occupancy_map.hpp:199-247).
+        ``devices`` (here and on every SDF member below): two or more distinct device ordinals
+        (at most 8) cut the map into one x-slab per device (the *_multi entries), for maps one
+        device cannot hold; the same fields and min/max as on one device."""
+        return self._from_cells(objects_to_use, parameters, dtype, device, devices)
 
-    def ExtractSignedDistanceFieldFloat(self, objects_to_use, parameters, device: int = 0):
-        return self.ExtractSignedDistanceField(objects_to_use, parameters, np.float32, device)
+    def ExtractSignedDistanceFieldFloat(self, objects_to_use, parameters, device: int = 0,
+                                        devices=None):
+        return self.ExtractSignedDistanceField(objects_to_use, parameters, np.float32, device,
+                                               devices)
 
-    def ExtractSignedDistanceFieldDouble(self, objects_to_use, parameters, device: int = 0):
-        return self.ExtractSignedDistanceField(objects_to_use, parameters, np.float64, device)
+    def ExtractSignedDistanceFieldDouble(self, objects_to_use, parameters, device: int = 0,
+                                         devices=None):
+        return self.ExtractSignedDistanceField(objects_to_use, parameters, np.float64, device,
+                                               devices)
 
-    def MakeSeparateObjectSDFs(self, object_ids, parameters, dtype=np.float32, device: int = 0):
+    def MakeSeparateObjectSDFs(self, object_ids, parameters, dtype=np.float32, device: int = 0,
+                               devices=None):
         """One SDF per object id, the cells uploaded once
         (tagged_object_occupancy_map.hpp:249-262). Returns {object_id: SignedDistanceField}."""
-        _capi.require_device(device)
         suffix, _ = _scalar_suffix(dtype)
+        function, device_arguments = self._cell_entry("sdf_per_object", suffix, device, devices)
         ids = np.ascontiguousarray(list(object_ids), dtype=np.uint32)
         if ids.size == 0:
             return {}
         out = np.empty((ids.size,) + self._sizes.shape, dtype=dtype)
         lows = np.empty(ids.size, dtype=dtype)
         highs = np.empty(ids.size, dtype=dtype)
-        function = getattr(_capi.library(), "vgt_b200_sdf_per_object_" + suffix)
         code = function(self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape,
                         self._sizes.voxel_size, int(parameters.UnknownIsFilled()),
-                        int(parameters.AddVirtualBorder()), ids.ctypes.data, ids.size, device,
-                        out.ctypes.data, lows.ctypes.data, highs.ctypes.data)
+                        int(parameters.AddVirtualBorder()), ids.ctypes.data, ids.size,
+                        *device_arguments, out.ctypes.data, lows.ctypes.data, highs.ctypes.data)
         _capi.check(code)
         return {int(object_id): self._wrap(out[k], lows[k], highs[k], parameters)
                 for k, object_id in enumerate(ids)}
 
-    def MakeAllObjectSDFs(self, parameters, dtype=np.float32, device: int = 0):
+    def MakeAllObjectSDFs(self, parameters, dtype=np.float32, device: int = 0, devices=None):
         """Every object id > 0 present in the map (tagged_object_occupancy_map.hpp:264-291)."""
         object_ids = np.unique(self._data["object_id"])
         return self.MakeSeparateObjectSDFs([i for i in object_ids.tolist() if i > 0], parameters,
-                                           dtype, device)
+                                           dtype, device, devices)
 
     def ExtractFreeAndNamedObjectsSignedDistanceField(self, parameters, dtype=np.float32,
-                                                      device: int = 0):
+                                                      device: int = 0, devices=None):
         """tagged_object_occupancy_map.hpp:293-378."""
-        _capi.require_device(device)
         suffix, scalar = _scalar_suffix(dtype)
+        function, device_arguments = self._cell_entry("sdf_free_and_named", suffix, device,
+                                                      devices)
         out = np.empty(self._sizes.shape, dtype=dtype)
         lo, hi = scalar(), scalar()
-        function = getattr(_capi.library(), "vgt_b200_sdf_free_and_named_" + suffix)
         code = function(self._data.ctypes.data, self.CELL.itemsize, *self._sizes.shape,
                         self._sizes.voxel_size, int(parameters.UnknownIsFilled()),
-                        int(parameters.AddVirtualBorder()), device, out.ctypes.data,
+                        int(parameters.AddVirtualBorder()), *device_arguments, out.ctypes.data,
                         ctypes.byref(lo), ctypes.byref(hi))
         _capi.check(code)
         return self._wrap(out, lo.value, hi.value, parameters)
