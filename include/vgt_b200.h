@@ -26,6 +26,7 @@
 #ifndef VGT_B200_H_
 #define VGT_B200_H_
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -663,16 +664,98 @@ VGT_B200_API int vgt_b200_connected_components_dev(
  * devices[g]; a device may be listed more than once, so one device labels a map of 2^32 cells or
  * more when its memory allows. The same bytes and count as vgt_b200_connected_components on every
  * map that entry accepts. Each slab is labelled on its own, the edges across the x-faces between
- * slabs are resolved on devices[0], and every slab then writes the reference's numbers.
+ * slabs are resolved on every slab's device, and every slab then writes the reference's numbers.
  *   1 <= num_slabs <= 8, num_slabs <= nx; num_slabs == 1 is vgt_b200_connected_components.
  *   Device memory, per slab on its device: the slab's cells + 4 B per cell + about 0.25 B per
- *   cell + about 4.25 B per component local to the slab; on devices[0] in addition up to 64 B per
- *   face edge, at most (num_slabs - 1) * ny * nz edges.
+ *   cell + about 4.25 B per component local to the slab, and up to 64 B per face edge, at most
+ *   (num_slabs - 1) * ny * nz edges.
  * Slabs of 2^32 cells or more fail with VGT_B200_ERR_UNSUPPORTED before any device call, and so
  * does a map of more than 0xFFFFFFFF components, before any cell is written (cells unchanged). */
 VGT_B200_API int vgt_b200_connected_components_multi(
     void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, const int* devices,
     int num_slabs, uint32_t* out_num_components);
+
+/* The phases of vgt_b200_connected_components_multi for one x-slab whose cells are already on
+ * its device, one slab per process (DESIGN.md section 8): the caller moves what crosses slabs
+ * (collectives) and owns every array that lives from one phase to the next. Every entry is
+ * asynchronous on `stream`; values the caller needs on the host are written to device memory.
+ * Slab r holds the x-planes [x0_r, x1_r) of the map; its base is x0_r * ny * nz, the global index
+ * of its first cell. In order, on every slab:
+ *   scan_bytes, local, face_edges (every slab but the first), resolve, count, publish, write.
+ * Arguments are checked before any device call: VGT_B200_ERR_INVALID_ARGUMENT for a null
+ * pointer, a cell size other than 8 or 16, bad dimensions or ranges (a slab has at least one
+ * x-plane), VGT_B200_ERR_UNSUPPORTED for a slab of 2^32 cells or more. */
+
+/* The bytes of scan storage the local and count phases of a slab of nx*ny*nz cells need
+ * (ComputeConnectedComponents, topology_computation.hpp:138-196, per slab). */
+VGT_B200_API int vgt_b200_components_slab_scan_bytes(
+    int64_t nx, int64_t ny, int64_t nz, int device, size_t* out_bytes);
+
+/* Labels the slab as a grid of its own (32-bit local indices; topology_computation.hpp:138-196).
+ *   d_parent       uint32[nx*ny*nz]            the local union-find, kept until the write phase
+ *   d_mask         uint32[words]               words = (nx*ny*nz + 31) / 32: the local roots
+ *   d_word_prefix  uint32[words + 1]           their ranks; K_g, the number of local
+ *                                              components, ends in d_word_prefix[words]
+ *   d_scan_storage scan_bytes bytes            (vgt_b200_components_slab_scan_bytes)
+ *   d_face_roots   uint32[ny*nz] or NULL       the local roots of the slab's last x-plane, for
+ *                                              the slab above (NULL on the last slab) */
+VGT_B200_API int vgt_b200_components_slab_local(
+    void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, int device,
+    uint32_t* d_parent, uint32_t* d_mask, uint32_t* d_word_prefix, void* d_scan_storage,
+    size_t scan_bytes, uint32_t* d_face_roots, void* stream);
+
+/* The edges of the x-face below the slab (the face neighbours of topology_computation.hpp:138-196
+ * that lie in two slabs): d_below_cells (ny*nz cells as stored) and
+ * d_below_roots (their local roots, d_face_roots of the local phase there) are the last x-plane
+ * of the slab below, whose base is below_base. Writes up to ny*nz edges
+ * d_edges[e] = {global root below, global root above} (int64[ny*nz][2]) and their number to
+ * *d_edge_count. */
+VGT_B200_API int vgt_b200_components_slab_face_edges(
+    const void* d_below_cells, const uint32_t* d_below_roots, int64_t below_base, void* d_cells,
+    int cell_bytes, int64_t nx, int64_t ny, int64_t nz, int64_t base, int device,
+    uint32_t* d_parent, int64_t* d_edges, uint32_t* d_edge_count, void* stream);
+
+/* The edges of all faces of a map of num_cells cells (topology_computation.hpp:138-196), in any order (d_edges may be NULL without
+ * edges), sorted and made unique into nodes and joined; every slab that passes the same edges
+ * gets the same nodes and compact roots. d_nodes (int64) and d_node_roots (uint32) hold
+ * max(1, 2*num_edges) entries; d_node_range[3] = {number of nodes, first node of the slab
+ * [base, end), one past its last}. */
+VGT_B200_API int vgt_b200_components_resolve(
+    const int64_t* d_edges, int64_t num_edges, int64_t num_cells, int64_t base, int64_t end,
+    int device, int64_t* d_nodes, uint32_t* d_node_roots, uint32_t* d_node_range, void* stream);
+
+/* The slab's global roots (topology_computation.hpp:138-196): its local components that are not merged into a component whose
+ * smallest index lies in a lower slab. num_components = K_g; num_nodes, first_node and
+ * num_slab_nodes from d_node_range. d_bits uint32[bit_words], d_bit_prefix uint32[bit_words + 1]
+ * with bit_words = (K_g + 31) / 32; count_g ends in d_bit_prefix[bit_words]. */
+VGT_B200_API int vgt_b200_components_slab_count(
+    int64_t nx, int64_t ny, int64_t nz, int64_t base, int64_t num_components, int device,
+    const uint32_t* d_mask, const uint32_t* d_word_prefix, const int64_t* d_nodes,
+    const uint32_t* d_node_roots, int64_t num_nodes, int64_t first_node, int64_t num_slab_nodes,
+    uint32_t* d_bits, uint32_t* d_bit_prefix, void* d_scan_storage, size_t scan_bytes,
+    void* stream);
+
+/* The reference's numbers (topology_computation.hpp:138-196) of the slab's global roots:
+ * offset = the sum of count_g over the slabs below (the caller refuses a map whose total is
+ * above 0xFFFFFFFF before this phase). Writes d_final_ids (uint32[K_g]) and the ids of the slab's
+ * nodes into d_node_ids (uint32[num_nodes], zero-filled by the caller; the slab writes only its
+ * own nodes, 0 for those whose compact root is another node). */
+VGT_B200_API int vgt_b200_components_slab_publish(
+    int64_t nx, int64_t ny, int64_t nz, int64_t base, int64_t num_components, int64_t offset,
+    int device, const uint32_t* d_mask, const uint32_t* d_word_prefix, const int64_t* d_nodes,
+    int64_t num_nodes, int64_t first_node, int64_t num_slab_nodes, const uint32_t* d_bits,
+    const uint32_t* d_bit_prefix, uint32_t* d_final_ids, uint32_t* d_node_ids, void* stream);
+
+/* The component words (topology_computation.hpp:138-196). d_node_ids = the sum over all slabs
+ * of their published arrays (each entry is written by one
+ * slab only). Every node takes its compact root's id, then the component word of every cell of
+ * the slab is written; every other word of every cell stays as it was. */
+VGT_B200_API int vgt_b200_components_slab_write(
+    void* d_cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz, int64_t base,
+    int64_t num_components, int device, uint32_t* d_parent, const uint32_t* d_mask,
+    const uint32_t* d_word_prefix, const int64_t* d_nodes, const uint32_t* d_node_roots,
+    int64_t num_nodes, int64_t first_node, int64_t num_slab_nodes, uint32_t* d_node_ids,
+    uint32_t* d_final_ids, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * On-disk formats (SURVEY.md section 8 f3): the reference's own grid files, so that results

@@ -179,6 +179,23 @@ SIGNATURES = {
     "vgt_b200_connected_components": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp]),
     "vgt_b200_connected_components_dev": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp, _vp]),
     "vgt_b200_connected_components_multi": (_int, [_vp, _int, _i64, _i64, _i64, _vp, _int, _vp]),
+    "vgt_b200_components_slab_scan_bytes": (_int, [_i64, _i64, _i64, _int,
+                                                   ctypes.POINTER(ctypes.c_size_t)]),
+    "vgt_b200_components_slab_local": (_int, [_vp, _int, _i64, _i64, _i64, _int, _vp, _vp, _vp,
+                                              _vp, ctypes.c_size_t, _vp, _vp]),
+    "vgt_b200_components_slab_face_edges": (_int, [_vp, _vp, _i64, _vp, _int, _i64, _i64, _i64,
+                                                   _i64, _int, _vp, _vp, _vp, _vp]),
+    "vgt_b200_components_resolve": (_int, [_vp, _i64, _i64, _i64, _i64, _int, _vp, _vp, _vp,
+                                           _vp]),
+    "vgt_b200_components_slab_count": (_int, [_i64, _i64, _i64, _i64, _i64, _int, _vp, _vp, _vp,
+                                              _vp, _i64, _i64, _i64, _vp, _vp, _vp,
+                                              ctypes.c_size_t, _vp]),
+    "vgt_b200_components_slab_publish": (_int, [_i64, _i64, _i64, _i64, _i64, _i64, _int, _vp,
+                                                _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp,
+                                                _vp]),
+    "vgt_b200_components_slab_write": (_int, [_vp, _int, _i64, _i64, _i64, _i64, _i64, _int, _vp,
+                                              _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp,
+                                              _vp]),
     "vgt_b200_grid_file_save": (_int, [ctypes.c_char_p, _int, _int, _vp,
                                        ctypes.POINTER(GridFileInfo), ctypes.c_char_p]),
     "vgt_b200_grid_file_save_dev": (_int, [ctypes.c_char_p, _int, _int, _vp,

@@ -25,8 +25,10 @@
 
 #include <atomic>
 #include <functional>
+#include <initializer_list>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "common.cuh"
@@ -389,23 +391,26 @@ int Launch(void* d_cells, int cell_bytes, const Grid& grid, uint32_t* d_num_comp
 // slabs. So:
 //   a. per face, FaceEdgesKernel emits (global root of the cell below, global root of the cell
 //      above) where the keys are equal and the edge is not implied by the (y, z - 1) pair;
-//   b. on devices[0] the endpoints are sorted and made unique (the nodes), the edges are mapped
-//      to compact node ids by binary search and joined by union-find with parent <= self;
-//      compact order is global order, so a node's compact root is the smallest global index of
-//      its merged set;
+//   b. on every slab's device the endpoints of all faces' edges are sorted and made unique (the
+//      nodes), the edges are mapped to compact node ids by binary search and joined by
+//      union-find with parent <= self; compact order is global order, so a node's compact root
+//      is the smallest global index of its merged set, and every slab gets the same table;
 //   c. per slab, one bit per local component, cleared for the slab's nodes whose compact root is
 //      another node; the bits left are the components whose smallest index lies in the slab,
 //      count_g of them, and component ids are offset_g + 1 + rank among them (offset_g = the
 //      sum of the counts of the slabs below): the reference's numbering;
-//   d. root nodes publish their id to devices[0], every node takes the id of its compact root,
-//      and each slab writes final[local rank] into the component word of its cells.
-// Everything that crosses slabs (face planes and roots, edges, node tables) goes through host
-// memory: it is O(num_slabs * ny * nz).
+//   d. each slab publishes the ids of its nodes into a node-id array that is zero elsewhere; with
+//      the arrays of all slabs added up, every node takes the id of its compact root, and each
+//      slab writes final[local rank] into the component word of its cells.
+// In vgt_b200_connected_components_multi everything that crosses slabs (face planes and roots,
+// edges, node ids) goes through host memory: it is O(num_slabs * ny * nz). The
+// vgt_b200_components_* entries run the same phases on one slab per process and leave the
+// crossing to the caller's collectives.
 // Scratch per slab, on its device: the slab's cells + 4 B per cell (parent) + about 0.25 B per
 // cell (root mask, word prefix) + 4 B per local component (final ids) + about 0.25 B per local
-// component (root bits, word prefix), + O(ny * nz) for the faces and the slab's nodes. On
-// devices[0] in addition, E = at most (num_slabs - 1) * ny * nz edges: at most 64 B per edge
-// (the edges, their sorted endpoints, the nodes, their parents and compact roots).
+// component (root bits, word prefix), + O(ny * nz) for the faces, and the face graph of
+// E = at most (num_slabs - 1) * ny * nz edges: at most 64 B per edge (the edges, their sorted
+// endpoints, the nodes, their parents and compact roots).
 // =============================================================================================
 struct Edge
 {
@@ -666,6 +671,241 @@ inline uint32_t Blocks(uint64_t threads)
     VGT_CUDA_TRY(cudaGetLastError(), what " launch");       \
   } while (0)
 
+// ---------------------------------------------------------------------------------------------
+// The phases of one slab, each asynchronous on `stream`: steps 1-5 of the slab scheme above.
+// vgt_b200_connected_components_multi runs them on host threads and passes what crosses slabs
+// through host memory; the vgt_b200_components_* entries run one slab per process and leave the
+// crossing to the caller (collectives). Every array that lives from one phase to the next is the
+// caller's.
+// ---------------------------------------------------------------------------------------------
+struct SlabArrays
+{
+  Grid grid;
+  uint64_t base;          // global index of the slab's first cell
+  uint32_t* cells;
+  uint32_t* parent;       // grid.count
+  uint32_t* mask;         // (grid.count + 31) / 32
+  uint32_t* word_prefix;  // (grid.count + 31) / 32 + 1; the last entry ends as K_g
+  void* scan_storage;     // ScanBytes(grid.count): both scans of the slab
+  size_t scan_bytes;
+};
+
+// The face graph's nodes as ResolvePhase leaves them, and the slab's share of them.
+struct SlabNodes
+{
+  const uint64_t* nodes;       // the sorted unique endpoints of all edges
+  const uint32_t* node_roots;  // their compact roots
+  uint32_t num_nodes;
+  uint32_t first;              // the slab's nodes are [first, first + count)
+  uint32_t count;
+};
+
+uint32_t RootWords(uint32_t cells)
+{
+  return (cells + 31) / 32;
+}
+
+// Temporary storage of the scan of a slab's word counts (words + 1 entries); it also fits the
+// scan of the root bits (at most as many words).
+int ScanBytes(uint32_t count, size_t* bytes)
+{
+  size_t needed = 0;
+  VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, needed, static_cast<uint32_t*>(nullptr),
+                                             static_cast<uint32_t*>(nullptr),
+                                             static_cast<int>(RootWords(count)) + 1),
+               "scan size query");
+  *bytes = std::max<size_t>(needed, 1);
+  return VGT_B200_OK;
+}
+
+// Step 1: steps 1-4 of the whole-grid labelling on the slab alone; K_g ends in
+// word_prefix[words]. face_roots (may be null): the local roots of the slab's last x-plane.
+template <int kCellWords>
+int LocalPhase(const SlabArrays& slab, uint32_t* face_roots, cudaStream_t stream)
+{
+  const Grid& grid = slab.grid;
+  const uint32_t words = RootWords(grid.count);
+  const uint32_t blocks = Blocks(grid.count);
+  VGT_CUDA_TRY(cudaMemsetAsync(slab.word_prefix + words, 0, sizeof(uint32_t), stream),
+               "count reset");
+  InitRunsKernel<kCellWords><<<blocks, kThreads, 0, stream>>>(slab.cells, grid, slab.parent);
+  VGT_LAUNCHED("InitRunsKernel");
+  MergeKernel<kCellWords><<<blocks, kThreads, 0, stream>>>(slab.cells, grid, slab.parent);
+  VGT_LAUNCHED("MergeKernel");
+  MarkRootsKernel<<<blocks, kThreads, 0, stream>>>(slab.parent, grid.count, slab.mask,
+                                                   slab.word_prefix);
+  VGT_LAUNCHED("MarkRootsKernel");
+  size_t scan_bytes = slab.scan_bytes;
+  VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(slab.scan_storage, scan_bytes, slab.word_prefix,
+                                             slab.word_prefix, static_cast<int>(words) + 1,
+                                             stream),
+               "root rank scan");
+  NoteKernelLaunch();  // the scan is two kernels (tile-state init, then the scan)
+  NoteKernelLaunch();
+  if (face_roots != nullptr)
+  {
+    const uint32_t plane = grid.ny * grid.nz;
+    FaceRootsKernel<<<Blocks(plane), kThreads, 0, stream>>>(slab.parent, grid.count - plane,
+                                                            plane, face_roots);
+    VGT_LAUNCHED("FaceRootsKernel");
+  }
+  return VGT_B200_OK;
+}
+
+// Step 2, on the slab above the face: below_cells / below_roots are the last x-plane of the slab
+// below (its cells as stored and their local roots), below_base that slab's first global index.
+// At most ny * nz edges; their number ends in *edge_count.
+template <int kCellWords>
+int FaceEdgesPhase(const uint32_t* below_cells, const uint32_t* below_roots, uint64_t below_base,
+                   const SlabArrays& slab, Edge* edges, uint32_t* edge_count, cudaStream_t stream)
+{
+  const uint32_t plane = slab.grid.ny * slab.grid.nz;
+  VGT_CUDA_TRY(cudaMemsetAsync(edge_count, 0, sizeof(uint32_t), stream), "edge count reset");
+  FaceEdgesKernel<kCellWords><<<Blocks(plane), kThreads, 0, stream>>>(
+      below_cells, below_roots, below_base, slab.cells, slab.parent, slab.base, plane,
+      slab.grid.nz, edges, edge_count);
+  VGT_LAUNCHED("FaceEdgesKernel");
+  return VGT_B200_OK;
+}
+
+// Step 3: the edges of all faces (any order) sorted and made unique into nodes, joined and
+// flattened. nodes / node_roots hold max(1, 2 * num_edges) entries: nodes past the node count
+// are all ones (so binary searches over the whole array find the real ones) and their roots are
+// themselves. node_words[0] = the node count, node_words[1 + b] = the first node >= bases[b]
+// (host array, num_bases entries below num_cells). Compact roots are set minima, so every caller
+// that passes the same edges gets the same nodes and roots whatever their order.
+int ResolvePhase(const Edge* edges, uint32_t num_edges, uint64_t num_cells,
+                 const uint64_t* bases, int num_bases, uint64_t* nodes, uint32_t* node_roots,
+                 uint32_t* node_words, cudaStream_t stream)
+{
+  const int num_endpoints = static_cast<int>(2 * num_edges);
+  const uint32_t capacity = std::max<uint32_t>(1, 2 * num_edges);
+  StreamScratch<uint64_t> sorted;
+  StreamScratch<uint32_t> node_parent;
+  StreamScratch<uint64_t> d_bases;
+  StreamScratch<char> storage;
+  VGT_CUDA_TRY(sorted.Allocate(capacity, stream), "endpoint allocation");
+  VGT_CUDA_TRY(node_parent.Allocate(capacity, stream), "node parent allocation");
+  VGT_CUDA_TRY(d_bases.Allocate(num_bases, stream), "base allocation");
+  VGT_CUDA_TRY(cudaMemcpyAsync(d_bases.get(), bases, sizeof(uint64_t) * num_bases,
+                               cudaMemcpyHostToDevice, stream),
+               "copy bases");
+  VGT_CUDA_TRY(cudaMemsetAsync(nodes, 0xff, sizeof(uint64_t) * capacity, stream), "node reset");
+  VGT_CUDA_TRY(cudaMemsetAsync(node_words, 0, sizeof(uint32_t), stream), "node count reset");
+  int end_bit = 1;
+  while (end_bit < 64 && (num_cells >> end_bit) != 0)
+  {
+    end_bit++;
+  }
+  const uint64_t* endpoints = reinterpret_cast<const uint64_t*>(edges);
+  size_t sort_bytes = 0;
+  size_t unique_bytes = 0;
+  VGT_CUDA_TRY(cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, endpoints, sorted.get(),
+                                              num_endpoints, 0, end_bit, stream),
+               "sort size query");
+  VGT_CUDA_TRY(cub::DeviceSelect::Unique(nullptr, unique_bytes, sorted.get(), nodes, node_words,
+                                         num_endpoints, stream),
+               "unique size query");
+  const size_t storage_bytes = std::max<size_t>({sort_bytes, unique_bytes, 1});
+  VGT_CUDA_TRY(storage.Allocate(static_cast<int64_t>(storage_bytes), stream),
+               "resolve storage allocation");
+  if (num_edges > 0)
+  {
+    VGT_CUDA_TRY(cub::DeviceRadixSort::SortKeys(storage.get(), sort_bytes, endpoints, sorted.get(),
+                                                num_endpoints, 0, end_bit, stream),
+                 "endpoint sort");
+    NoteKernelLaunch();
+    VGT_CUDA_TRY(cub::DeviceSelect::Unique(storage.get(), unique_bytes, sorted.get(), nodes,
+                                           node_words, num_endpoints, stream),
+                 "endpoint unique");
+    NoteKernelLaunch();
+    NodeInitKernel<<<Blocks(capacity), kThreads, 0, stream>>>(node_parent.get(), capacity);
+    VGT_LAUNCHED("NodeInitKernel");
+    NodeUnionKernel<<<Blocks(num_edges), kThreads, 0, stream>>>(edges, num_edges, nodes,
+                                                                capacity, node_parent.get());
+    VGT_LAUNCHED("NodeUnionKernel");
+  }
+  const uint32_t flattened = num_edges > 0 ? capacity : 0;
+  NodeFlattenKernel<<<Blocks(std::max<uint32_t>(capacity, num_bases)), kThreads, 0, stream>>>(
+      node_parent.get(), nodes, flattened, d_bases.get(), num_bases, node_roots, node_words + 1);
+  VGT_LAUNCHED("NodeFlattenKernel");
+  return VGT_B200_OK;
+}
+
+// Step 4: one bit per local component, cleared for the slab's nodes whose compact root is another
+// node; count_g (the bits left) ends in bit_prefix[bit words].
+int CountPhase(const SlabArrays& slab, uint32_t num_components, const SlabNodes& graph,
+               uint32_t* bits, uint32_t* bit_prefix, cudaStream_t stream)
+{
+  const uint32_t bit_words = RootWords(num_components);
+  GlobalRootBitsInitKernel<<<Blocks(bit_words), kThreads, 0, stream>>>(bits, num_components);
+  VGT_LAUNCHED("GlobalRootBitsInitKernel");
+  if (graph.count > 0)
+  {
+    ClearMergedBitsKernel<<<Blocks(graph.count), kThreads, 0, stream>>>(
+        graph.nodes + graph.first, graph.node_roots + graph.first, graph.count, graph.first,
+        slab.base, slab.mask, slab.word_prefix, bits);
+    VGT_LAUNCHED("ClearMergedBitsKernel");
+  }
+  VGT_CUDA_TRY(cudaMemsetAsync(bit_prefix + bit_words, 0, sizeof(uint32_t), stream),
+               "count reset");
+  BitCountsKernel<<<Blocks(bit_words), kThreads, 0, stream>>>(bits, bit_words, bit_prefix);
+  VGT_LAUNCHED("BitCountsKernel");
+  size_t scan_bytes = slab.scan_bytes;
+  VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(slab.scan_storage, scan_bytes, bit_prefix, bit_prefix,
+                                             static_cast<int>(bit_words) + 1, stream),
+               "global root scan");
+  NoteKernelLaunch();
+  NoteKernelLaunch();
+  return VGT_B200_OK;
+}
+
+// Step 5a: final[r] = offset + 1 + rank among the slab's global roots (0 for merged components);
+// node_ids[first + k] = the final id of the slab's node k (node_ids: one word per node, zero
+// elsewhere; after the ids of all slabs are added up, every root node holds its id).
+int PublishPhase(const SlabArrays& slab, uint32_t num_components, uint32_t offset,
+                 const SlabNodes& graph, const uint32_t* bits, const uint32_t* bit_prefix,
+                 uint32_t* final_ids, uint32_t* node_ids, cudaStream_t stream)
+{
+  FinalIdsKernel<<<Blocks(num_components), kThreads, 0, stream>>>(bits, bit_prefix,
+                                                                  num_components, offset,
+                                                                  final_ids);
+  VGT_LAUNCHED("FinalIdsKernel");
+  if (graph.count > 0)
+  {
+    PublishNodeIdsKernel<<<Blocks(graph.count), kThreads, 0, stream>>>(
+        graph.nodes + graph.first, graph.count, slab.base, slab.mask, slab.word_prefix, final_ids,
+        node_ids + graph.first);
+    VGT_LAUNCHED("PublishNodeIdsKernel");
+  }
+  return VGT_B200_OK;
+}
+
+// Step 5b, on the ids of every slab added up: every node takes its compact root's id, the
+// slab's merged components take their nodes' ids, and every cell's component word is written.
+template <int kCellWords>
+int WritePhase(const SlabArrays& slab, const SlabNodes& graph, uint32_t* node_ids,
+               uint32_t* final_ids, cudaStream_t stream)
+{
+  if (graph.num_nodes > 0)
+  {
+    NodeIdsFromRootsKernel<<<Blocks(graph.num_nodes), kThreads, 0, stream>>>(
+        graph.node_roots, graph.num_nodes, node_ids);
+    VGT_LAUNCHED("NodeIdsFromRootsKernel");
+  }
+  if (graph.count > 0)
+  {
+    ApplyNodeIdsKernel<<<Blocks(graph.count), kThreads, 0, stream>>>(
+        graph.nodes + graph.first, node_ids + graph.first, graph.count, slab.base, slab.mask,
+        slab.word_prefix, final_ids);
+    VGT_LAUNCHED("ApplyNodeIdsKernel");
+  }
+  WriteSlabComponentsKernel<kCellWords><<<Blocks(slab.grid.count), kThreads, 0, stream>>>(
+      slab.cells, slab.grid.count, slab.parent, slab.mask, slab.word_prefix, final_ids);
+  VGT_LAUNCHED("WriteSlabComponentsKernel");
+  return VGT_B200_OK;
+}
+
 // Every check of vgt_b200_connected_components_multi, before any device call.
 int CheckMultiArguments(const void* cells, int cell_bytes, int64_t nx, int64_t ny, int64_t nz,
                         const int* devices, int num_slabs, const void* num_components)
@@ -739,6 +979,7 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
     slab_base[static_cast<size_t>(g)] = static_cast<uint64_t>(x_begin[static_cast<size_t>(g)])
                                       * plane;
   }
+  const uint64_t num_cells = slab_base[static_cast<size_t>(num_slabs)];
 
   // What one slab's thread shows the others between phases (written before a barrier, read
   // after it). Everything that crosses slabs goes through host memory with plain async copies:
@@ -750,13 +991,10 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
     std::vector<uint32_t> face_roots;  // and the local roots of its cells
     std::vector<Edge> edges;           // the edges of the face below the slab
     uint64_t num_global_roots = 0;     // count_g
+    std::vector<uint32_t> node_ids;    // the ids of the slab's nodes (PublishPhase)
+    uint32_t first_node = 0;
   };
   std::vector<Shared> shared(static_cast<size_t>(num_slabs));
-  // the face graph as resolved on devices[0]: the nodes, their compact roots, their ids
-  std::vector<uint64_t> nodes;
-  std::vector<uint32_t> node_roots;
-  std::vector<uint32_t> node_ids;
-  std::vector<uint32_t> slab_first(static_cast<size_t>(num_slabs) + 1, 0);
   std::atomic<uint64_t> total_components{0};
 
   ThreadBarrier barrier(num_slabs);
@@ -773,40 +1011,33 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
     const int64_t slab_x = x_begin[s + 1] - x_begin[s];
     const Grid grid{static_cast<uint32_t>(slab_x), static_cast<uint32_t>(ny),
                     static_cast<uint32_t>(nz), static_cast<uint32_t>(slab_x * plane)};
-    const uint32_t words = (grid.count + 31) / 32;
+    const uint32_t words = RootWords(grid.count);
     const size_t slab_bytes = kCellBytes * grid.count;
     char* const h_slab = h_cells + kCellBytes * slab_base[s];
     uint32_t num_components = 0;
-    uint32_t first_node = 0;
-    uint32_t num_nodes = 0;  // of this slab
-    uint64_t offset = 0;
+    uint32_t node_words[3] = {0, 0, 0};  // node count, the slab's first node, its end
+    SlabNodes graph{};
 
     StreamGuard guard;
     StreamScratch<uint32_t> d_cells;
     StreamScratch<uint32_t> parent;
     StreamScratch<uint32_t> mask;
-    StreamScratch<uint32_t> word_prefix;  // words + 1 entries
+    StreamScratch<uint32_t> word_prefix;
     StreamScratch<char> scan_storage;
     StreamScratch<uint32_t> face_roots;
     StreamScratch<uint32_t> below_plane;
     StreamScratch<uint32_t> below_roots;
     StreamScratch<Edge> edges;
     StreamScratch<uint32_t> edge_count;
+    StreamScratch<Edge> all_edges;
+    StreamScratch<uint64_t> nodes;
+    StreamScratch<uint32_t> node_roots;
+    StreamScratch<uint32_t> d_node_words;
     StreamScratch<uint32_t> bits;
     StreamScratch<uint32_t> bit_prefix;
     StreamScratch<uint32_t> final_ids;
-    StreamScratch<uint64_t> my_nodes;
-    StreamScratch<uint32_t> my_roots;
-    StreamScratch<uint32_t> my_ids;
-    // devices[0] only: the face graph
-    StreamScratch<Edge> all_edges;
-    StreamScratch<uint64_t> sorted;
-    StreamScratch<uint64_t> all_nodes;
-    StreamScratch<uint32_t> all_parent;
-    StreamScratch<uint32_t> all_roots;
-    StreamScratch<uint32_t> resolve_words;  // node count, then slab_first[]
-    StreamScratch<uint64_t> d_slab_base;
-    StreamScratch<char> resolve_storage;
+    StreamScratch<uint32_t> node_ids;
+    SlabArrays slab{grid, slab_base[s], nullptr, nullptr, nullptr, nullptr, nullptr, 0};
     StagedTransfer transfer;
     if (num_slabs >= 6)
     {
@@ -826,55 +1057,50 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
       }
     } drain{guard};
 
-    // 1. the slab up, steps 1-4 on it, K_g; the local roots of its last plane for the slab above
+    // 1. the slab up, labelled on its own, K_g; the local roots of its last plane for the slab
+    //    above
     const auto local_labelling = [&]() -> int
     {
       VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
       KeepPoolMemory(device);
       VGT_CUDA_TRY(cudaStreamCreateWithFlags(&guard.stream, cudaStreamNonBlocking), "stream");
       cudaStream_t stream = guard.stream;
+      const int scanned = ScanBytes(grid.count, &slab.scan_bytes);
+      if (scanned != VGT_B200_OK)
+      {
+        return scanned;
+      }
       VGT_CUDA_TRY(d_cells.Allocate(static_cast<int64_t>(grid.count) * kCellWords, stream),
                    "cell slab allocation");
       VGT_CUDA_TRY(parent.Allocate(grid.count, stream), "parent allocation");
       VGT_CUDA_TRY(mask.Allocate(words, stream), "root mask allocation");
       VGT_CUDA_TRY(word_prefix.Allocate(int64_t{words} + 1, stream), "word count allocation");
-      size_t scan_bytes = 0;
-      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, word_prefix.get(),
-                                                 word_prefix.get(), static_cast<int>(words) + 1,
-                                                 stream),
-                   "scan size query");
-      VGT_CUDA_TRY(scan_storage.Allocate(static_cast<int64_t>(std::max<size_t>(scan_bytes, 1)),
-                                         stream),
+      VGT_CUDA_TRY(scan_storage.Allocate(static_cast<int64_t>(slab.scan_bytes), stream),
                    "scan storage allocation");
-      VGT_CUDA_TRY(cudaMemsetAsync(word_prefix.get() + words, 0, sizeof(uint32_t), stream),
-                   "count reset");
+      slab.cells = d_cells.get();
+      slab.parent = parent.get();
+      slab.mask = mask.get();
+      slab.word_prefix = word_prefix.get();
+      slab.scan_storage = scan_storage.get();
       VGT_CUDA_TRY(transfer.ToDevice(reinterpret_cast<char*>(d_cells.get()), slab_bytes, h_slab,
                                      slab_bytes, slab_bytes, 1, stream),
                    "copy cell slab to device");
-      const uint32_t blocks = Blocks(grid.count);
-      InitRunsKernel<kCellWords><<<blocks, kThreads, 0, stream>>>(d_cells.get(), grid,
-                                                                  parent.get());
-      VGT_LAUNCHED("InitRunsKernel");
-      MergeKernel<kCellWords><<<blocks, kThreads, 0, stream>>>(d_cells.get(), grid, parent.get());
-      VGT_LAUNCHED("MergeKernel");
-      MarkRootsKernel<<<blocks, kThreads, 0, stream>>>(parent.get(), grid.count, mask.get(),
-                                                       word_prefix.get());
-      VGT_LAUNCHED("MarkRootsKernel");
-      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(scan_storage.get(), scan_bytes,
-                                                 word_prefix.get(), word_prefix.get(),
-                                                 static_cast<int>(words) + 1, stream),
-                   "root rank scan");
-      NoteKernelLaunch();
-      NoteKernelLaunch();
-      if (g + 1 < num_slabs)
+      const bool above = g + 1 < num_slabs;
+      if (above)
+      {
+        VGT_CUDA_TRY(face_roots.Allocate(plane, stream), "face root allocation");
+      }
+      const int labelled = LocalPhase<kCellWords>(slab, above ? face_roots.get() : nullptr,
+                                                  stream);
+      if (labelled != VGT_B200_OK)
+      {
+        return labelled;
+      }
+      if (above)
       {
         Shared& face = shared[s];
         face.last_plane.resize(size_t{plane} * kCellWords);
         face.face_roots.resize(plane);
-        VGT_CUDA_TRY(face_roots.Allocate(plane, stream), "face root allocation");
-        FaceRootsKernel<<<Blocks(plane), kThreads, 0, stream>>>(
-            parent.get(), grid.count - plane, plane, face_roots.get());
-        VGT_LAUNCHED("FaceRootsKernel");
         VGT_CUDA_TRY(cudaMemcpyAsync(face.face_roots.data(), face_roots.get(),
                                      sizeof(uint32_t) * plane, cudaMemcpyDeviceToHost, stream),
                      "copy face roots to host");
@@ -910,12 +1136,13 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
       VGT_CUDA_TRY(cudaMemcpyAsync(below_roots.get(), below.face_roots.data(),
                                    sizeof(uint32_t) * plane, cudaMemcpyHostToDevice, stream),
                    "copy face roots to device");
-      VGT_CUDA_TRY(cudaMemsetAsync(edge_count.get(), 0, sizeof(uint32_t), stream),
-                   "edge count reset");
-      FaceEdgesKernel<kCellWords><<<Blocks(plane), kThreads, 0, stream>>>(
-          below_plane.get(), below_roots.get(), slab_base[s - 1], d_cells.get(), parent.get(),
-          slab_base[s], plane, static_cast<uint32_t>(nz), edges.get(), edge_count.get());
-      VGT_LAUNCHED("FaceEdgesKernel");
+      const int emitted = FaceEdgesPhase<kCellWords>(below_plane.get(), below_roots.get(),
+                                                     slab_base[s - 1], slab, edges.get(),
+                                                     edge_count.get(), stream);
+      if (emitted != VGT_B200_OK)
+      {
+        return emitted;
+      }
       uint32_t count = 0;
       VGT_CUDA_TRY(cudaMemcpyAsync(&count, edge_count.get(), sizeof(uint32_t),
                                    cudaMemcpyDeviceToHost, stream),
@@ -929,13 +1156,9 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
       return VGT_B200_OK;
     };
 
-    // 3. devices[0]: the face graph resolved into compact roots
+    // 3. the edges of every face gathered, the face graph resolved (on every slab's device)
     const auto resolve = [&]() -> int
     {
-      if (g != 0)
-      {
-        return VGT_B200_OK;
-      }
       cudaStream_t stream = guard.stream;
       uint64_t total = 0;
       for (int f = 1; f < num_slabs; f++)
@@ -943,21 +1166,11 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
         total += shared[static_cast<size_t>(f)].edges.size();
       }
       const uint32_t num_edges = static_cast<uint32_t>(total);  // <= 7 * 2^26
-      const int num_endpoints = static_cast<int>(2 * total);
+      const int64_t capacity = std::max<int64_t>(1, 2 * total);
       VGT_CUDA_TRY(all_edges.Allocate(std::max<int64_t>(1, num_edges), stream), "edge allocation");
-      VGT_CUDA_TRY(sorted.Allocate(std::max(1, num_endpoints), stream), "endpoint allocation");
-      VGT_CUDA_TRY(all_nodes.Allocate(std::max(1, num_endpoints), stream), "node allocation");
-      VGT_CUDA_TRY(all_parent.Allocate(std::max(1, num_endpoints), stream),
-                   "node parent allocation");
-      VGT_CUDA_TRY(all_roots.Allocate(std::max(1, num_endpoints), stream), "node root allocation");
-      VGT_CUDA_TRY(resolve_words.Allocate(num_slabs + 2, stream), "node count allocation");
-      VGT_CUDA_TRY(d_slab_base.Allocate(num_slabs + 1, stream), "slab base allocation");
-      VGT_CUDA_TRY(cudaMemcpyAsync(d_slab_base.get(), slab_base.data(),
-                                   sizeof(uint64_t) * (num_slabs + 1), cudaMemcpyHostToDevice,
-                                   stream),
-                   "copy slab bases");
-      VGT_CUDA_TRY(cudaMemsetAsync(resolve_words.get(), 0, sizeof(uint32_t), stream),
-                   "node count reset");
+      VGT_CUDA_TRY(nodes.Allocate(capacity, stream), "node allocation");
+      VGT_CUDA_TRY(node_roots.Allocate(capacity, stream), "node root allocation");
+      VGT_CUDA_TRY(d_node_words.Allocate(3, stream), "node count allocation");
       uint32_t at = 0;
       for (int f = 1; f < num_slabs; f++)
       {
@@ -970,74 +1183,19 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
         }
         at += static_cast<uint32_t>(face.size());
       }
-      int end_bit = 1;
-      while (end_bit < 64 && (slab_base[static_cast<size_t>(num_slabs)] >> end_bit) != 0)
+      const uint64_t range[2] = {slab_base[s], slab_base[s + 1]};
+      const int resolved = ResolvePhase(all_edges.get(), num_edges, num_cells, range, 2,
+                                        nodes.get(), node_roots.get(), d_node_words.get(), stream);
+      if (resolved != VGT_B200_OK)
       {
-        end_bit++;
+        return resolved;
       }
-      const uint64_t* endpoints = reinterpret_cast<const uint64_t*>(all_edges.get());
-      size_t sort_bytes = 0;
-      size_t unique_bytes = 0;
-      VGT_CUDA_TRY(cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, endpoints, sorted.get(),
-                                                  num_endpoints, 0, end_bit, stream),
-                   "sort size query");
-      VGT_CUDA_TRY(cub::DeviceSelect::Unique(nullptr, unique_bytes, sorted.get(),
-                                             all_nodes.get(), resolve_words.get(),
-                                             num_endpoints, stream),
-                   "unique size query");
-      size_t storage_bytes = std::max<size_t>({sort_bytes, unique_bytes, 1});
-      VGT_CUDA_TRY(resolve_storage.Allocate(static_cast<int64_t>(storage_bytes), stream),
-                   "resolve storage allocation");
-      if (num_endpoints > 0)
-      {
-        VGT_CUDA_TRY(cub::DeviceRadixSort::SortKeys(resolve_storage.get(), sort_bytes, endpoints,
-                                                    sorted.get(), num_endpoints, 0, end_bit,
-                                                    stream),
-                     "endpoint sort");
-        NoteKernelLaunch();
-        VGT_CUDA_TRY(cub::DeviceSelect::Unique(resolve_storage.get(), unique_bytes, sorted.get(),
-                                               all_nodes.get(), resolve_words.get(),
-                                               num_endpoints, stream),
-                     "endpoint unique");
-        NoteKernelLaunch();
-      }
-      uint32_t nodes_total = 0;
-      VGT_CUDA_TRY(cudaMemcpyAsync(&nodes_total, resolve_words.get(), sizeof(uint32_t),
+      VGT_CUDA_TRY(cudaMemcpyAsync(node_words, d_node_words.get(), sizeof(node_words),
                                    cudaMemcpyDeviceToHost, stream),
                    "copy node count");
-      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "face graph nodes");
-      if (num_edges > 0)
-      {
-        NodeInitKernel<<<Blocks(nodes_total), kThreads, 0, stream>>>(all_parent.get(),
-                                                                     nodes_total);
-        VGT_LAUNCHED("NodeInitKernel");
-        NodeUnionKernel<<<Blocks(num_edges), kThreads, 0, stream>>>(
-            all_edges.get(), num_edges, all_nodes.get(), nodes_total, all_parent.get());
-        VGT_LAUNCHED("NodeUnionKernel");
-      }
-      NodeFlattenKernel<<<Blocks(std::max<uint32_t>(nodes_total, num_slabs + 1)), kThreads, 0,
-                          stream>>>(all_parent.get(), all_nodes.get(), nodes_total,
-                                    d_slab_base.get(), num_slabs + 1, all_roots.get(),
-                                    resolve_words.get() + 1);
-      VGT_LAUNCHED("NodeFlattenKernel");
-      VGT_CUDA_TRY(cudaMemcpyAsync(slab_first.data(), resolve_words.get() + 1,
-                                   sizeof(uint32_t) * (num_slabs + 1), cudaMemcpyDeviceToHost,
-                                   stream),
-                   "copy slab node ranges");
-      nodes.resize(nodes_total);
-      node_roots.resize(nodes_total);
-      node_ids.resize(nodes_total);
-      if (nodes_total > 0)
-      {
-        VGT_CUDA_TRY(cudaMemcpyAsync(nodes.data(), all_nodes.get(), sizeof(uint64_t) * nodes_total,
-                                     cudaMemcpyDeviceToHost, stream),
-                     "copy nodes to host");
-        VGT_CUDA_TRY(cudaMemcpyAsync(node_roots.data(), all_roots.get(),
-                                     sizeof(uint32_t) * nodes_total, cudaMemcpyDeviceToHost,
-                                     stream),
-                     "copy node roots to host");
-      }
       VGT_CUDA_TRY(cudaStreamSynchronize(stream), "face graph");
+      graph = SlabNodes{nodes.get(), node_roots.get(), node_words[0], node_words[1],
+                        node_words[2] - node_words[1]};
       return VGT_B200_OK;
     };
 
@@ -1045,51 +1203,15 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
     const auto count_global_roots = [&]() -> int
     {
       cudaStream_t stream = guard.stream;
-      first_node = slab_first[s];
-      num_nodes = slab_first[s + 1] - first_node;
-      const uint32_t bit_words = (num_components + 31) / 32;
+      const uint32_t bit_words = RootWords(num_components);
       VGT_CUDA_TRY(bits.Allocate(bit_words, stream), "root bit allocation");
       VGT_CUDA_TRY(bit_prefix.Allocate(int64_t{bit_words} + 1, stream), "root bit prefix allocation");
-      VGT_CUDA_TRY(my_nodes.Allocate(std::max<uint32_t>(1, num_nodes), stream), "node allocation");
-      VGT_CUDA_TRY(my_roots.Allocate(std::max<uint32_t>(1, num_nodes), stream),
-                   "node root allocation");
-      VGT_CUDA_TRY(my_ids.Allocate(std::max<uint32_t>(1, num_nodes), stream), "node id allocation");
-      GlobalRootBitsInitKernel<<<Blocks(bit_words), kThreads, 0, stream>>>(bits.get(),
-                                                                          num_components);
-      VGT_LAUNCHED("GlobalRootBitsInitKernel");
-      if (num_nodes > 0)
+      const int counted = CountPhase(slab, num_components, graph, bits.get(), bit_prefix.get(),
+                                     stream);
+      if (counted != VGT_B200_OK)
       {
-        VGT_CUDA_TRY(cudaMemcpyAsync(my_nodes.get(), nodes.data() + first_node,
-                                     sizeof(uint64_t) * num_nodes, cudaMemcpyHostToDevice, stream),
-                     "copy slab nodes to device");
-        VGT_CUDA_TRY(cudaMemcpyAsync(my_roots.get(), node_roots.data() + first_node,
-                                     sizeof(uint32_t) * num_nodes, cudaMemcpyHostToDevice, stream),
-                     "copy slab node roots to device");
-        ClearMergedBitsKernel<<<Blocks(num_nodes), kThreads, 0, stream>>>(
-            my_nodes.get(), my_roots.get(), num_nodes, first_node, slab_base[s], mask.get(),
-            word_prefix.get(), bits.get());
-        VGT_LAUNCHED("ClearMergedBitsKernel");
+        return counted;
       }
-      VGT_CUDA_TRY(cudaMemsetAsync(bit_prefix.get() + bit_words, 0, sizeof(uint32_t), stream),
-                   "count reset");
-      BitCountsKernel<<<Blocks(bit_words), kThreads, 0, stream>>>(bits.get(), bit_words,
-                                                                  bit_prefix.get());
-      VGT_LAUNCHED("BitCountsKernel");
-      // (bit_words + 1 <= words + 1: the scan storage of step 4 fits)
-      size_t scan_bytes = 0;
-      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, bit_prefix.get(),
-                                                 bit_prefix.get(),
-                                                 static_cast<int>(bit_words) + 1, stream),
-                   "scan size query");
-      StreamScratch<char> storage;
-      VGT_CUDA_TRY(storage.Allocate(static_cast<int64_t>(std::max<size_t>(scan_bytes, 1)), stream),
-                   "scan storage allocation");
-      VGT_CUDA_TRY(cub::DeviceScan::ExclusiveSum(storage.get(), scan_bytes, bit_prefix.get(),
-                                                 bit_prefix.get(),
-                                                 static_cast<int>(bit_words) + 1, stream),
-                   "global root scan");
-      NoteKernelLaunch();
-      NoteKernelLaunch();
       uint32_t count = 0;
       VGT_CUDA_TRY(cudaMemcpyAsync(&count, bit_prefix.get() + bit_words, sizeof(uint32_t),
                                    cudaMemcpyDeviceToHost, stream),
@@ -1099,11 +1221,12 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
       return VGT_B200_OK;
     };
 
-    // 5. offsets (refused past 0xFFFFFFFF, before any cell is written), ids of the slab's global
-    //    roots, published to devices[0]
+    // 5. offsets (refused past 0xFFFFFFFF, before any cell is written), the final ids of the
+    //    slab's global roots, the ids of its nodes published to the other slabs
     const auto publish = [&]() -> int
     {
       uint64_t total = 0;
+      uint64_t offset = 0;
       for (int f = 0; f < num_slabs; f++)
       {
         if (f == g)
@@ -1120,18 +1243,22 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
       }
       cudaStream_t stream = guard.stream;
       VGT_CUDA_TRY(final_ids.Allocate(num_components, stream), "final id allocation");
-      FinalIdsKernel<<<Blocks(num_components), kThreads, 0, stream>>>(
-          bits.get(), bit_prefix.get(), num_components, static_cast<uint32_t>(offset),
-          final_ids.get());
-      VGT_LAUNCHED("FinalIdsKernel");
-      if (num_nodes > 0)
+      VGT_CUDA_TRY(node_ids.Allocate(std::max<uint32_t>(1, graph.num_nodes), stream),
+                   "node id allocation");
+      const int published = PublishPhase(slab, num_components, static_cast<uint32_t>(offset),
+                                         graph, bits.get(), bit_prefix.get(), final_ids.get(),
+                                         node_ids.get(), stream);
+      if (published != VGT_B200_OK)
       {
-        PublishNodeIdsKernel<<<Blocks(num_nodes), kThreads, 0, stream>>>(
-            my_nodes.get(), num_nodes, slab_base[s], mask.get(), word_prefix.get(),
-            final_ids.get(), my_ids.get());
-        VGT_LAUNCHED("PublishNodeIdsKernel");
-        VGT_CUDA_TRY(cudaMemcpyAsync(node_ids.data() + first_node, my_ids.get(),
-                                     sizeof(uint32_t) * num_nodes, cudaMemcpyDeviceToHost, stream),
+        return published;
+      }
+      shared[s].first_node = graph.first;
+      shared[s].node_ids.resize(graph.count);
+      if (graph.count > 0)
+      {
+        VGT_CUDA_TRY(cudaMemcpyAsync(shared[s].node_ids.data(), node_ids.get() + graph.first,
+                                     sizeof(uint32_t) * graph.count, cudaMemcpyDeviceToHost,
+                                     stream),
                      "publish node ids");
       }
       VGT_CUDA_TRY(cudaStreamSynchronize(stream), "node id publication");
@@ -1139,52 +1266,34 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
       return VGT_B200_OK;
     };
 
-    // 6. devices[0]: every node takes its compact root's id
-    const auto propagate = [&]() -> int
-    {
-      const uint32_t nodes_total = slab_first[static_cast<size_t>(num_slabs)];
-      if (g != 0 || nodes_total == 0)
-      {
-        return VGT_B200_OK;
-      }
-      cudaStream_t stream = guard.stream;
-      StreamScratch<uint32_t> ids;
-      VGT_CUDA_TRY(ids.Allocate(nodes_total, stream), "node id allocation");
-      VGT_CUDA_TRY(cudaMemcpyAsync(ids.get(), node_ids.data(), sizeof(uint32_t) * nodes_total,
-                                   cudaMemcpyHostToDevice, stream),
-                   "copy node ids to device");
-      NodeIdsFromRootsKernel<<<Blocks(nodes_total), kThreads, 0, stream>>>(all_roots.get(),
-                                                                           nodes_total, ids.get());
-      VGT_LAUNCHED("NodeIdsFromRootsKernel");
-      VGT_CUDA_TRY(cudaMemcpyAsync(node_ids.data(), ids.get(), sizeof(uint32_t) * nodes_total,
-                                   cudaMemcpyDeviceToHost, stream),
-                   "copy node ids to host");
-      VGT_CUDA_TRY(cudaStreamSynchronize(stream), "node ids");
-      return VGT_B200_OK;
-    };
-
-    // 7. the final ids of the merged components, then the component word of every cell
+    // 6. the published ids of every slab together (their node ranges do not overlap), then the
+    //    component word of every cell
     const auto write = [&]() -> int
     {
       cudaStream_t stream = guard.stream;
-      if (num_nodes > 0)
+      std::vector<uint32_t> ids(graph.num_nodes, 0);
+      for (const Shared& other : shared)
       {
-        VGT_CUDA_TRY(cudaMemcpyAsync(my_ids.get(), node_ids.data() + first_node,
-                                     sizeof(uint32_t) * num_nodes, cudaMemcpyHostToDevice, stream),
-                     "copy node ids to device");
-        ApplyNodeIdsKernel<<<Blocks(num_nodes), kThreads, 0, stream>>>(
-            my_nodes.get(), my_ids.get(), num_nodes, slab_base[s], mask.get(), word_prefix.get(),
-            final_ids.get());
-        VGT_LAUNCHED("ApplyNodeIdsKernel");
+        std::copy(other.node_ids.begin(), other.node_ids.end(),
+                  ids.begin() + other.first_node);
       }
-      WriteSlabComponentsKernel<kCellWords><<<Blocks(grid.count), kThreads, 0, stream>>>(
-          d_cells.get(), grid.count, parent.get(), mask.get(), word_prefix.get(), final_ids.get());
-      VGT_LAUNCHED("WriteSlabComponentsKernel");
+      if (!ids.empty())
+      {
+        VGT_CUDA_TRY(cudaMemcpyAsync(node_ids.get(), ids.data(), sizeof(uint32_t) * ids.size(),
+                                     cudaMemcpyHostToDevice, stream),
+                     "copy node ids to device");
+      }
+      const int written = WritePhase<kCellWords>(slab, graph, node_ids.get(), final_ids.get(),
+                                                 stream);
+      if (written != VGT_B200_OK)
+      {
+        return written;
+      }
       VGT_CUDA_TRY(cudaStreamSynchronize(stream), "component write");
       return VGT_B200_OK;
     };
 
-    // 8. every slab has written: the cells back
+    // 7. every slab has written: the cells back
     const auto copy_back = [&]() -> int
     {
       VGT_CUDA_TRY(transfer.ToHost(h_slab, slab_bytes, reinterpret_cast<char*>(d_cells.get()),
@@ -1198,8 +1307,7 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
     // remaining phases are skipped.
     int status = VGT_B200_OK;
     const std::function<int()> phases[] = {local_labelling, face_edges, resolve,
-                                           count_global_roots, publish, propagate, write,
-                                           copy_back};
+                                           count_global_roots, publish, write, copy_back};
     for (const auto& phase : phases)
     {
       if (status == VGT_B200_OK && failed.load() != 0)
@@ -1246,6 +1354,73 @@ int ConnectedComponentsSlabs(char* h_cells, int64_t nx, int64_t ny, int64_t nz,
     }
   }
   *out_num_components = static_cast<uint32_t>(total_components);
+  return VGT_B200_OK;
+}
+
+// ---- checks of the per-slab entries (vgt_b200_components_*), before any device call ---------
+int CheckSlab(int cell_bytes, int64_t nx, int64_t ny, int64_t nz, Grid* grid)
+{
+  if (cell_bytes != 8 && cell_bytes != 16)
+  {
+    return FailInvalid("cell size must be 8 (OccupancyComponentCell) or 16 "
+                       "(TaggedObjectOccupancyComponentCell) bytes");
+  }
+  if (!ValidDims(nx, ny, nz))
+  {
+    return FailInvalid("slab dimensions %lld x %lld x %lld out of range (a slab has at least one "
+                       "x-plane)", static_cast<long long>(nx), static_cast<long long>(ny),
+                       static_cast<long long>(nz));
+  }
+  const int64_t count = nx * ny * nz;
+  if (count >= (int64_t{1} << 32))
+  {
+    SetLastError("connected components: slabs of 2^32 cells or more are not supported "
+                 "(%lld cells)", static_cast<long long>(count));
+    return VGT_B200_ERR_UNSUPPORTED;
+  }
+  *grid = Grid{static_cast<uint32_t>(nx), static_cast<uint32_t>(ny), static_cast<uint32_t>(nz),
+               static_cast<uint32_t>(count)};
+  return VGT_B200_OK;
+}
+
+int CheckPointers(std::initializer_list<std::pair<const void*, const char*>> pointers)
+{
+  for (const auto& pointer : pointers)
+  {
+    if (pointer.first == nullptr)
+    {
+      return FailInvalid("null %s", pointer.second);
+    }
+  }
+  return VGT_B200_OK;
+}
+
+// The slab's arrays and its share of the face graph, checked.
+int CheckSlabState(int64_t nx, int64_t ny, int64_t nz, int64_t base, int64_t num_components,
+                   int64_t num_nodes, int64_t first_node, int64_t num_slab_nodes, Grid* grid)
+{
+  const int checked = CheckSlab(8, nx, ny, nz, grid);
+  if (checked != VGT_B200_OK)
+  {
+    return checked;
+  }
+  if (base < 0 || base > (int64_t{1} << 62))
+  {
+    return FailInvalid("slab base %lld out of range", static_cast<long long>(base));
+  }
+  if (num_components < 1 || num_components > grid->count)
+  {
+    return FailInvalid("%lld local components in a slab of %u cells",
+                       static_cast<long long>(num_components), grid->count);
+  }
+  if (num_nodes < 0 || num_nodes > 0xFFFFFFFFll || first_node < 0 || num_slab_nodes < 0
+      || first_node + num_slab_nodes > num_nodes)
+  {
+    return FailInvalid("node range [%lld, %lld) outside the %lld nodes",
+                       static_cast<long long>(first_node),
+                       static_cast<long long>(first_node + num_slab_nodes),
+                       static_cast<long long>(num_nodes));
+  }
   return VGT_B200_OK;
 }
 }  // namespace
@@ -1353,5 +1528,240 @@ int vgt_b200_connected_components_multi(void* cells, int cell_bytes, int64_t nx,
   }
   return ConnectedComponentsSlabs<4>(static_cast<char*>(cells), nx, ny, nz, devices, num_slabs,
                                      out_num_components);
+}
+
+int vgt_b200_components_slab_scan_bytes(int64_t nx, int64_t ny, int64_t nz, int device,
+                                        size_t* out_bytes)
+{
+  Grid grid;
+  const int check = CheckSlab(8, nx, ny, nz, &grid);
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  const int pointers = CheckPointers({{out_bytes, "scan size"}});
+  if (pointers != VGT_B200_OK)
+  {
+    return pointers;
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  return ScanBytes(grid.count, out_bytes);
+}
+
+int vgt_b200_components_slab_local(void* d_cells, int cell_bytes, int64_t nx, int64_t ny,
+                                   int64_t nz, int device, uint32_t* d_parent, uint32_t* d_mask,
+                                   uint32_t* d_word_prefix, void* d_scan_storage,
+                                   size_t scan_bytes, uint32_t* d_face_roots, void* stream)
+{
+  Grid grid;
+  int check = CheckSlab(cell_bytes, nx, ny, nz, &grid);
+  if (check == VGT_B200_OK)
+  {
+    check = CheckPointers({{d_cells, "cell array"}, {d_parent, "parent array"},
+                           {d_mask, "root mask"}, {d_word_prefix, "word prefix"},
+                           {d_scan_storage, "scan storage"}});
+  }
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  const SlabArrays slab{grid, 0, static_cast<uint32_t*>(d_cells), d_parent, d_mask,
+                        d_word_prefix, d_scan_storage, scan_bytes};
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  return cell_bytes == 8 ? LocalPhase<2>(slab, d_face_roots, s)
+                         : LocalPhase<4>(slab, d_face_roots, s);
+}
+
+int vgt_b200_components_slab_face_edges(const void* d_below_cells, const uint32_t* d_below_roots,
+                                        int64_t below_base, void* d_cells, int cell_bytes,
+                                        int64_t nx, int64_t ny, int64_t nz, int64_t base,
+                                        int device, uint32_t* d_parent, int64_t* d_edges,
+                                        uint32_t* d_edge_count, void* stream)
+{
+  Grid grid;
+  int check = CheckSlab(cell_bytes, nx, ny, nz, &grid);
+  if (check == VGT_B200_OK)
+  {
+    check = CheckPointers({{d_below_cells, "face cell array"}, {d_below_roots, "face roots"},
+                           {d_cells, "cell array"}, {d_parent, "parent array"},
+                           {d_edges, "edge array"}, {d_edge_count, "edge count"}});
+  }
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  if (below_base < 0 || base < below_base + ny * nz)
+  {
+    return FailInvalid("slab bases %lld (below) and %lld out of order",
+                       static_cast<long long>(below_base), static_cast<long long>(base));
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  const SlabArrays slab{grid, static_cast<uint64_t>(base), static_cast<uint32_t*>(d_cells),
+                        d_parent, nullptr, nullptr, nullptr, 0};
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const uint32_t* below = static_cast<const uint32_t*>(d_below_cells);
+  Edge* edges = reinterpret_cast<Edge*>(d_edges);
+  return cell_bytes == 8
+             ? FaceEdgesPhase<2>(below, d_below_roots, static_cast<uint64_t>(below_base), slab,
+                                 edges, d_edge_count, s)
+             : FaceEdgesPhase<4>(below, d_below_roots, static_cast<uint64_t>(below_base), slab,
+                                 edges, d_edge_count, s);
+}
+
+int vgt_b200_components_resolve(const int64_t* d_edges, int64_t num_edges, int64_t num_cells,
+                                int64_t base, int64_t end, int device, int64_t* d_nodes,
+                                uint32_t* d_node_roots, uint32_t* d_node_range, void* stream)
+{
+  int check = CheckPointers({{d_nodes, "node array"}, {d_node_roots, "node roots"},
+                             {d_node_range, "node range"}});
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  if (num_edges < 0 || num_edges > (int64_t{1} << 30) || (num_edges > 0 && d_edges == nullptr))
+  {
+    return FailInvalid("%lld edges (at most 2^30, and a null edge array only without edges)",
+                       static_cast<long long>(num_edges));
+  }
+  if (num_cells < 1 || base < 0 || end <= base || end > num_cells)
+  {
+    return FailInvalid("slab [%lld, %lld) outside a map of %lld cells",
+                       static_cast<long long>(base), static_cast<long long>(end),
+                       static_cast<long long>(num_cells));
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  KeepPoolMemory(device);
+  const uint64_t range[2] = {static_cast<uint64_t>(base), static_cast<uint64_t>(end)};
+  return ResolvePhase(reinterpret_cast<const Edge*>(d_edges), static_cast<uint32_t>(num_edges),
+                      static_cast<uint64_t>(num_cells), range, 2,
+                      reinterpret_cast<uint64_t*>(d_nodes), d_node_roots, d_node_range,
+                      static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_components_slab_count(int64_t nx, int64_t ny, int64_t nz, int64_t base,
+                                   int64_t num_components, int device, const uint32_t* d_mask,
+                                   const uint32_t* d_word_prefix, const int64_t* d_nodes,
+                                   const uint32_t* d_node_roots, int64_t num_nodes,
+                                   int64_t first_node, int64_t num_slab_nodes, uint32_t* d_bits,
+                                   uint32_t* d_bit_prefix, void* d_scan_storage,
+                                   size_t scan_bytes, void* stream)
+{
+  Grid grid;
+  int check = CheckSlabState(nx, ny, nz, base, num_components, num_nodes, first_node,
+                             num_slab_nodes, &grid);
+  if (check == VGT_B200_OK)
+  {
+    check = CheckPointers({{d_mask, "root mask"}, {d_word_prefix, "word prefix"},
+                           {d_bits, "root bits"}, {d_bit_prefix, "root bit prefix"},
+                           {d_scan_storage, "scan storage"}});
+  }
+  if (check == VGT_B200_OK && num_slab_nodes > 0)
+  {
+    check = CheckPointers({{d_nodes, "node array"}, {d_node_roots, "node roots"}});
+  }
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  const SlabArrays slab{grid, static_cast<uint64_t>(base), nullptr, nullptr,
+                        const_cast<uint32_t*>(d_mask), const_cast<uint32_t*>(d_word_prefix),
+                        d_scan_storage, scan_bytes};
+  const SlabNodes graph{reinterpret_cast<const uint64_t*>(d_nodes), d_node_roots,
+                        static_cast<uint32_t>(num_nodes), static_cast<uint32_t>(first_node),
+                        static_cast<uint32_t>(num_slab_nodes)};
+  return CountPhase(slab, static_cast<uint32_t>(num_components), graph, d_bits, d_bit_prefix,
+                    static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_components_slab_publish(int64_t nx, int64_t ny, int64_t nz, int64_t base,
+                                     int64_t num_components, int64_t offset, int device,
+                                     const uint32_t* d_mask, const uint32_t* d_word_prefix,
+                                     const int64_t* d_nodes, int64_t num_nodes,
+                                     int64_t first_node, int64_t num_slab_nodes,
+                                     const uint32_t* d_bits, const uint32_t* d_bit_prefix,
+                                     uint32_t* d_final_ids, uint32_t* d_node_ids, void* stream)
+{
+  Grid grid;
+  int check = CheckSlabState(nx, ny, nz, base, num_components, num_nodes, first_node,
+                             num_slab_nodes, &grid);
+  if (check == VGT_B200_OK)
+  {
+    check = CheckPointers({{d_mask, "root mask"}, {d_word_prefix, "word prefix"},
+                           {d_bits, "root bits"}, {d_bit_prefix, "root bit prefix"},
+                           {d_final_ids, "final id array"}});
+  }
+  if (check == VGT_B200_OK && num_slab_nodes > 0)
+  {
+    check = CheckPointers({{d_nodes, "node array"}, {d_node_ids, "node id array"}});
+  }
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  if (offset < 0 || offset > 0xFFFFFFFFll)
+  {
+    return FailInvalid("component offset %lld out of range", static_cast<long long>(offset));
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  const SlabArrays slab{grid, static_cast<uint64_t>(base), nullptr, nullptr,
+                        const_cast<uint32_t*>(d_mask), const_cast<uint32_t*>(d_word_prefix),
+                        nullptr, 0};
+  const SlabNodes graph{reinterpret_cast<const uint64_t*>(d_nodes), nullptr,
+                        static_cast<uint32_t>(num_nodes), static_cast<uint32_t>(first_node),
+                        static_cast<uint32_t>(num_slab_nodes)};
+  return PublishPhase(slab, static_cast<uint32_t>(num_components), static_cast<uint32_t>(offset),
+                      graph, d_bits, d_bit_prefix, d_final_ids, d_node_ids,
+                      static_cast<cudaStream_t>(stream));
+}
+
+int vgt_b200_components_slab_write(void* d_cells, int cell_bytes, int64_t nx, int64_t ny,
+                                   int64_t nz, int64_t base, int64_t num_components, int device,
+                                   uint32_t* d_parent, const uint32_t* d_mask,
+                                   const uint32_t* d_word_prefix, const int64_t* d_nodes,
+                                   const uint32_t* d_node_roots, int64_t num_nodes,
+                                   int64_t first_node, int64_t num_slab_nodes,
+                                   uint32_t* d_node_ids, uint32_t* d_final_ids, void* stream)
+{
+  Grid grid;
+  int check = CheckSlab(cell_bytes, nx, ny, nz, &grid);
+  if (check == VGT_B200_OK)
+  {
+    check = CheckSlabState(nx, ny, nz, base, num_components, num_nodes, first_node,
+                           num_slab_nodes, &grid);
+  }
+  if (check == VGT_B200_OK)
+  {
+    check = CheckPointers({{d_cells, "cell array"}, {d_parent, "parent array"},
+                           {d_mask, "root mask"}, {d_word_prefix, "word prefix"},
+                           {d_final_ids, "final id array"}});
+  }
+  if (check == VGT_B200_OK && num_nodes > 0)
+  {
+    check = CheckPointers({{d_nodes, "node array"}, {d_node_roots, "node roots"},
+                           {d_node_ids, "node id array"}});
+  }
+  if (check != VGT_B200_OK)
+  {
+    return check;
+  }
+  ScopedDevice scoped(device);
+  VGT_CUDA_TRY(scoped.Status(), "cudaSetDevice");
+  const SlabArrays slab{grid, static_cast<uint64_t>(base), static_cast<uint32_t*>(d_cells),
+                        d_parent, const_cast<uint32_t*>(d_mask),
+                        const_cast<uint32_t*>(d_word_prefix), nullptr, 0};
+  const SlabNodes graph{reinterpret_cast<const uint64_t*>(d_nodes), d_node_roots,
+                        static_cast<uint32_t>(num_nodes), static_cast<uint32_t>(first_node),
+                        static_cast<uint32_t>(num_slab_nodes)};
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  return cell_bytes == 8 ? WritePhase<2>(slab, graph, d_node_ids, d_final_ids, s)
+                         : WritePhase<4>(slab, graph, d_node_ids, d_final_ids, s);
 }
 }  // extern "C"

@@ -398,3 +398,138 @@ class DeviceSignedDistanceField:
                         _stream_handle(device))
         _capi.check(code)
         return extrema
+
+
+class ComponentSlab:
+    """One rank's x-slab of a component map between the phases of the per-slab connected-
+    component entries (``vgt_b200_components_*``; DESIGN.md section 8): the cells [nx_r, ny, nz,
+    2 | 4] (contiguous int32 or uint32, labelled in place) and every array that lives from one
+    phase to the next. ``base`` is the global index of the slab's first cell. Each phase is
+    asynchronous on torch's current stream; the ones that return a number read it back."""
+
+    def __init__(self, cells: torch.Tensor, base: int):
+        if not cells.is_cuda:
+            raise _capi.BackendUnavailable("cells must live on a CUDA device (no CPU fallback)")
+        if cells.dtype not in (torch.int32, torch.uint32) or not cells.is_contiguous():
+            raise ValueError("cells must be a contiguous int32 or uint32 tensor")
+        if cells.dim() != 4 or cells.shape[3] not in (2, 4):
+            raise ValueError("cells must be [nx, ny, nz, 2] or [nx, ny, nz, 4]")
+        self.cells = cells
+        self.base = int(base)
+        self.device = cells.device
+        self.dims = tuple(int(d) for d in cells.shape[:3])
+        self.cell_bytes = 4 * int(cells.shape[3])
+        nx, ny, nz = self.dims
+        count = nx * ny * nz
+        root_words = (count + 31) // 32
+        scan_bytes = ctypes.c_size_t()
+        _capi.check(_capi.library().vgt_b200_components_slab_scan_bytes(
+            nx, ny, nz, self._index(), ctypes.byref(scan_bytes)))
+        self.parent = self._empty(count, torch.int32)
+        self.mask = self._empty(root_words, torch.int32)
+        self.word_prefix = self._empty(root_words + 1, torch.int32)
+        self.scan_storage = self._empty(scan_bytes.value, torch.uint8)
+        self.num_local = self.num_nodes = self.first_node = self.num_slab_nodes = 0
+        self.nodes = self.node_roots = self.bits = self.bit_prefix = self.final_ids = None
+
+    def _index(self) -> int:
+        return self.device.index or 0
+
+    def _empty(self, count: int, dtype: torch.dtype) -> torch.Tensor:
+        return torch.empty(count, dtype=dtype, device=self.device)
+
+    def _stream(self) -> int:
+        return _stream_handle(self.device)
+
+    def local(self, face_roots: bool) -> torch.Tensor | None:
+        """Labels the slab on its own; returns the local roots of its last x-plane (int32
+        [ny * nz]) when ``face_roots``, for the slab above."""
+        nx, ny, nz = self.dims
+        roots = self._empty(ny * nz, torch.int32) if face_roots else None
+        _capi.check(_capi.library().vgt_b200_components_slab_local(
+            self.cells.data_ptr(), self.cell_bytes, nx, ny, nz, self._index(),
+            self.parent.data_ptr(), self.mask.data_ptr(), self.word_prefix.data_ptr(),
+            self.scan_storage.data_ptr(), self.scan_storage.numel(),
+            None if roots is None else roots.data_ptr(), self._stream()))
+        return roots
+
+    def face_edges(self, below_cells: torch.Tensor, below_roots: torch.Tensor,
+                   below_base: int) -> torch.Tensor:
+        """The edges (int64 [E, 2]) of the face between the last x-plane of the slab below
+        (its cells [ny, nz, words] and local roots [ny * nz]) and this slab's first."""
+        nx, ny, nz = self.dims
+        _require_cuda(below_roots, torch.int32, "below_roots")
+        if (not below_cells.is_cuda or not below_cells.is_contiguous()
+                or below_cells.numel() != ny * nz * self.cell_bytes // 4
+                or below_roots.numel() != ny * nz):
+            raise ValueError("the face below must be one contiguous x-plane of cells and roots")
+        edges = torch.empty((ny * nz, 2), dtype=torch.int64, device=self.device)
+        count = self._empty(1, torch.int32)
+        _capi.check(_capi.library().vgt_b200_components_slab_face_edges(
+            below_cells.data_ptr(), below_roots.data_ptr(), int(below_base),
+            self.cells.data_ptr(), self.cell_bytes, nx, ny, nz, self.base, self._index(),
+            self.parent.data_ptr(), edges.data_ptr(), count.data_ptr(), self._stream()))
+        return edges[:int(count.item())]
+
+    def resolve(self, edges: torch.Tensor, num_cells: int) -> int:
+        """The face graph of all faces' edges (int64 [E, 2], any order) of a map of ``num_cells``
+        cells; returns the number of nodes (the same on every slab given the same edges)."""
+        _require_cuda(edges, torch.int64, "edges")
+        capacity = max(1, 2 * edges.shape[0])
+        self.nodes = self._empty(capacity, torch.int64)
+        self.node_roots = self._empty(capacity, torch.int32)
+        node_range = self._empty(3, torch.int32)
+        nx, ny, nz = self.dims
+        _capi.check(_capi.library().vgt_b200_components_resolve(
+            edges.data_ptr() if edges.numel() else None, edges.shape[0], int(num_cells), self.base,
+            self.base + nx * ny * nz, self._index(), self.nodes.data_ptr(),
+            self.node_roots.data_ptr(), node_range.data_ptr(), self._stream()))
+        self.num_nodes, self.first_node, end = node_range.tolist()
+        self.num_slab_nodes = end - self.first_node
+        return self.num_nodes
+
+    def _node_arguments(self):
+        return (self.nodes.data_ptr(), self.num_nodes, self.first_node, self.num_slab_nodes)
+
+    def count(self) -> int:
+        """count_g: the slab's components whose smallest index lies in the slab."""
+        nx, ny, nz = self.dims
+        self.num_local = int(self.word_prefix[-1].item()) & 0xFFFFFFFF
+        bit_words = (self.num_local + 31) // 32
+        self.bits = self._empty(bit_words, torch.int32)
+        self.bit_prefix = self._empty(bit_words + 1, torch.int32)
+        nodes, num_nodes, first, own = self._node_arguments()
+        _capi.check(_capi.library().vgt_b200_components_slab_count(
+            nx, ny, nz, self.base, self.num_local, self._index(), self.mask.data_ptr(),
+            self.word_prefix.data_ptr(), nodes, self.node_roots.data_ptr(), num_nodes, first, own,
+            self.bits.data_ptr(), self.bit_prefix.data_ptr(), self.scan_storage.data_ptr(),
+            self.scan_storage.numel(), self._stream()))
+        return int(self.bit_prefix[-1].item()) & 0xFFFFFFFF
+
+    def publish(self, offset: int) -> torch.Tensor:
+        """The final ids of the slab's components numbered from ``offset`` + 1; returns the node
+        ids (int32 [number of nodes] holding uint32 ids): this slab's nodes set, zero elsewhere."""
+        nx, ny, nz = self.dims
+        self.final_ids = self._empty(self.num_local, torch.int32)
+        node_ids = torch.zeros(max(1, self.num_nodes), dtype=torch.int32, device=self.device)
+        nodes, num_nodes, first, own = self._node_arguments()
+        _capi.check(_capi.library().vgt_b200_components_slab_publish(
+            nx, ny, nz, self.base, self.num_local, int(offset), self._index(),
+            self.mask.data_ptr(), self.word_prefix.data_ptr(), nodes, num_nodes, first, own,
+            self.bits.data_ptr(), self.bit_prefix.data_ptr(), self.final_ids.data_ptr(),
+            node_ids.data_ptr(), self._stream()))
+        return node_ids[:self.num_nodes]
+
+    def write(self, node_ids: torch.Tensor) -> None:
+        """The component word of every cell, from the node ids of every slab added up."""
+        nx, ny, nz = self.dims
+        if node_ids.numel() != self.num_nodes:
+            raise ValueError(f"expected {self.num_nodes} node ids, got {node_ids.numel()}")
+        _require_cuda(node_ids, torch.int32, "node_ids")
+        nodes, num_nodes, first, own = self._node_arguments()
+        _capi.check(_capi.library().vgt_b200_components_slab_write(
+            self.cells.data_ptr(), self.cell_bytes, nx, ny, nz, self.base, self.num_local,
+            self._index(), self.parent.data_ptr(), self.mask.data_ptr(),
+            self.word_prefix.data_ptr(), nodes, self.node_roots.data_ptr(), num_nodes, first, own,
+            node_ids.data_ptr() if num_nodes else None, self.final_ids.data_ptr(),
+            self._stream()))

@@ -479,3 +479,142 @@ class ShardedPointCloudVoxelizer:
         self.stages.filter(camera_counts, occupancy, filter_options)
         self.last_counts = camera_counts if keep_counts else None
         return occupancy
+
+
+# --------------------------------------------------------------------------------------------------
+# Sharded connected components: one x-slab of a component map per rank (DESIGN.md section 8)
+# --------------------------------------------------------------------------------------------------
+@dataclass
+class ComponentStages:
+    """The device phases of ShardedConnectedComponents.label on one rank's x-slab:
+    local(cells_slab, base, face_roots) -> (state, roots int32 [ny * nz] of the last x-plane, or
+        None when not face_roots)
+    face_edges(state, below_cells [ny, nz, words], below_roots [ny * nz], below_base)
+        -> int64 [E, 2] (global root below, global root above)
+    resolve(state, edges int64 [E, 2] of every face, num_cells) -> number of nodes
+    count(state) -> count_g
+    publish(state, offset) -> node ids int32 [number of nodes]: the slab's own set, zero elsewhere
+    write(state, node_ids summed over the ranks) -> None: the slab's component words written."""
+    local: Callable
+    face_edges: Callable
+    resolve: Callable
+    count: Callable
+    publish: Callable
+    write: Callable
+
+
+def cuda_component_stages() -> ComponentStages:
+    from . import device
+
+    def local(cells_slab, base, face_roots):
+        state = device.ComponentSlab(cells_slab, base)
+        return state, state.local(face_roots)
+
+    return ComponentStages(
+        local=local,
+        face_edges=lambda state, cells, roots, base: state.face_edges(cells, roots, base),
+        resolve=lambda state, edges, num_cells: state.resolve(edges, num_cells),
+        count=lambda state: state.count(),
+        publish=lambda state, offset: state.publish(offset),
+        write=lambda state, node_ids: state.write(node_ids))
+
+
+class ShardedConnectedComponents:
+    """ComputeConnectedComponents (topology_computation.hpp:138-196) on a component map cut into
+    x-slabs, one per rank, each on its rank's device: rank r holds the x-planes
+    split_range(nx, world_size, r) (the cut of ShardedSignedDistanceField). The result is the
+    whole-map labelling, the same bytes as the one-device entry.
+
+    Collectives, in order: the last x-plane of rank r (cells and local roots) sent to rank r + 1;
+    all_gather of the edge counts, then of the edges padded to the longest list; all_gather of
+    count_g (the offsets and the total); all_reduce SUM of the node ids."""
+
+    def __init__(self, dims, rank: int | None = None, world_size: int | None = None,
+                 group=None, stages: ComponentStages | None = None):
+        self.dims = tuple(int(d) for d in dims)
+        self.group = group
+        self.rank = dist.get_rank(group) if rank is None else rank
+        self.world_size = dist.get_world_size(group) if world_size is None else world_size
+        if self.world_size > self.dims[0]:
+            raise ValueError("more ranks than voxels along x")
+        self.stages = stages if stages is not None else cuda_component_stages()
+        self.x_range = split_range(self.dims[0], self.world_size, self.rank)
+
+    def x_slab_shape(self):
+        return (self.x_range[1] - self.x_range[0], self.dims[1], self.dims[2])
+
+    def label(self, cells_slab: torch.Tensor) -> int:
+        """cells_slab: this rank's x-slab [nx_r, ny, nz, 2 | 4], a contiguous int32 or uint32
+        tensor (2 words per OccupancyComponentCell, 4 per TaggedObjectOccupancyComponentCell).
+        Its component words are written in place; returns the number of components of the whole
+        map (the same on every rank). A map of more than 0xFFFFFFFF components raises
+        NotImplementedError on every rank before any cell is written."""
+        if tuple(cells_slab.shape[:3]) != self.x_slab_shape() or cells_slab.dim() != 4:
+            raise ValueError(f"expected an x-slab of shape {self.x_slab_shape()} + (words,)")
+        nx, ny, nz = self.dims
+        plane = ny * nz
+        world, rank = self.world_size, self.rank
+        base = self.x_range[0] * plane
+        stages = self.stages
+        state, roots = stages.local(cells_slab, base, rank + 1 < world)
+        edges = torch.zeros((0, 2), dtype=torch.int64, device=cells_slab.device)
+        if world > 1:
+            below_cells, below_roots = self._exchange_face(cells_slab, roots)
+            if rank > 0:
+                below_base = split_range(nx, world, rank - 1)[0] * plane
+                edges = stages.face_edges(state, below_cells, below_roots, below_base)
+            edges = self._gather_edges(edges)
+        stages.resolve(state, edges, nx * plane)
+        count = stages.count(state)
+        counts = [count]
+        if world > 1:
+            gathered = self._all_gather(torch.tensor([count], dtype=torch.int64,
+                                                     device=cells_slab.device))
+            counts = [int(c) for c in gathered.tolist()]
+        total = sum(counts)
+        if total > 0xFFFFFFFF:
+            raise NotImplementedError(f"connected components: {total} components do not fit the "
+                                      "32-bit component word")
+        node_ids = stages.publish(state, sum(counts[:rank]))
+        if world > 1 and node_ids.numel() > 0:
+            dist.all_reduce(node_ids, op=dist.ReduceOp.SUM, group=self.group)
+        stages.write(state, node_ids)
+        return total
+
+    def _exchange_face(self, cells_slab, roots):
+        """Rank r's last x-plane (cells as stored, their local roots) to rank r + 1."""
+        ny, nz = self.dims[1], self.dims[2]
+        words = cells_slab.shape[3]
+        device = cells_slab.device
+        below_cells = below_roots = None
+        ops = []
+        if self.rank + 1 < self.world_size:
+            last = cells_slab[-1].contiguous().view(torch.int32)
+            ops += [dist.P2POp(dist.isend, last, self.rank + 1, group=self.group),
+                    dist.P2POp(dist.isend, roots, self.rank + 1, group=self.group)]
+        if self.rank > 0:
+            below_cells = torch.empty((ny, nz, words), dtype=torch.int32, device=device)
+            below_roots = torch.empty(ny * nz, dtype=torch.int32, device=device)
+            ops += [dist.P2POp(dist.irecv, below_cells, self.rank - 1, group=self.group),
+                    dist.P2POp(dist.irecv, below_roots, self.rank - 1, group=self.group)]
+        for work in dist.batch_isend_irecv(ops):
+            work.wait()
+        return below_cells, below_roots
+
+    def _all_gather(self, tensor):
+        pieces = [torch.empty_like(tensor) for _ in range(self.world_size)]
+        dist.all_gather(pieces, tensor, group=self.group)
+        return torch.cat(pieces)
+
+    def _gather_edges(self, edges):
+        """Every rank's face edges, on every rank: their counts, then the edges padded to the
+        longest list."""
+        counts = self._all_gather(torch.tensor([edges.shape[0]], dtype=torch.int64,
+                                               device=edges.device)).tolist()
+        longest = max(counts)
+        if longest == 0:
+            return edges[:0]
+        padded = torch.zeros((longest, 2), dtype=torch.int64, device=edges.device)
+        padded[:edges.shape[0]] = edges
+        gathered = self._all_gather(padded.unsqueeze(0))
+        return torch.cat([gathered[r, :counts[r]] for r in range(self.world_size)]).contiguous()
